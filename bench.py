@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — throughput of the Tacotron2 decoder recurrence (the hot path, SURVEY.md §8) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[2] — data-parallel TRAINING, batch 64 per GPU,
 150 tokens, 800x80 mel frames — one "step" is Tacotron2.train_step (tacotron2.py:515-522) restricted to
@@ -198,35 +198,40 @@ def torch_gpu_legs(dev, steps=2, warmup=1, sample_T=GPU_TORCH_SAMPLE_T, infer_st
     autocast - plus the batched decode loop (initialize_decoder_states / prenet / decode driven for B rows, as the public
     inference is B = 1 only).  This is the "cuDNN/PyTorch GPU path" north_star asks to beat."""
     import torch
+    import torch.nn.functional as F
     import genvox_b200
+    from oracle import decoder_oracle as O
     B, N = TRAIN["B"], TRAIN["N"]
     out = {"device": torch.cuda.get_device_name(dev), "sample": f"B={B}, N={N}, {sample_T} of {TRAIN['T']} frames per train step; "
                                                                f"{infer_steps} of {INFER['steps']} decode steps"}
     memory, mel, gate, lengths = (t.to(dev) for t in synthetic_batch(torch, B, N, sample_T))
-    for name, ac in (("train_fp32", None), ("train_bf16_autocast", torch.bfloat16)):
-        dec = _baseline_decoder(dev)
-        P = None
-        if dec is None:
-            torch.manual_seed(0)
-            cont = genvox_b200.Decoder(**decoder_dims())
-            P = {k: v.detach().clone().to(dev).requires_grad_(True) for k, v in cont.named_parameters()}
-            import torch.nn.functional as F
-            from oracle import decoder_oracle as O
-            O.philox_dropout = lambda x, p, on, *a, **k: F.dropout(x, p, on)
-            O.get_mask_from_lengths = lambda lengths, max_len=None: (
-                torch.arange(max_len if max_len is not None else int(lengths.max()), device=dev)[None, :] >= lengths.to(dev)[:, None])
-        opt = torch.optim.Adam(list(dec.parameters()) if dec is not None else list(P.values()), lr=1e-3, weight_decay=1e-6)
-        step = _train_step_fn(torch, dec, P, opt, memory, mel, gate, lengths, autocast=ac)
-        for i in range(warmup):
-            step(i)
-        torch.cuda.synchronize(dev)
-        t0 = time.perf_counter()
-        for i in range(steps):
-            step(warmup + i)
-        torch.cuda.synchronize(dev)
-        dt = (time.perf_counter() - t0) / steps
-        out[name] = {"mel_frames_per_s": B * sample_T / dt, "ms_per_step": dt * 1e3, "kind": "reference" if dec is not None else "port"}
-        del opt, step, dec, P
+    # the port runs on the GPU here with torch's dropout and a device mask; the CPU leg after this one needs the originals
+    oracle_fns = O.philox_dropout, O.get_mask_from_lengths
+    try:
+        for name, ac in (("train_fp32", None), ("train_bf16_autocast", torch.bfloat16)):
+            dec = _baseline_decoder(dev)
+            P = None
+            if dec is None:
+                torch.manual_seed(0)
+                cont = genvox_b200.Decoder(**decoder_dims())
+                P = {k: v.detach().clone().to(dev).requires_grad_(True) for k, v in cont.named_parameters()}
+                O.philox_dropout = lambda x, p, on, *a, **k: F.dropout(x, p, on)
+                O.get_mask_from_lengths = lambda lengths, max_len=None: (
+                    torch.arange(max_len if max_len is not None else int(lengths.max()), device=dev)[None, :] >= lengths.to(dev)[:, None])
+            opt = torch.optim.Adam(list(dec.parameters()) if dec is not None else list(P.values()), lr=1e-3, weight_decay=1e-6)
+            step = _train_step_fn(torch, dec, P, opt, memory, mel, gate, lengths, autocast=ac)
+            for i in range(warmup):
+                step(i)
+            torch.cuda.synchronize(dev)
+            t0 = time.perf_counter()
+            for i in range(steps):
+                step(warmup + i)
+            torch.cuda.synchronize(dev)
+            dt = (time.perf_counter() - t0) / steps
+            out[name] = {"mel_frames_per_s": B * sample_T / dt, "ms_per_step": dt * 1e3, "kind": "reference" if dec is not None else "port"}
+            del opt, step, dec, P
+    finally:
+        O.philox_dropout, O.get_mask_from_lengths = oracle_fns
     dec = _baseline_decoder(dev)
     if dec is not None:
         dec.eval()
@@ -324,6 +329,27 @@ def slot_rooflines(phases, B, N, T, pk, precision):
 
 
 # ------------------------------------------------------------------------------------ GPU arm
+DUMP_MAX_ELEMS = 1 << 20      # per array; larger ones are sampled, so that a dump stays near 36 MB (at most 64 MB)
+
+
+def dump_outputs(out_dir, dec, loss, grad_norm):
+    """--dump-outputs: what the last timed train step hands its caller - the loss and the gradient norm it returns, and the
+    decoder's parameters and (clipped) gradients as the step leaves them - as float32 <name>.npy files in `out_dir`.  An array
+    of more than DUMP_MAX_ELEMS elements is stored flattened at a fixed, seeded sample of positions (the same in every run),
+    so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss, "grad_norm": grad_norm}
+    for k, p in dec.named_parameters():
+        arrays[f"param.{k}"] = p
+        arrays[f"grad.{k}"] = p.grad
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_MAX_ELEMS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def _stage(rank, msg):
     if os.environ.get("GVX_BENCH_TRACE"):
         print(f"[rank {rank}] {time.strftime('%H:%M:%S')} {msg}", file=sys.stderr, flush=True)
@@ -396,13 +422,15 @@ def run_ours(args, rank, world, local_rank):
     e0.record()
     host_t0 = time.perf_counter()
     for _ in range(K):
-        loss, _ = step_resident()
+        loss, grad_norm = step_resident()
     host_enqueue_ms = (time.perf_counter() - host_t0) * 1e3 / K      # host time to ENQUEUE a step (no sync inside)
     e1.record()
     barrier()
     launches = lib.gvx_launch_count() - launches0
     clocks = sampler.stop() if sampler else None
     _stage(rank, "timed region done")
+    if args.dump_outputs and rank == 0:          # before the e2e steps below change the parameters again
+        dump_outputs(args.dump_outputs, dec, loss, grad_norm)
     ms = max_over_ranks(e0.elapsed_time(e1)) / K
     value = world * B * T / (ms * 1e-3)
     final_loss = float(loss)
@@ -594,7 +622,14 @@ def main():
                     help="train: BASELINE configs[2] (the contract's line); infer_sharded: configs[3], utterances sharded over the GPUs")
     ap.add_argument("--precision", choices=["bf16", "fp32"], default="bf16",
                     help="arithmetic of the recurrent GEMMs (BASELINE configs[2] is bf16; fp32 = parity mode)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (loss, gradient norm, the decoder's "
+                         "parameters and gradients) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "train"):
+        ap.error("--dump-outputs needs --impl ours --mode train")
 
     # watchdog: a run that has not finished after 10 minutes (the default run takes about one) dumps every thread's Python
     # stack and exits instead of hanging its caller; GVX_BENCH_TRACE=1 adds per-stage progress lines on stderr

@@ -26,17 +26,24 @@ GOLDEN_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file
 LSTM_ROWS = [0, 1, 2, 3, 511, 1023, 1024, 1025, 2047, 2048, 2049, 3071, 3072, 3073, 4094, 4095]
 
 
-def grad_digest(name, g, full_limit=70000):
-    """What we keep of one gradient tensor: everything if small, else selected rows + norms."""
+def grad_digest(name, g, full_limit=70000, n_sample=1024, colsum_limit=20000):
+    """What we keep of one gradient tensor: everything if small, else norms, the sum over the first axis when it has at
+    most `colsum_limit` entries, and the values at a fixed sample of `n_sample` positions inside the rows LSTM_ROWS (`idx`:
+    flat indices into the tensor).  The limits keep every fixture file under 1 MB (the (60, 512) sum of d memory in
+    fwd_default_long would not fit)."""
     g = np.asarray(g)
     out = {f"{name}|sum": np.float64(g.astype(np.float64).sum()),
            f"{name}|l2": np.float64(np.sqrt((g.astype(np.float64) ** 2).sum()))}
     if g.size <= full_limit:
         out[f"{name}|full"] = g
-    else:
-        rows = [r for r in LSTM_ROWS if r < g.shape[0]]
-        out[f"{name}|rows"] = np.asarray(rows, dtype=np.int64)
-        out[f"{name}|rowvals"] = g[rows]
+        return out
+    rows = np.asarray([r for r in LSTM_ROWS if r < g.shape[0]], dtype=np.int64)
+    width = g.size // g.shape[0]
+    pick = np.sort(np.random.default_rng(0).choice(len(rows) * width, min(n_sample, len(rows) * width), replace=False))
+    idx = rows[pick // width] * width + pick % width
+    out[f"{name}|idx"] = idx
+    out[f"{name}|vals"] = g.reshape(-1)[idx]
+    if width <= colsum_limit:
         out[f"{name}|colsum"] = g.astype(np.float64).sum(0)
     return out
 
@@ -81,7 +88,8 @@ def keep_frames_of(T, head=12, stride=13, tail=12):
     return sorted(set(range(min(head, T))) | set(range(0, T, stride)) | set(range(max(0, T - tail), T)))
 
 
-def case_forward(tag, dims, B, N, T, wseed, iseed, dseed, training=True, with_grads=True, wscale=1.0, subsample=False):
+def case_forward(tag, dims, B, N, T, wseed, iseed, dseed, training=True, with_grads=True, wscale=1.0, subsample=False,
+                 full_limit=70000):
     W = synth.make_decoder_weights(wseed, dims, wscale)
     mem, mel, lens = synth.make_inputs(iseed, B, N, T, dims)
     r_mel = (synth.uniform01(iseed, 20, B * dims.n_mels * T) - 0.5).astype(np.float32).reshape(B, dims.n_mels, T)
@@ -96,7 +104,7 @@ def case_forward(tag, dims, B, N, T, wseed, iseed, dseed, training=True, with_gr
         out[f"mel_{sfx}"], out[f"gate_{sfx}"], out[f"align_{sfx}"] = m, g, a
         if grads is not None:
             for k, v in grads.items():
-                for kk, vv in grad_digest(k, v, 20000 if subsample else 70000).items():
+                for kk, vv in grad_digest(k, v, full_limit).items():
                     out[f"grad_{sfx}|{kk}"] = vv
     meta = dict(kind="forward", dims=dims.kwargs(), B=B, N=N, T=T, weight_seed=wseed, input_seed=iseed,
                 dropout_seed=dseed, training=training, weight_scale=wscale, lengths=lens.tolist(),
@@ -195,19 +203,19 @@ def main():
     D, S = synth.DecoderDims(), synth.SMALL_DIMS
     if "--new" in sys.argv:      # only the fixtures added in round 2 (the others regenerate bit-identically)
         if "--stops-only" not in sys.argv:
-            case_forward("fwd_default_long", D, B=4, N=60, T=400, wseed=7, iseed=19, dseed=131, subsample=True)
+            case_forward("fwd_default_long", D, B=4, N=60, T=400, wseed=7, iseed=19, dseed=131, subsample=True, full_limit=8192)
         case_decode_stops("stops_default_masked", D, B=6, N=33, steps=24, wseed=8, iseed=21, dseed=132, wscale=2.0)
         return 0
     case_forward("fwd_small_train", S, B=3, N=11, T=7, wseed=7, iseed=11, dseed=123, wscale=3.0)
     case_forward("fwd_small_eval", S, B=2, N=9, T=5, wseed=8, iseed=12, dseed=124, training=False, wscale=3.0)
-    case_forward("fwd_default_train", D, B=4, N=37, T=10, wseed=7, iseed=11, dseed=123)
+    case_forward("fwd_default_train", D, B=4, N=37, T=10, wseed=7, iseed=11, dseed=123, full_limit=8192)
     case_forward("fwd_default_eval_b1", D, B=1, N=16, T=6, wseed=9, iseed=13, dseed=125, training=False, with_grads=False)
     case_decode_loop("loop_default_nomask", D, B=3, N=23, steps=12, wseed=7, iseed=14, dseed=126, masked=False)
     case_decode_loop("loop_default_masked", D, B=5, N=40, steps=9, wseed=7, iseed=15, dseed=127, masked=True)
     case_decode_loop("loop_small_masked", S, B=4, N=13, steps=15, wseed=8, iseed=16, dseed=128, masked=True, wscale=3.0)
     case_public_inference("infer_default_b1_gate", D, N=29, wseed=7, iseed=17, dseed=129)
     case_public_inference("infer_small_b1_gate", S, N=10, wseed=8, iseed=18, dseed=130, wscale=3.0)
-    case_forward("fwd_default_long", D, B=4, N=60, T=400, wseed=7, iseed=19, dseed=131, subsample=True)
+    case_forward("fwd_default_long", D, B=4, N=60, T=400, wseed=7, iseed=19, dseed=131, subsample=True, full_limit=8192)
     case_decode_stops("stops_default_masked", D, B=6, N=33, steps=24, wseed=8, iseed=21, dseed=132, wscale=2.0)
 
 

@@ -1,11 +1,11 @@
-"""GPU tests of the drop-in wiring on the REAL reference Tacotron2 (imported unmodified from oracle/_ref on the GPU box): the
-reference model on the CPU is the yardstick, the same model with `genvox_b200.install`ed decoder on the B200 is the subject.
+"""GPU tests of the drop-in wiring on a whole Tacotron2 model (oracle/standin.py: the reference model's interface, its
+decoder the CPU oracle that tests/test_oracle_golden.py pins to the unmodified reference): that model on the CPU is the
+yardstick, the same model with `genvox_b200.install`ed decoder on the B200 is the subject.
 
   * `model_train_step` vs `Tacotron2.train_step` (tacotron2.py:515-522) on the same batch: same loss items, same gradient for
     every parameter of the model (embedding, encoder, decoder, postnet - the encoder's come through d memory);
   * `batched_inference` / `wiring.tts_batch` vs `Tacotron2.inference` (tacotron2.py:483-499) run once per utterance.
-The reference draws its dropout masks from torch's RNG; both sides are given the same counter-based Philox masks
-(oracle/ref_import.py::philox_dropout_patch), the encoder / postnet run in eval mode (no dropout, BatchNorm running statistics)."""
+Both decoders draw the same counter-based Philox dropout masks (same seed and row offset)."""
 import numpy as np
 import pytest
 import torch
@@ -14,9 +14,13 @@ import genvox_b200
 from conftest import rel_err
 from genvox_b200 import synthesis
 from genvox_b200.training import model_train_step
-from oracle import ref_import as R
+from oracle import standin, synth
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not R.reference_available(), reason="reference tree not staged (oracle/_ref)")]
+pytestmark = pytest.mark.gpu
+
+
+def _model(seed):
+    return standin.Tacotron2(synth.DecoderDims(), seed=seed)
 
 
 def _batch(B, n_tok, T, seed):
@@ -38,17 +42,15 @@ def test_model_train_step_matches_reference_train_step(cuda_device):
     # the encoder / postnet stay stock PyTorch on the GPU: keep cuDNN / cuBLAS out of TF32 so that they are comparable with the CPU
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
-    ref = R.build_reference_model(seed=2)
-    ours = genvox_b200.install(R.build_reference_model(seed=2)).to(cuda_device)
+    ref = _model(2)
+    ours = genvox_b200.install(_model(2)).to(cuda_device)
     for m in (ref, ours):
-        m.eval()                    # encoder / postnet: no dropout, BatchNorm running statistics
-        m.decoder.train()           # decoder: LSTM-state dropout on, like a training step
-        m.encoder.lstm.train()      # (cuDNN's RNN backward exists in training mode only; the BiLSTM has no dropout)
+        m.train()                   # decoder: LSTM-state dropout on, like a training step
     batch = _batch(B, n_tok, T, 5)
     # ---- reference: its own train_step on the CPU
     crit, opt = ref.get_criterion(), ref.get_optimizer()
-    with R.philox_dropout_patch(seed, "forward", count_inactive=False):
-        ref.train_step(batch={k: v.clone() for k, v in batch.items()}, criterion=crit, optimizer=opt)
+    ref.decoder.set_dropout_seed(seed)
+    ref.train_step(batch={k: v.clone() for k, v in batch.items()}, criterion=crit, optimizer=opt)
     ref_grads = {k: p.grad.clone() for k, p in ref.named_parameters()}
     # ---- installed model on the GPU through the data-parallel-ready step (no group: single process)
     ours.decoder.set_dropout_seed(seed)
@@ -69,8 +71,9 @@ def test_model_train_step_matches_reference_train_step(cuda_device):
 
 def test_batched_synthesis_matches_reference_inference_per_utterance(cuda_device):
     seed, steps = 77, 10
-    ref = R.build_reference_model(seed=4).eval()
-    ours = genvox_b200.install(R.build_reference_model(seed=4)).to(cuda_device).eval()
+    torch.backends.cudnn.allow_tf32 = False         # the postnet runs on the GPU on one side: no TF32 convolutions
+    ref = _model(4).eval()
+    ours = genvox_b200.install(_model(4)).to(cuda_device).eval()
     for m in (ref, ours):
         m.decoder.max_decoder_steps = steps
         m.decoder.gate_threshold = 0.999999            # random-init gate logits: every utterance runs to max_decoder_steps
@@ -82,8 +85,9 @@ def test_batched_synthesis_matches_reference_inference_per_utterance(cuda_device
     genvox_b200.check_device_errors()
     order = sorted(range(len(rows)), key=lambda i: -len(rows[i]))             # batched_inference decodes longest first
     for slot, i in enumerate(order):
-        with R.philox_dropout_patch(seed, "inference", row_offset=slot, skip=3):        # 3 = the encoder's conv dropout calls
-            r = ref.inference(inputs={"tokens": torch.IntTensor(rows[i]).unsqueeze(0)})
+        ref.decoder.set_dropout_seed(seed)
+        ref.decoder.dropout_row_offset = slot                                    # the row the utterance has in the batch
+        r = ref.inference(inputs={"tokens": torch.IntTensor(rows[i]).unsqueeze(0)})
         o = outs[i]
         assert set(o.keys()) == set(r.keys())
         for k in r:

@@ -1,28 +1,29 @@
-"""CPU tests of the drop-in wiring around the REAL reference Tacotron2 (SURVEY.md section 8b / 8f N2): `genvox_b200.install`
+"""CPU tests of the drop-in wiring around a Tacotron2 model (SURVEY.md section 8b / 8f N2): `genvox_b200.install`
 keeps the checkpoint contract, `genvox_b200.wiring.enable_data_parallel` shards the data and exchanges gradients
-(world_size 2, gloo).  The reference is imported unmodified (oracle/ref_import.py: /root/reference, or the staged copy
-oracle/_ref); the tests skip when neither exists."""
+(world_size 2, gloo).  The model is oracle/standin.py's Tacotron2: the reference model's interface around the CPU oracle
+decoder."""
 import os
 import socket
 import tempfile
 
-import pytest
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
 import genvox_b200
-from oracle import ref_import as R
+from oracle import standin, synth
 
-pytestmark = pytest.mark.skipif(not R.reference_available(), reason="reference tree not available")
+
+def _model(seed):
+    return standin.Tacotron2(synth.DecoderDims(), seed=seed)
 
 
 def test_install_keeps_state_dict_and_checkpoints_load_both_ways():
-    model = R.build_reference_model(seed=3)
+    model = _model(3)
     before = {k: v.clone() for k, v in model.state_dict().items()}
     ref_decoder_type = type(model.decoder)
     genvox_b200.install(model, precision="bf16")
-    assert isinstance(model.decoder, genvox_b200.Decoder) and model.decoder.precision == "bf16"
+    assert type(model.decoder) is genvox_b200.Decoder and model.decoder.precision == "bf16"
     after = model.state_dict()
     assert list(after.keys()) == list(before.keys())                       # same names, same order (checkpoint_manager.py:35-37)
     assert all(torch.equal(after[k], before[k]) for k in before)
@@ -33,13 +34,13 @@ def test_install_keeps_state_dict_and_checkpoints_load_both_ways():
     with tempfile.TemporaryDirectory() as d:
         path = os.path.join(d, "ckpt.pt")
         torch.save(ckpt, path)
-        fresh = R.build_reference_model(seed=99)
+        fresh = _model(99)
         assert isinstance(fresh.decoder, ref_decoder_type)
         fresh.load_checkpoint_statedicts(torch.load(path), save_optimizer_dict=True, optimizer=fresh.get_optimizer())
         assert all(torch.equal(fresh.state_dict()[k], before[k]) for k in before)
         # ... and a reference checkpoint -> an installed model
         torch.save(fresh.get_checkpoint_statedicts(optimizer=None), path)
-        other = genvox_b200.install(R.build_reference_model(seed=5))
+        other = genvox_b200.install(_model(5))
         other.load_checkpoint_statedicts(torch.load(path), save_optimizer_dict=False, optimizer=None)
         assert all(torch.equal(other.state_dict()[k], before[k]) for k in before)
     # train / eval mode follows the swapped module
@@ -87,7 +88,7 @@ def _dp_worker(rank, world, port, out):
     try:
         torch.set_num_threads(2)
         from genvox_b200 import wiring
-        model = R.build_reference_model(seed=1)              # identical init on both ranks; reference decoder (CPU)
+        model = _model(1)              # identical init on both ranks; oracle decoder (CPU)
         model.get_train_dataloader = lambda dump_dir, num_loader_workers, batch_size: torch.utils.data.DataLoader(
             _ToySet(12), batch_size=batch_size, shuffle=True, collate_fn=_collate)
         wiring.enable_data_parallel(model, rank, world, group=dist.group.WORLD, seed=4)
