@@ -294,6 +294,19 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(FB_THREADS, 1) k_att
         ws[tid] = tid < n_own ? a.align[((size_t)row * T + (T - 1)) * N + n_lo + tid] : 0.f;
         dals[tid] = (a.d_align && tid < n_own) ? a.d_align[((size_t)row * T + (T - 1)) * N + n_lo + tid] : 0.f;
     }
+    if (wid == 0 && a.d_align && rvalid) {
+        // carry dots of the first step: <w_{T-1}, d align_{T-1}> of every part of the row (there are no carries yet, but the
+        // alignment gradient is part of d w).  Later steps get theirs pushed by the parts; this sums in the same order as the
+        // parts do, so a run is bit-identical to the prefix of a longer run whose upstream gradient is zero after it.
+        const float *al = a.align + ((size_t)row * T + (T - 1)) * N, *dal = a.d_align + ((size_t)row * T + (T - 1)) * N;
+        for (int q = 0; q < RS; ++q) {
+            const int q_lo = q * G.NH, q_own = max(0, min(N, q_lo + G.NH) - q_lo), q_len = max(0, min(len, q_lo + q_own) - q_lo);
+            float p = 0.f;
+            for (int n = lane; n < q_len; n += 32) p = fmaf(al[q_lo + n], dal[q_lo + n], p);
+            p = warp_sum(p);
+            if (lane == 0) xch[q] = p;
+        }
+    }
     __syncthreads();
     cluster.sync();          // every CTA's mbarriers are initialised before any remote arrive
     const bool okw = fa_wait_mbar(&sh->wbar, 0, &sh->dead, a.err, 51);

@@ -260,13 +260,14 @@ def inference(P, memory, memory_lengths=None, max_decoder_steps: int = 1000, gat
 
 
 def loss_and_grads(P, memory, mel_in, memory_lengths, r_mel, r_gate, seed, training=True,
-                   p_att=0.1, p_dec=0.1, r_align=None):
+                   p_att=0.1, p_dec=0.1, r_align=None, row_offset: int = 0):
     """BPTT reference (a13): L = <mel, r_mel> + <gate, r_gate> (+ <align, r_align>), gradients
     to every parameter and to `memory` by torch autograd — what loss.backward()
-    (tacotron2.py:520) does to the decoder graph for upstream gradients r_*."""
+    (tacotron2.py:520) does to the decoder graph for upstream gradients r_*.
+    row_offset: the rows' first index in the dropout stream (a data-parallel rank's share of the batch)."""
     P = {k: v.detach().clone().requires_grad_(True) for k, v in P.items()}
     memory = memory.detach().clone().requires_grad_(True)
-    mel, gate, align = forward_teacher(P, memory, mel_in, memory_lengths, seed, training, p_att, p_dec)
+    mel, gate, align = forward_teacher(P, memory, mel_in, memory_lengths, seed, training, p_att, p_dec, row_offset)
     loss = (mel * r_mel).sum() + (gate * r_gate).sum()
     if r_align is not None:
         loss = loss + (align * r_align).sum()

@@ -158,3 +158,22 @@ def test_bf16_semantics_memory_rounding_is_opt_in_and_small():
     d01 = float((b0[0] - b1[0]).abs().max() / b0[0].abs().max())
     assert 0.0 < d01 < 5e-3                                                    # one more bf16 rounding: visible but small
     assert float((b0[0] - plain[0]).abs().max() / plain[0].abs().max()) < 3e-2
+
+
+def test_loss_and_grads_row_offset_selects_rows_of_one_dropout_stream():
+    """Rows k.. of a batch run at row offset 0 are what the same rows compute on their own at row offset k (rows never interact;
+    the dropout masks are drawn per global row): outputs and d memory equal, and the offset really changes the masks."""
+    dims = synth.SMALL_DIMS
+    B, N, T, k, seed = 5, 9, 4, 2, 11
+    P = O.as_params(synth.make_decoder_weights(3, dims), torch.float64)
+    mem, mel, lens = synth.make_inputs(5, B, N, T, dims)
+    mem, mel = torch.from_numpy(mem).double(), torch.from_numpy(mel).double()
+    u = lambda s, shape: torch.from_numpy(synth.uniform01(5, s, int(np.prod(shape))).reshape(shape) - 0.5)
+    r_mel, r_gate = u(20, (B, dims.n_mels, T)), u(21, (B, T))
+    r_mel[:k], r_gate[:k] = 0.0, 0.0
+    (m, g, a), _, dm = O.loss_and_grads(P, mem, mel, lens, r_mel, r_gate, seed)
+    (ms, gs, as_), _, dms = O.loss_and_grads(P, mem[k:], mel[k:], lens[k:], r_mel[k:], r_gate[k:], seed, row_offset=k)
+    for x, y in ((ms, m[k:]), (gs, g[k:]), (as_, a[k:]), (dms, dm[k:])):
+        assert rel_err(x, y) < 1e-12
+    (m0, _, _), _, _ = O.loss_and_grads(P, mem[k:], mel[k:], lens[k:], r_mel[k:], r_gate[k:], seed)
+    assert rel_err(m0, m[k:]) > 1e-2
