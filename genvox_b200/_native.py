@@ -69,6 +69,10 @@ _SIGNATURES = {
                                     C.c_uint64, C.c_int, C.c_int, _P, _P, _P, _P, _P, C.POINTER(GvxGrads), _P, _P]),
     "gvx_dec_infer": (C.c_int, [C.POINTER(GvxDims), C.POINTER(GvxWeights), _P, _P, _P, C.c_int, C.c_int, C.c_int,
                                 C.c_float, C.c_int, C.c_uint64, C.c_int, C.c_int, _P, _P, _P, _P, C.POINTER(C.c_int), _P, _P]),
+    "gvx_dec_infer_continuous_workspace_bytes": (C.c_size_t, [C.POINTER(GvxDims), C.c_int, C.c_int, C.c_int]),
+    "gvx_dec_infer_continuous": (C.c_int, [C.POINTER(GvxDims), C.POINTER(GvxWeights), _P, _P, _P, C.c_int, C.c_int, C.c_int,
+                                           C.c_int, _P, C.c_float, C.c_int, C.c_uint64, C.c_int, _P, _P, _P, _P,
+                                           C.POINTER(C.c_longlong), _P, _P]),
     "gvx_test_tc_gemm": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
     "gvx_test_nt_gemm": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
     "gvx_bench_nt_gemm": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float)]),

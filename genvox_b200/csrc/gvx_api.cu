@@ -55,21 +55,26 @@ int check_dims(const gvx_dims *d) {
 // ReLU + always-on dropout of a prenet layer in place (tacotron2.py:143), plus the optional bf16 copies: the epilogue of the
 // time-batched path below.  Element (row m, column c): frame m / rows_per_frame, batch row m % rows_per_frame.
 __global__ void __launch_bounds__(256) k_prenet_epilogue(float *__restrict__ x, int ld, size_t rows, int cols, DropCfg drop, uint32_t site,
-                                                         int t0, int rows_per_frame, int row_offset, BfDsts bf) {
+                                                         int t0, int rows_per_frame, int row_offset, BfDsts bf,
+                                                         const int *__restrict__ row_frame, const int *__restrict__ row_id) {
     const size_t total = rows * (size_t)cols;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t m = i / cols;
         const int c = (int)(i - m * cols);
         const int f = (int)(m / rows_per_frame), brow = (int)(m - (size_t)f * rows_per_frame);
-        const float v = fmaxf(x[m * ld + c], 0.f) * drop_mult(drop, site, (uint32_t)(t0 + f), (uint32_t)(brow + row_offset), (uint32_t)c);
+        const uint32_t tf = row_frame ? (uint32_t)row_frame[brow] : (uint32_t)(t0 + f);
+        const uint32_t rw = (uint32_t)((row_id ? row_id[brow] : brow) + row_offset);
+        const float v = fmaxf(x[m * ld + c], 0.f) * drop_mult(drop, site, tf, rw, (uint32_t)c);
         x[m * ld + c] = v;
         if (bf.n) bf_store1_t(bf, f, brow, c, v);
     }
 }
 
-// Prenet.forward over `rows` = F*B rows (tacotron2.py:140-144)
+// Prenet.forward over `rows` = F*B rows (tacotron2.py:140-144).  row_frame / row_id (optional, device [B], one frame only):
+// per-row Philox t and row (before row_offset) in place of t0 and the batch row.
 int run_prenet(const Dims &d, const gvx_weights *w, const float *frames, int frames_ld, int rows, int B, uint64_t seed,
-               int t0, int row_offset, float *pre1, float *pre2, cudaStream_t st, const BfDsts *bf = nullptr) {
+               int t0, int row_offset, float *pre1, float *pre2, cudaStream_t st, const BfDsts *bf = nullptr,
+               const int *row_frame = nullptr, const int *row_id = nullptr) {
     if (rows >= 4096) {
         // all frames of a teacher-forced pass at once: a plain fp32 library GEMM per layer (exact fp32 products, like the skinny
         // FFMA kernel below, which needs 0.84 ms for the 51200 rows of configs[2]) + one elementwise pass
@@ -81,7 +86,7 @@ int run_prenet(const Dims &d, const gvx_weights *w, const float *frames, int fra
             memset(&none, 0, sizeof(none));
             k_prenet_epilogue<<<grid_for((size_t)rows * d.P), 256, 0, st>>>(out, d.P, (size_t)rows, d.P, make_drop(seed, 0.5f, 1),
                                                                           layer == 0 ? SITE_PRENET0 : SITE_PRENET1, t0, B, row_offset,
-                                                                          (layer == 1 && bf) ? *bf : none);
+                                                                          (layer == 1 && bf) ? *bf : none, row_frame, row_id);
             GVX_LAUNCHED(1);
             GVX_CUDA(cudaGetLastError());
         }
@@ -101,6 +106,8 @@ int run_prenet(const Dims &d, const gvx_weights *w, const float *frames, int fra
         e.t0 = t0;
         e.rows_per_frame = B;
         e.row_offset = row_offset;
+        e.row_frame = row_frame;
+        e.row_id = row_id;
         if (layer == 1 && bf) e.bf = *bf;
         GVX_TRY((launch_gemm<32, EpiStore>(g, e, st)));
     }
@@ -351,6 +358,43 @@ static int train_fwd_body(const gvx_dims *dd, const gvx_weights *w, const void *
     return 0;
 }
 
+// One decoder step of inference (tacotron2.py:398-403): prenet on the previous mel frame `prev` (dropout on, :143), attention
+// LSTM, attention (weights to align_t, row stride align_bstride), decoder LSTM, [mel | gate] projection to out_t.
+// row_frame / row_id: optional per-row prenet dropout frame and row (run_prenet).
+static int infer_step(const Dims &d, const gvx_weights *w, const float *packed, const InferL &L, float *s, const float *memory,
+                      const int64_t *mem_lengths, int B, int N, uint64_t seed, int t, int training, int row_offset,
+                      const int *row_frame, const int *row_id, const float *prev, float *align_t, long long align_bstride,
+                      float *out_t, bool fused_prenet, cudaStream_t st) {
+    const int cur = t & 1, nxt = cur ^ 1;
+    const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H;
+    int *flags = (int *)(s + L.FLAGS);
+    { ProfScope ps(PS_PRENET, st);
+      if (fused_prenet) {
+          GVX_TRY(run_infer_prenet(d, w, prev, d.OL, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, nullptr, (unsigned *)(flags + 40), flags + 41, st,
+                                   row_frame, row_id));
+      } else {
+          GVX_TRY(run_prenet(d, w, prev, d.OL, B, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, st, nullptr, row_frame, row_id));
+      } }
+    LstmIO a;
+    a.x0 = s + L.PRE2; a.w0 = d.P; a.ld0 = d.P;
+    a.x1 = s + L.CTX; a.w1 = d.E; a.ld1 = d.E;
+    a.x2 = s + L.HA + cur * BA; a.w2 = d.A; a.ld2 = d.A;
+    a.c_prev = s + L.CA; a.c_out = s + L.CA; a.h_out = s + L.HA + nxt * BA; a.gates_out = nullptr;
+    { ProfScope ps(PS_ATT_LSTM, st); GVX_TRY(run_lstm(d, packed, 0, a, B, seed, t, training, row_offset, st)); }
+    { ProfScope ps(PS_QUERY, st); GVX_TRY(run_query(d, w, s + L.HA + nxt * BA, B, s + L.Q, st)); }
+    { ProfScope ps(PS_ATTENTION, st);
+      GVX_TRY(run_attention(d, w, packed, s + L.Q, s + L.PM, memory, mem_lengths, B, N, s + L.WPREV, s + L.CUM,
+                            align_t, align_bstride, nullptr, s + L.CTX, nullptr, nullptr, st)); }
+    LstmIO c;
+    c.x0 = s + L.HA + nxt * BA; c.w0 = d.A; c.ld0 = d.A;
+    c.x1 = s + L.CTX; c.w1 = d.E; c.ld1 = d.E;
+    c.x2 = s + L.HD + cur * BH; c.w2 = d.H; c.ld2 = d.H;
+    c.c_prev = s + L.CD; c.c_out = s + L.CD; c.h_out = s + L.HD + nxt * BH; c.gates_out = nullptr;
+    { ProfScope ps(PS_DEC_LSTM, st); GVX_TRY(run_lstm(d, packed, 1, c, B, seed, t, training, row_offset, st)); }
+    { ProfScope ps(PS_PROJ, st); GVX_TRY(run_projection(d, packed, s + L.HD + nxt * BH, d.H, s + L.CTX, d.E, B, out_t, st, true)); }
+    return 0;
+}
+
 static int infer_body(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
                       const int64_t *mem_lengths, int B, int N, int max_steps, float gate_threshold, int ignore_gate,
                       uint64_t seed, int training, int row_offset, float *mel_out, float *gate_out, float *align_out,
@@ -386,33 +430,10 @@ static int infer_body(const gvx_dims *dd, const gvx_weights *w, const void *pack
     int t = 0, host_running = B;
     pdl_barrier_next();
     for (; t < max_steps; ++t) {
-        const int cur = t & 1, nxt = cur ^ 1;
-        // prenet on the previous mel frame, dropout on (tacotron2.py:398, :143)
         const float *prev = t == 0 ? s + L.ZERO : s + L.OUT + (size_t)(t - 1) * B * d.OL;
-        { ProfScope ps(PS_PRENET, st);
-          if (fused_prenet) {
-              GVX_TRY(run_infer_prenet(d, w, prev, d.OL, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, nullptr, (unsigned *)(flags + 40), flags + 41, st));
-          } else {
-              GVX_TRY(run_prenet(d, w, prev, d.OL, B, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, st));
-          } }
-        LstmIO a;
-        a.x0 = s + L.PRE2; a.w0 = d.P; a.ld0 = d.P;
-        a.x1 = s + L.CTX; a.w1 = d.E; a.ld1 = d.E;
-        a.x2 = s + L.HA + cur * BA; a.w2 = d.A; a.ld2 = d.A;
-        a.c_prev = s + L.CA; a.c_out = s + L.CA; a.h_out = s + L.HA + nxt * BA; a.gates_out = nullptr;
-        { ProfScope ps(PS_ATT_LSTM, st); GVX_TRY(run_lstm(d, packed, 0, a, B, seed, t, training, row_offset, st)); }
-        { ProfScope ps(PS_QUERY, st); GVX_TRY(run_query(d, w, s + L.HA + nxt * BA, B, s + L.Q, st)); }
-        { ProfScope ps(PS_ATTENTION, st);
-          GVX_TRY(run_attention(d, w, packed, s + L.Q, s + L.PM, memory, mem_lengths, B, N, s + L.WPREV, s + L.CUM,
-                                align_out + (size_t)t * N, (long long)max_steps * N, nullptr, s + L.CTX, nullptr, nullptr, st)); }
-        LstmIO c;
-        c.x0 = s + L.HA + nxt * BA; c.w0 = d.A; c.ld0 = d.A;
-        c.x1 = s + L.CTX; c.w1 = d.E; c.ld1 = d.E;
-        c.x2 = s + L.HD + cur * BH; c.w2 = d.H; c.ld2 = d.H;
-        c.c_prev = s + L.CD; c.c_out = s + L.CD; c.h_out = s + L.HD + nxt * BH; c.gates_out = nullptr;
-        { ProfScope ps(PS_DEC_LSTM, st); GVX_TRY(run_lstm(d, packed, 1, c, B, seed, t, training, row_offset, st)); }
         float *out_t = s + L.OUT + (size_t)t * B * d.OL;
-        { ProfScope ps(PS_PROJ, st); GVX_TRY(run_projection(d, packed, s + L.HD + nxt * BH, d.H, s + L.CTX, d.E, B, out_t, st, true)); }
+        GVX_TRY(infer_step(d, w, packed, L, s, memory, mem_lengths, B, N, seed, t, training, row_offset, nullptr, nullptr, prev,
+                           align_out + (size_t)t * N, (long long)max_steps * N, out_t, fused_prenet, st));
         if (!ignore_gate) {
             GVX_CUDA(launch_pdl(k_gate_check, dim3(1), dim3(128), 0, st, (const float *)out_t, B, d.M, d.OL, gate_threshold, t, n_frames, flags));
     GVX_LAUNCHED(1);
@@ -605,3 +626,4 @@ int gvx_attention_step(const gvx_dims *dd, const gvx_weights *w, const void *pac
 // backward through time (gvx_dec_train_bwd) lives in its own file, same translation unit
 #include "gvx_bwd.cuh"
 #include "gvx_bf16_api.cuh"
+#include "gvx_continuous.cuh"

@@ -822,20 +822,90 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
 }
 
 // ======================================================================================= inference
+// One decoder step (tacotron2.py:398-403): prenet on the previous mel frame `prev` (straight into the attention-LSTM operand
+// image), attention LSTM, query, attention (weights to align_t, row stride align_bstride), decoder LSTM, [mel | gate] projection
+// to out_t.  row_frame / row_id: optional per-row prenet dropout frame and row (run_infer_prenet, run_prenet).
+static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *packed, const InferBfL &L, float *s, const float *memory,
+                           const int64_t *mem_lengths, int B, int N, uint64_t seed, int t, int training, int row_offset,
+                           const int *row_frame, const int *row_id, const float *prev, float *align_t, long long align_bstride,
+                           float *out_t, cudaStream_t st) {
+    const BfGeom g(d);
+    const PackedL PL(d);
+    const PackedBfL BL(d, PL.total);
+    const int NPAD = L.NPAD;
+    bf16 *XAI = (bf16 *)(s + L.XAI), *XDI = (bf16 *)(s + L.XDI), *XPI = (bf16 *)(s + L.XPI);
+    int *err = (int *)(s + L.ERR), *flags = (int *)(s + L.FLAGS);
+    const bf16 *WaI = (const bf16 *)(packed + BL.WaI), *WdI = (const bf16 *)(packed + BL.WdI), *WqI = (const bf16 *)(packed + BL.WqI),
+               *WpgI = (const bf16 *)(packed + BL.WpgI);
+    bf16 *xa = XAI + (size_t)(t & 1) * L.xai_stride, *xa_n = XAI + (size_t)((t + 1) & 1) * L.xai_stride;
+    bf16 *xd = XDI + (size_t)(t & 1) * L.xdi_stride, *xd_n = XDI + (size_t)((t + 1) & 1) * L.xdi_stride;
+    {
+        ProfScope ps(PS_PRENET, st);
+        BfDsts bf;
+        memset(&bf, 0, sizeof(bf));
+        add_img(bf, xa, 0, NPAD);
+        if (infer_prenet_fused_ok(d, B)) {
+            GVX_TRY(run_infer_prenet(d, w, prev, d.OL, B, seed, t, row_offset, s + L.PRE1, nullptr, &bf, (unsigned *)(flags + 40), err, st,
+                                     row_frame, row_id));
+        } else {
+            GVX_TRY(run_prenet(d, w, prev, d.OL, B, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, st, &bf, row_frame, row_id));
+        }
+    }
+    {
+        ProfScope ps(PS_ATT_LSTM, st);
+        BfDsts h;
+        memset(&h, 0, sizeof(h));
+        add_img(h, xd, 0, NPAD); add_img(h, xa_n, d.P + d.E, NPAD);
+        GVX_TRY(run_lstm_bf16(d, packed, 0, WaI, xa, s + L.PA, L.KSa, g.Ta, g.Kpa, s + L.CA, s + L.CA, nullptr, h, B, seed, t,
+                              training, row_offset, err, st));
+    }
+    {
+        ProfScope ps(PS_QUERY, st);
+        GVX_TRY(run_tc(WqI, xd, s + L.PQ, g.Tq, g.Kpq, L.KSq, B, err, st));
+    }
+    {
+        ProfScope ps(PS_ATTENTION, st);
+        AttnFwdArgs a;
+        memset(&a, 0, sizeof(a));
+        a.s = AttnShape{B, N, d.D, d.E, d.F, d.KS};
+        a.q = src_split(s + L.PQ, g.Tq * TC_M, L.KSq, (long long)B * g.Tq * TC_M);
+        a.pm = s + L.PM; a.memory = memory;
+        a.wlc = w->loc_conv_w; a.wldT = packed + PL.wldT; a.v = w->v_w; a.lengths = mem_lengths;
+        a.w_prev = s + L.WPREV; a.cum = s + L.CUM;
+        a.align_out = align_t; a.align_bstride = align_bstride;
+        a.ctx_ld = d.E;
+        add_img(a.ctx_bf, xd, d.A, NPAD); add_img(a.ctx_bf, xa_n, d.P, NPAD); add_img(a.ctx_bf, XPI, d.H, NPAD);
+        GVX_TRY(launch_attention_fwd_best(a, st));
+    }
+    {
+        ProfScope ps(PS_DEC_LSTM, st);
+        BfDsts h;
+        memset(&h, 0, sizeof(h));
+        add_img(h, XPI, 0, NPAD); add_img(h, xd_n, d.A + d.E, NPAD);
+        GVX_TRY(run_lstm_bf16(d, packed, 1, WdI, xd, s + L.PD, L.KSd, g.Td, g.Kpd, s + L.CD, s + L.CD, nullptr, h, B, seed, t,
+                              training, row_offset, err, st));
+    }
+    {
+        ProfScope ps(PS_PROJ, st);
+        GVX_TRY(run_tc(WpgI, XPI, s + L.PP, g.Tp, g.Kpp, L.KSp, B, err, st));
+        GVX_CUDA(launch_pdl(k_bf_finalize, dim3(grid_for((size_t)B * (d.M + 1))), dim3(256), 0, st, (const float *)(s + L.PP), L.KSp,
+                            B, g.Tp * TC_M, d.M + 1, (const float *)(packed + PL.bpg), out_t, d.OL));
+        GVX_LAUNCHED(1);
+        GVX_CUDA(cudaGetLastError());
+    }
+    return 0;
+}
+
 int infer_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
                       int B, int N, int max_steps, float gate_threshold, int ignore_gate, uint64_t seed, int training,
                       int row_offset, float *mel_out, float *gate_out, float *align_out, int32_t *n_frames, int *steps_run, float *s,
                       cudaStream_t st) {
     GVX_TRY(check_bf16_dims(d, B));
     const BfGeom g(d);
-    const PackedL PL(d);
-    const PackedBfL BL(d, PL.total);
     const InferBfL L(d, B, N, max_steps);
     const int NPAD = L.NPAD;
     bf16 *XAI = (bf16 *)(s + L.XAI), *XDI = (bf16 *)(s + L.XDI), *XPI = (bf16 *)(s + L.XPI);
     int *err = (int *)(s + L.ERR), *flags = (int *)(s + L.FLAGS);
-    const bf16 *WaI = (const bf16 *)(packed + BL.WaI), *WdI = (const bf16 *)(packed + BL.WdI), *WqI = (const bf16 *)(packed + BL.WqI),
-               *WpgI = (const bf16 *)(packed + BL.WpgI);
 
     GVX_TRY(run_processed_memory(d, w, memory, B, N, s + L.PM, st));
     GVX_CUDA(cudaMemsetAsync(err, 0, 64 * sizeof(float), st));
@@ -856,63 +926,10 @@ int infer_bf16(const Dims &d, const gvx_weights *w, const float *packed, const f
     int t = 0, host_running = B;
     pdl_barrier_next();
     for (; t < max_steps; ++t) {
-        bf16 *xa = XAI + (size_t)(t & 1) * L.xai_stride, *xa_n = XAI + (size_t)((t + 1) & 1) * L.xai_stride;
-        bf16 *xd = XDI + (size_t)(t & 1) * L.xdi_stride, *xd_n = XDI + (size_t)((t + 1) & 1) * L.xdi_stride;
-        {   // prenet on the previous mel frame (tacotron2.py:398), output straight into the attention-LSTM operand image
-            ProfScope ps(PS_PRENET, st);
-            const float *prev = t == 0 ? s + L.ZERO : s + L.OUT + (size_t)(t - 1) * B * d.OL;
-            BfDsts bf;
-            memset(&bf, 0, sizeof(bf));
-            add_img(bf, xa, 0, NPAD);
-            if (infer_prenet_fused_ok(d, B)) {
-                GVX_TRY(run_infer_prenet(d, w, prev, d.OL, B, seed, t, row_offset, s + L.PRE1, nullptr, &bf, (unsigned *)(flags + 40), err, st));
-            } else {
-                GVX_TRY(run_prenet(d, w, prev, d.OL, B, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, st, &bf));
-            }
-        }
-        {
-            ProfScope ps(PS_ATT_LSTM, st);
-            BfDsts h;
-            memset(&h, 0, sizeof(h));
-            add_img(h, xd, 0, NPAD); add_img(h, xa_n, d.P + d.E, NPAD);
-            GVX_TRY(run_lstm_bf16(d, packed, 0, WaI, xa, s + L.PA, L.KSa, g.Ta, g.Kpa, s + L.CA, s + L.CA, nullptr, h, B, seed, t,
-                                  training, row_offset, err, st));
-        }
-        {
-            ProfScope ps(PS_QUERY, st);
-            GVX_TRY(run_tc(WqI, xd, s + L.PQ, g.Tq, g.Kpq, L.KSq, B, err, st));
-        }
-        {
-            ProfScope ps(PS_ATTENTION, st);
-            AttnFwdArgs a;
-            memset(&a, 0, sizeof(a));
-            a.s = AttnShape{B, N, d.D, d.E, d.F, d.KS};
-            a.q = src_split(s + L.PQ, g.Tq * TC_M, L.KSq, (long long)B * g.Tq * TC_M);
-            a.pm = s + L.PM; a.memory = memory;
-            a.wlc = w->loc_conv_w; a.wldT = packed + PL.wldT; a.v = w->v_w; a.lengths = mem_lengths;
-            a.w_prev = s + L.WPREV; a.cum = s + L.CUM;
-            a.align_out = align_out + (size_t)t * N; a.align_bstride = (long long)max_steps * N;
-            a.ctx_ld = d.E;
-            add_img(a.ctx_bf, xd, d.A, NPAD); add_img(a.ctx_bf, xa_n, d.P, NPAD); add_img(a.ctx_bf, XPI, d.H, NPAD);
-            GVX_TRY(launch_attention_fwd_best(a, st));
-        }
-        {
-            ProfScope ps(PS_DEC_LSTM, st);
-            BfDsts h;
-            memset(&h, 0, sizeof(h));
-            add_img(h, XPI, 0, NPAD); add_img(h, xd_n, d.A + d.E, NPAD);
-            GVX_TRY(run_lstm_bf16(d, packed, 1, WdI, xd, s + L.PD, L.KSd, g.Td, g.Kpd, s + L.CD, s + L.CD, nullptr, h, B, seed, t,
-                                  training, row_offset, err, st));
-        }
+        const float *prev = t == 0 ? s + L.ZERO : s + L.OUT + (size_t)(t - 1) * B * d.OL;
         float *out_t = s + L.OUT + (size_t)t * B * d.OL;
-        {
-            ProfScope ps(PS_PROJ, st);
-            GVX_TRY(run_tc(WpgI, XPI, s + L.PP, g.Tp, g.Kpp, L.KSp, B, err, st));
-            GVX_CUDA(launch_pdl(k_bf_finalize, dim3(grid_for((size_t)B * (d.M + 1))), dim3(256), 0, st, (const float *)(s + L.PP), L.KSp,
-                                B, g.Tp * TC_M, d.M + 1, (const float *)(packed + PL.bpg), out_t, d.OL));
-            GVX_LAUNCHED(1);
-            GVX_CUDA(cudaGetLastError());
-        }
+        GVX_TRY(infer_step_bf16(d, w, packed, L, s, memory, mem_lengths, B, N, seed, t, training, row_offset, nullptr, nullptr, prev,
+                                align_out + (size_t)t * N, (long long)max_steps * N, out_t, st));
         if (!ignore_gate) {
             GVX_CUDA(launch_pdl(k_gate_check, dim3(1), dim3(128), 0, st, (const float *)out_t, B, d.M, d.OL, gate_threshold, t, n_frames, flags));
             GVX_LAUNCHED(1);

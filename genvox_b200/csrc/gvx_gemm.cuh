@@ -67,6 +67,8 @@ struct EpiStore {
     int t0;                // Philox t of the first frame
     int rows_per_frame;    // rows of X per frame (B); row m -> frame m / B, batch row m % B
     int row_offset;
+    // optional per batch row (continuous batching): Philox t = row_frame[brow] instead of t0 + f, row = row_id[brow] + row_offset
+    const int *row_frame, *row_id;
     BfDsts bf;             // optional bf16 copies (bf16 mode), addressed by (frame, batch row, column)
 
     template <int BT, int R>
@@ -82,7 +84,9 @@ struct EpiStore {
             if (add2) v += add2[(size_t)m * ld2 + rr];
             if (mode == 1) {
                 const int f = m / rows_per_frame, brow = m - f * rows_per_frame;
-                v = fmaxf(v, 0.f) * drop_mult(drop, site, (uint32_t)(t0 + f), (uint32_t)(brow + row_offset), (uint32_t)rr);
+                const uint32_t tf = row_frame ? (uint32_t)row_frame[brow] : (uint32_t)(t0 + f);
+                const uint32_t rw = (uint32_t)((row_id ? row_id[brow] : brow) + row_offset);
+                v = fmaxf(v, 0.f) * drop_mult(drop, site, tf, rw, (uint32_t)rr);
             }
             out[(size_t)m * ldo + rr] = v;
             if (bf.n) {

@@ -33,6 +33,7 @@ struct InferPrenetArgs {
     DropCfg drop;                      // p = 0.5, always on
     uint32_t t;
     int row_offset, B, M, P;
+    const int *row_frame, *row_id;     // optional [B] (continuous batching): Philox t and row (before row_offset) per batch row
 };
 
 __global__ void __launch_bounds__(IPN_THREADS, 1) k_infer_prenet(const InferPrenetArgs a) {
@@ -51,6 +52,9 @@ __global__ void __launch_bounds__(IPN_THREADS, 1) k_infer_prenet(const InferPren
     for (int i = tid; i < IPN_COLS * M; i += IPN_THREADS) w0s[i] = a.w0[(size_t)blockIdx.x * IPN_COLS * M + i];
     for (int i = tid; i < IPN_COLS * P; i += IPN_THREADS) w1s[i] = a.w1[(size_t)blockIdx.x * IPN_COLS * P + i];
     pdl_wait();
+    const int rb = b < B ? b : 0;
+    const uint32_t dt = a.row_frame ? (uint32_t)a.row_frame[rb] : a.t;
+    const uint32_t drow = (uint32_t)((a.row_id ? a.row_id[rb] : b) + a.row_offset);
     for (int i = tid; i < IPN_ROWS * M; i += IPN_THREADS) {
         const int r = i / M, k = i - r * M;
         xs[r * ldx0 + k] = r < B ? a.prev[(size_t)r * a.prev_ld + k] : 0.f;
@@ -67,7 +71,7 @@ __global__ void __launch_bounds__(IPN_THREADS, 1) k_infer_prenet(const InferPren
             acc = fmaf(xr[k + 2], w4.z, acc); acc = fmaf(xr[k + 3], w4.w, acc);
         }
         if (b < B)
-            a.pre1[(size_t)b * P + col] = fmaxf(acc, 0.f) * drop_mult(a.drop, SITE_PRENET0, a.t, (uint32_t)(b + a.row_offset), (uint32_t)col);
+            a.pre1[(size_t)b * P + col] = fmaxf(acc, 0.f) * drop_mult(a.drop, SITE_PRENET0, dt, drow, (uint32_t)col);
     }
     // ---- all 32 column slices of the layer-0 output are needed by every CTA
     __syncthreads();
@@ -93,7 +97,7 @@ __global__ void __launch_bounds__(IPN_THREADS, 1) k_infer_prenet(const InferPren
             acc = fmaf(xr[k], w4.x, acc); acc = fmaf(xr[k + 1], w4.y, acc);
             acc = fmaf(xr[k + 2], w4.z, acc); acc = fmaf(xr[k + 3], w4.w, acc);
         }
-        const float v = fmaxf(acc, 0.f) * drop_mult(a.drop, SITE_PRENET1, a.t, (uint32_t)(b + a.row_offset), (uint32_t)col);
+        const float v = fmaxf(acc, 0.f) * drop_mult(a.drop, SITE_PRENET1, dt, drow, (uint32_t)col);
         if (b < B && a.pre2) a.pre2[(size_t)b * P + col] = v;
         tile[b * IPN_COLS + c] = v;
     }
@@ -117,9 +121,11 @@ inline bool infer_prenet_fused_ok(const Dims &d, int B) {
     return on == 1 && B <= IPN_ROWS && d.M % 4 == 0 && d.M <= d.P && d.P % IPN_COLS == 0 && d.P / IPN_COLS <= 64;
 }
 
-// prev -> PRE2 (fp32, optional) and/or bf16 images; `bar` = monotonic counter zeroed before step 0, t = step index
+// prev -> PRE2 (fp32, optional) and/or bf16 images; `bar` = monotonic counter zeroed before step 0, t = step index.
+// row_frame / row_id (optional, device [B]): per-row Philox t and row (before row_offset) in place of t and the batch row.
 inline int run_infer_prenet(const Dims &d, const gvx_weights *w, const float *prev, int prev_ld, int B, uint64_t seed, int t,
-                            int row_offset, float *pre1, float *pre2, const BfDsts *bf, unsigned *bar, int *err, cudaStream_t st) {
+                            int row_offset, float *pre1, float *pre2, const BfDsts *bf, unsigned *bar, int *err, cudaStream_t st,
+                            const int *row_frame = nullptr, const int *row_id = nullptr) {
     InferPrenetArgs a;
     memset(&a, 0, sizeof(a));
     a.prev = prev; a.prev_ld = prev_ld; a.w0 = w->prenet_w0; a.w1 = w->prenet_w1;
@@ -129,6 +135,7 @@ inline int run_infer_prenet(const Dims &d, const gvx_weights *w, const float *pr
     a.bar = bar; a.target = (unsigned)grid * (unsigned)(t + 1); a.err = err;
     a.drop = make_drop(seed, 0.5f, 1);
     a.t = (uint32_t)t; a.row_offset = row_offset; a.B = B; a.M = d.M; a.P = d.P;
+    a.row_frame = row_frame; a.row_id = row_id;
     const size_t smem = ((size_t)((IPN_COLS * d.M + 3) & ~3) + (size_t)IPN_COLS * d.P + (size_t)IPN_ROWS * (d.P + 1) + IPN_ROWS * IPN_COLS) * sizeof(float);
     static size_t configured = 0;
     if (smem > configured) {

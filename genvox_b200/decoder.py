@@ -121,6 +121,7 @@ class Decoder(nn.Module):
         self._forced_seed = None
         self.last_dropout_seed = None
         self.last_n_frames = None
+        self.last_steps_run = None      # decoder steps of the last inference_continuous call
         self._pack_key = None
         self._packed = None
         self._pack_epoch = 0          # bumped by invalidate_packed()
@@ -233,6 +234,63 @@ class Decoder(nn.Module):
         if not ignore_gate and tmax >= steps and int(ran.value) >= steps and not self._last_step_gate_fired(gate, n_frames, steps):
             print("Warning! Reached max decoder steps")      # tacotron2.py:408
         return mel[:, :, :tmax], gate[:, :tmax], align[:, :tmax]
+
+    @torch.no_grad()
+    def inference_continuous(self, memory, memory_lengths, slots=64, max_decoder_steps=None, frame_caps=None, ignore_gate=False,
+                             return_alignments=True):
+        """Continuous batching: decode the U utterances of `memory` [U,N,E] through `slots` decoder rows; a row whose utterance
+        stops takes the next one of the queue on the device (include/genvox_b200.h, gvx_dec_infer_continuous).  Utterance u
+        stops at its first gate over the threshold or after min(max_decoder_steps, frame_caps[u]) frames, and draws the prenet
+        dropout of row u + dropout_row_offset.  Returns (mel [U,n_mels,Tmax], gate [U,Tmax], alignments [U,Tmax,N] or None)
+        with Tmax = max over utterances of the frame count; frames past an utterance's count are zero.  The counts are left
+        in `self.last_n_frames` (int32 [U], device).  Eval mode only."""
+        lib = _native.load()
+        steps = int(max_decoder_steps if max_decoder_steps is not None else self.max_decoder_steps)
+        if self.training:
+            raise RuntimeError("genvox_b200: inference_continuous runs in eval mode only (call .eval())")
+        limit = 128 if self.precision == "bf16" else None
+        if int(slots) < 1 or (limit is not None and int(slots) > limit):
+            raise ValueError(f"genvox_b200: slots must be in 1 .. {limit or 'inf'} in {self.precision} mode, got {slots}")
+        if steps < 1:
+            raise ValueError(f"genvox_b200: max_decoder_steps must be positive, got {steps}")
+        caps = None
+        if frame_caps is not None:
+            caps = torch.as_tensor(frame_caps).reshape(-1)
+            if caps.numel() != memory.shape[0]:
+                raise ValueError(f"genvox_b200: frame_caps needs one entry per utterance ({memory.shape[0]}), got {caps.numel()}")
+            if bool((caps < 1).any()) or bool((caps > steps).any()):
+                raise ValueError(f"genvox_b200: frame_caps must lie in 1 .. max_decoder_steps ({steps})")
+        memory = _f32c(memory, "memory")
+        U, N, _ = memory.shape
+        dev = memory.device
+        lengths = None
+        if memory_lengths is not None:
+            lengths = memory_lengths.to(device=dev, dtype=torch.int64).contiguous()
+        if caps is not None:
+            caps = caps.to(device=dev, dtype=torch.int32).contiguous()
+        params = [p.detach() for p in self._ordered_params()]
+        dims, weights, packed = self._native_state(params)
+        mel = torch.zeros(U, self.n_mel_channels, steps, device=dev, dtype=torch.float32)
+        gate = torch.zeros(U, steps, device=dev, dtype=torch.float32)
+        align = torch.zeros(U, steps, N, device=dev, dtype=torch.float32) if return_alignments else None
+        n_frames = torch.empty(U, device=dev, dtype=torch.int32)
+        nbytes = lib.gvx_dec_infer_continuous_workspace_bytes(C.byref(dims), U, N, int(slots))
+        if nbytes == 0:
+            _native.check(1, "gvx_dec_infer_continuous_workspace_bytes")
+        work = _buffer(nbytes, dev)
+        ran = C.c_longlong(0)
+        _native.check(lib.gvx_dec_infer_continuous(C.byref(dims), C.byref(weights), _ptr(packed), _ptr(memory), _ptr(lengths), U, N,
+                                                   int(slots), steps, _ptr(caps), float(self.gate_threshold), int(bool(ignore_gate)),
+                                                   self._next_seed(), self.dropout_row_offset, _ptr(mel), _ptr(gate), _ptr(align),
+                                                   _ptr(n_frames), C.byref(ran), _ptr(work), _stream()),
+                      "gvx_dec_infer_continuous")
+        self.last_n_frames = n_frames
+        self.last_steps_run = int(ran.value)
+        tmax = int(n_frames.max().item())
+        # as in inference(): an utterance that reached the last allowed step warns unless its gate fired there
+        if not ignore_gate and tmax >= steps and not self._last_step_gate_fired(gate, n_frames, steps):
+            print("Warning! Reached max decoder steps")      # tacotron2.py:408
+        return mel[:, :, :tmax], gate[:, :tmax], (align[:, :tmax] if align is not None else None)
 
 
 def decoder_kwargs_from(ref_decoder):

@@ -14,7 +14,9 @@ the batch is built AROUND it while everything that is not row-independent in the
 `batched_inference(model, token_rows)` therefore returns, for every utterance, exactly the dictionary
 `Tacotron2.inference` returns for it alone (same keys, leading batch dimension of 1), up to fp32 rounding of the
 decoder (the token split over the two CTAs of a row depends on the padded length).  `sharded_inference` is the
-multi-GPU form: utterances are sharded over ranks, no collective (BASELINE configs[3]).
+multi-GPU form: utterances are sharded over ranks, no collective (BASELINE configs[3]).  `continuous_inference` returns
+the same dictionaries from one continuous-batching call (`Decoder.inference_continuous`): a decoder row whose utterance
+stops takes the next utterance of the queue instead of idling until its batch ends.
 """
 import torch
 
@@ -73,3 +75,34 @@ def sharded_inference(model, token_rows, rank, world, **kwargs):
     """Utterances [lo, hi) of `token_rows` on this rank (contiguous shards, no collective).  Returns (lo, outputs)."""
     lo, hi = shard_rows(len(token_rows), rank, world)
     return lo, batched_inference(model, token_rows[lo:hi], **kwargs)
+
+
+@torch.no_grad()
+def continuous_inference(model, token_rows, slots=64, **kw):
+    """Like `batched_inference`, but the decoder runs every utterance in one `Decoder.inference_continuous` call through
+    `slots` rows, in the order given (utterance i draws prenet dropout row i + dropout_row_offset).  `kw` goes to
+    `inference_continuous` (max_decoder_steps, frame_caps, ignore_gate, return_alignments); "alignments" is None when
+    alignments are not returned."""
+    dev = next(model.parameters()).device
+    rows = _as_rows(token_rows, dev)
+    enc = []
+    for r in rows:      # Encoder.inference per utterance (tacotron2.py:486-487), outputs zero-padded to the longest
+        emb = model.embedding(r.unsqueeze(0)).transpose(1, 2)
+        enc.append(model.encoder.inference(emb))
+    lengths = torch.tensor([e.shape[1] for e in enc], dtype=torch.int64, device=dev)
+    memory = torch.zeros(len(rows), int(lengths.max()), enc[0].shape[2], dtype=torch.float32, device=dev)
+    for i, e in enumerate(enc):
+        memory[i, :e.shape[1]] = e[0]
+    mel, gate, align = model.decoder.inference_continuous(memory, lengths, slots=slots, **kw)
+    n_frames = model.decoder.last_n_frames.tolist()
+    out = []
+    for i in range(len(rows)):
+        t_i, n_i = int(n_frames[i]), int(lengths[i])
+        m = mel[i:i + 1, :, :t_i].contiguous()
+        out.append({
+            "mel_outputs": m,
+            "mel_outputs_postnet": m + model.postnet(m),     # tacotron2.py:490-491
+            "gate_outputs": gate[i:i + 1, :t_i].contiguous(),
+            "alignments": align[i:i + 1, :t_i, :n_i].contiguous() if align is not None else None,
+        })
+    return out

@@ -167,6 +167,26 @@ int gvx_dec_infer(const gvx_dims *d, const gvx_weights *w, const void *packed,
                   float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
                   int *steps_run, void *workspace, void *stream);
 
+/* Continuous batching: decode a queue of U utterances (all padded to N tokens) through `slots` decoder rows.  Slots start
+ * with utterances 0 .. slots-1; when a slot's utterance stops, the slot takes the next utterance of the queue on the device
+ * before the next decoder step (slots stopping in the same step take them in slot order), with its recurrent state zeroed.
+ * Utterance u stops at the first frame whose sigmoid(gate) > gate_threshold (as gvx_dec_infer; not with ignore_gate) or
+ * after cap[u] = min(max_steps, frame_caps[u]) frames.  Its prenet dropout at local frame f draws Philox row
+ * u + row_offset, t = f.  Eval mode only (no LSTM-state dropout).  bf16 mode: slots <= 128.
+ * Output identity: utterance u's frames 0 .. n_frames[u]-1 are bit-identical to row r of a gvx_dec_infer call with the same
+ * slots rows, N, seed and precision, u in row r and row_offset' = u + row_offset - r; n_frames[u] is that row's stop step.
+ *   memory [U, N, E]; mem_lengths [U] int64 or NULL; frame_caps [U] int32 or NULL
+ *   mel_out [U, n_mels, max_steps], gate_out [U, max_steps], align_out [U, max_steps, N] or NULL, n_frames [U] int32
+ *   *steps_run (host) = decoder steps executed (at most ceil(U / slots) * max_steps)
+ * Only frames 0 .. n_frames[u]-1 of the outputs are written. */
+size_t gvx_dec_infer_continuous_workspace_bytes(const gvx_dims *d, int U, int N, int slots);
+int gvx_dec_infer_continuous(const gvx_dims *d, const gvx_weights *w, const void *packed,
+                             const float *memory, const int64_t *mem_lengths, int U, int N, int slots,
+                             int max_steps, const int32_t *frame_caps, float gate_threshold, int ignore_gate,
+                             uint64_t seed, int row_offset,
+                             float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
+                             long long *steps_run, void *workspace, void *stream);
+
 /* ---- single-phase entry points (used by the parity tests to localise a failure) ---- */
 
 /* The tcgen05 / TMEM / TMA gate-GEMM engine on its own: out[B, Mtot] = X[B, K] . W[Mtot, K]^T with both
