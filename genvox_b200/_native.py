@@ -47,6 +47,14 @@ class GvxGrads(C.Structure):
     _fields_ = [(f, _P) for f, _ in PARAM_FIELDS]
 
 
+class GvxSession(C.Structure):
+    _fields_ = [("N", C.c_int32), ("slots", C.c_int32), ("capacity", C.c_int32), ("max_steps", C.c_int32),
+                ("ignore_gate", C.c_int32), ("with_alignments", C.c_int32), ("row_offset", C.c_int32),
+                ("gate_threshold", C.c_float), ("seed", C.c_uint64), ("steps_run", C.c_longlong), ("submitted", C.c_longlong),
+                ("admitted", C.c_longlong), ("finished", C.c_longlong), ("active", C.c_int32), ("parity", C.c_int32),
+                ("ready", C.c_int32)]
+
+
 _SIGNATURES = {
     "gvx_abi_version": (C.c_int, []),
     "gvx_last_error": (C.c_char_p, []),
@@ -73,6 +81,12 @@ _SIGNATURES = {
     "gvx_dec_infer_continuous": (C.c_int, [C.POINTER(GvxDims), C.POINTER(GvxWeights), _P, _P, _P, C.c_int, C.c_int, C.c_int,
                                            C.c_int, _P, C.c_float, C.c_int, C.c_uint64, C.c_int, _P, _P, _P, _P,
                                            C.POINTER(C.c_longlong), _P, _P]),
+    "gvx_dec_session_workspace_bytes": (C.c_size_t, [C.POINTER(GvxDims), C.c_int, C.c_int, C.c_int]),
+    "gvx_dec_session_init": (C.c_int, [C.POINTER(GvxDims), C.POINTER(GvxSession), _P, _P]),
+    "gvx_dec_session_submit": (C.c_int, [C.POINTER(GvxDims), C.POINTER(GvxWeights), _P, C.POINTER(GvxSession), _P, _P, _P,
+                                         C.c_int, _P, _P]),
+    "gvx_dec_session_step": (C.c_int, [C.POINTER(GvxDims), C.POINTER(GvxWeights), _P, C.POINTER(GvxSession), C.c_int,
+                                       _P, _P, _P, _P, _P, C.POINTER(C.c_int), _P, _P]),
     "gvx_test_tc_gemm": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
     "gvx_test_nt_gemm": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
     "gvx_bench_nt_gemm": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float)]),

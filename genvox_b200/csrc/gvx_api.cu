@@ -627,3 +627,4 @@ int gvx_attention_step(const gvx_dims *dd, const gvx_weights *w, const void *pac
 #include "gvx_bwd.cuh"
 #include "gvx_bf16_api.cuh"
 #include "gvx_continuous.cuh"
+#include "gvx_session.cuh"

@@ -39,16 +39,26 @@ constexpr int ADMIT_MAXI = 5;
 struct AdmitArgs {
     float *out_t;                      // [S][OL] this step's [mel | gate] rows: the previous frame of the next step
     const float *align_t;              // [S][N] this step's attention weights
-    const float *memory, *pmq;         // [U][N][E], [Upad][N][D]
-    const int64_t *lengths;            // [U] or null (all N)
-    const int32_t *caps;               // [U] or null
+    const float *memory, *pmq;         // queue entry q at q (cap = 0) or q % cap: [..][N][E], [..][N][D]
+    const int64_t *lengths;            // per queue entry, or null (all N)
+    const int32_t *caps;               // per queue entry, or null
     float *mem_slot, *pm_slot;         // [S][N][E], [S][N][D]
     int64_t *len_slot;                 // [S]
     const int *utt_cur, *frame_cur, *next_cur;
     int *utt_nxt, *frame_nxt, *next_nxt;
-    float *mel_out, *gate_out, *align_out;
+    // session: each slot's frame cap, copied in at admission (a ring entry can be reused while its utterance still runs)
+    const int *cap_cur;
+    int *cap_nxt;
+    float *mel_out, *gate_out, *align_out;   // per-utterance outputs [U][..][max_steps] (continuous call)
     int32_t *n_frames;
-    int *flags;                        // [0] active slots after this step
+    // per-call chunk outputs of a session, used instead of the per-utterance ones when ch_utt is set: row [step][slot]
+    float *ch_frames, *ch_align;       // [steps][S][M+1], [steps][S][N] or null
+    int32_t *ch_utt, *ch_frame;        // [steps][S] utterance (-1: idle) and its local frame
+    int8_t *ch_last;                   // [steps][S] 1 on the utterance's last frame
+    int step;
+    int *flags;                        // [0] active slots after this step; sessions (cap > 0): [1] admission head, [2] += stops
+    unsigned *bar;                     // head mode: the fused prenet's grid-barrier counter, set to bar_value (or null)
+    unsigned bar_value;
     float *zero[ADMIT_MAXZ];           // per-row fp32 state, row s at zero[i] + s * zero_w[i]
     int zero_w[ADMIT_MAXZ];
     int nzero;
@@ -56,13 +66,17 @@ struct AdmitArgs {
     int img_k[ADMIT_MAXI];
     int nimg, npad;
     float thr;
-    int ignore_gate, S, U, N, E, D, M, OL, max_steps;
+    int ignore_gate, S, N, E, D, M, OL, max_steps;
+    int U;                             // queue entries q < U exist (a session passes its submitted count)
+    int cap;                           // session ring capacity; 0: the queue is a plain array
+    int head;                          // 1: admit into idle slots only, before the first step of a session call (no frame)
 };
 
 // stop test of gvx_dec_infer (tacotron2.py:405: sigmoid(gate) > threshold, strict, frame included) or the frame cap
 __device__ __forceinline__ bool slot_stops(const AdmitArgs &a, int j, int u, int f) {
     int cap = a.max_steps;
-    if (a.caps) cap = min(cap, max(1, (int)a.caps[u]));
+    if (a.cap_cur) cap = min(cap, a.cap_cur[j]);
+    else if (a.caps) cap = min(cap, max(1, (int)a.caps[u]));
     if (f + 1 >= cap) return true;
     return !a.ignore_gate && sigmoidf_(a.out_t[(size_t)j * a.OL + a.M]) > a.thr;
 }
@@ -78,29 +92,44 @@ __device__ void copy_rows(float *__restrict__ dst, const float *__restrict__ src
     }
 }
 
-// one CTA per slot
+// one CTA per slot.  Step mode: write the slot's frame, apply the stop test, and let the slots that stop take queue entries.
+// Head mode: no step ran; the idle slots take queue entries.  Either way the freed slots take entries next, next + 1, ...
+// in slot order, and every CTA recomputes all S decisions to find its own prefix count.
 __global__ void __launch_bounds__(ADMIT_THREADS) k_gate_admit(const AdmitArgs a) {
     pdl_trigger();
     pdl_wait();
     const int me = blockIdx.x, tid = threadIdx.x;
     const int next = a.next_cur[0];
-    int n_stop = 0, n_before = 0, n_active = 0;
+    int n_free = 0, n_before = 0, n_active = 0;
     for (int base = 0; base < a.S; base += blockDim.x) {
         const int j = base + tid;
-        bool act = false, stop = false;
+        bool act = false, fr = false;
         if (j < a.S) {
             const int u = a.utt_cur[j];
             act = u >= 0;
-            stop = act && slot_stops(a, j, u, a.frame_cur[j]);
+            fr = a.head ? !act : act && slot_stops(a, j, u, a.frame_cur[j]);
         }
-        n_stop += __syncthreads_count(stop);
-        n_before += __syncthreads_count(stop && j < me);
+        n_free += __syncthreads_count(fr);
+        n_before += __syncthreads_count(fr && j < me);
         n_active += __syncthreads_count(act);
     }
     const int u = a.utt_cur[me], f = a.frame_cur[me];
-    const bool stop = u >= 0 && slot_stops(a, me, u, f);
-    // 1. the slot's frame f of utterance u
-    if (u >= 0) {
+    const bool stop = !a.head && u >= 0 && slot_stops(a, me, u, f);
+    const int n_stop = a.head ? 0 : n_free;
+    if (!a.head && a.ch_utt) {
+        // 1. (session) the slot's row of this step in the chunk buffers
+        const size_t k = (size_t)a.step * a.S + me;
+        if (tid == 0) { a.ch_utt[k] = u; a.ch_frame[k] = u >= 0 ? f : 0; a.ch_last[k] = stop ? 1 : 0; }
+        if (u >= 0) {
+            const float *row = a.out_t + (size_t)me * a.OL;
+            for (int m = tid; m <= a.M; m += blockDim.x) a.ch_frames[k * (a.M + 1) + m] = row[m];
+            if (a.ch_align) {
+                const float *al = a.align_t + (size_t)me * a.N;
+                for (int n = tid; n < a.N; n += blockDim.x) a.ch_align[k * a.N + n] = al[n];
+            }
+        }
+    } else if (!a.head && u >= 0) {
+        // 1. the slot's frame f of utterance u
         const float *row = a.out_t + (size_t)me * a.OL;
         for (int m = tid; m < a.M; m += blockDim.x) a.mel_out[((size_t)u * a.M + m) * a.max_steps + f] = row[m];
         if (tid == 0) a.gate_out[(size_t)u * a.max_steps + f] = row[a.M];
@@ -112,17 +141,19 @@ __global__ void __launch_bounds__(ADMIT_THREADS) k_gate_admit(const AdmitArgs a)
         // 2. its frame count
         if (stop && tid == 0) a.n_frames[u] = f + 1;
     }
-    // 3. admission: the slots stopping in this step take queue entries next, next + 1, ... in slot order
-    int nu = u, nf = f + 1;
-    if (stop) {
+    // 3. admission
+    int nu = u, nf = a.head ? f : f + 1, ncap = a.cap_cur ? a.cap_cur[me] : 0;
+    if (a.head ? u < 0 : stop) {
         const int q = next + n_before;
         nu = q < a.U ? q : -1;
         nf = 0;
         if (nu >= 0) {
+            const size_t e = a.cap ? (size_t)(q % a.cap) : (size_t)q;
             __syncthreads();           // the output row read above is zeroed below
-            copy_rows(a.mem_slot + (size_t)me * a.N * a.E, a.memory + (size_t)q * a.N * a.E, (size_t)a.N * a.E);
-            copy_rows(a.pm_slot + (size_t)me * a.N * a.D, a.pmq + (size_t)q * a.N * a.D, (size_t)a.N * a.D);
-            if (tid == 0) a.len_slot[me] = a.lengths ? a.lengths[q] : (int64_t)a.N;
+            copy_rows(a.mem_slot + (size_t)me * a.N * a.E, a.memory + e * a.N * a.E, (size_t)a.N * a.E);
+            copy_rows(a.pm_slot + (size_t)me * a.N * a.D, a.pmq + e * a.N * a.D, (size_t)a.N * a.D);
+            if (tid == 0) a.len_slot[me] = a.lengths ? a.lengths[e] : (int64_t)a.N;
+            ncap = a.caps ? max(1, (int)a.caps[e]) : a.max_steps;
             // the go frame: only the mel columns, the gate column of every slot is read by every CTA
             for (int m = tid; m < a.M; m += blockDim.x) a.out_t[(size_t)me * a.OL + m] = 0.f;
             for (int z = 0; z < a.nzero; ++z) {
@@ -138,11 +169,14 @@ __global__ void __launch_bounds__(ADMIT_THREADS) k_gate_admit(const AdmitArgs a)
     if (tid == 0) {
         a.utt_nxt[me] = nu;
         a.frame_nxt[me] = nu >= 0 ? nf : 0;
+        if (a.cap_nxt) a.cap_nxt[me] = ncap;
         if (me == 0) {
             // 4. active slots after this step, for the host poll
-            const int admitted = min(n_stop, max(0, a.U - next));
+            const int admitted = min(n_free, max(0, a.U - next));
             a.next_nxt[0] = next + admitted;
             a.flags[0] = n_active - n_stop + admitted;
+            if (a.cap) { a.flags[1] = next + admitted; a.flags[2] += n_stop; }
+            if (a.bar) *a.bar = a.bar_value;
         }
     }
 }
@@ -160,6 +194,26 @@ __global__ void k_slot_start(int S, int U, int N, const int64_t *__restrict__ le
 
 inline size_t continuous_base(const Dims &d, bool bf, int S, int N) {
     return bf ? InferBfL(d, S, N, 2).total : InferL(d, S, N, 2).total;
+}
+
+// the per-row recurrent state an admission zeroes, in the layout it lives in: fp32 h/c of both LSTMs, ctx, attention weights
+// and cumulative weights; in bf16 mode the cell states, attention weights and the slot's rows of the tcgen05 operand images
+inline void admit_state(AdmitArgs &a, const Dims &d, bool bf, const InferL &Lf, const InferBfL &Lb, float *s, int S, int N) {
+    auto zrow = [&](float *p, int width) { a.zero[a.nzero] = p; a.zero_w[a.nzero] = width; ++a.nzero; };
+    if (bf) {
+        const BfGeom g(d);
+        zrow(s + Lb.CA, d.A); zrow(s + Lb.CD, d.H); zrow(s + Lb.WPREV, N); zrow(s + Lb.CUM, N);
+        bf16 *XAI = (bf16 *)(s + Lb.XAI), *XDI = (bf16 *)(s + Lb.XDI);
+        a.img[0] = XAI; a.img[1] = XAI + Lb.xai_stride; a.img_k[0] = a.img_k[1] = g.Kpa;
+        a.img[2] = XDI; a.img[3] = XDI + Lb.xdi_stride; a.img_k[2] = a.img_k[3] = g.Kpd;
+        a.img[4] = (bf16 *)(s + Lb.XPI); a.img_k[4] = g.Kpp;
+        a.nimg = 5;
+        a.npad = Lb.NPAD;
+    } else {
+        zrow(s + Lf.HA, d.A); zrow(s + Lf.HA + (size_t)S * d.A, d.A); zrow(s + Lf.CA, d.A);
+        zrow(s + Lf.HD, d.H); zrow(s + Lf.HD + (size_t)S * d.H, d.H); zrow(s + Lf.CD, d.H);
+        zrow(s + Lf.CTX, d.E); zrow(s + Lf.WPREV, N); zrow(s + Lf.CUM, N);
+    }
 }
 
 int infer_continuous(const gvx_dims *dd, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
@@ -203,24 +257,13 @@ int infer_continuous(const gvx_dims *dd, const gvx_weights *w, const float *pack
     // recurrent state: zero at the start, and per row at every admission (k_gate_admit)
     AdmitArgs a;
     memset(&a, 0, sizeof(a));
-    auto zrow = [&](float *p, int width) { a.zero[a.nzero] = p; a.zero_w[a.nzero] = width; ++a.nzero; };
+    admit_state(a, d, bf, Lf, Lb, s, S, N);
     if (bf) {
         const BfGeom g(d);
-        zrow(s + Lb.CA, d.A); zrow(s + Lb.CD, d.H); zrow(s + Lb.WPREV, N); zrow(s + Lb.CUM, N);
-        bf16 *XAI = (bf16 *)(s + Lb.XAI), *XDI = (bf16 *)(s + Lb.XDI);
-        a.img[0] = XAI; a.img[1] = XAI + Lb.xai_stride; a.img_k[0] = a.img_k[1] = g.Kpa;
-        a.img[2] = XDI; a.img[3] = XDI + Lb.xdi_stride; a.img_k[2] = a.img_k[3] = g.Kpd;
-        a.img[4] = (bf16 *)(s + Lb.XPI); a.img_k[4] = g.Kpp;
-        a.nimg = 5;
-        a.npad = Lb.NPAD;
         GVX_CUDA(cudaMemsetAsync(s + Lb.ERR, 0, 64 * sizeof(float), st));
         GVX_CUDA(cudaMemsetAsync(a.img[0], 0, 2 * Lb.xai_stride * sizeof(bf16), st));
         GVX_CUDA(cudaMemsetAsync(a.img[2], 0, 2 * Lb.xdi_stride * sizeof(bf16), st));
         GVX_CUDA(cudaMemsetAsync(a.img[4], 0, (size_t)g.Kpp * Lb.NPAD * sizeof(bf16), st));
-    } else {
-        zrow(s + Lf.HA, d.A); zrow(s + Lf.HA + (size_t)S * d.A, d.A); zrow(s + Lf.CA, d.A);
-        zrow(s + Lf.HD, d.H); zrow(s + Lf.HD + (size_t)S * d.H, d.H); zrow(s + Lf.CD, d.H);
-        zrow(s + Lf.CTX, d.E); zrow(s + Lf.WPREV, N); zrow(s + Lf.CUM, N);
     }
     for (int z = 0; z < a.nzero; ++z) GVX_CUDA(cudaMemsetAsync(a.zero[z], 0, (size_t)S * a.zero_w[z] * sizeof(float), st));
     GVX_CUDA(cudaMemsetAsync(s + OUT, 0, (size_t)2 * S * d.OL * sizeof(float), st));     // the previous-frame ring: go frames

@@ -168,6 +168,10 @@ class Decoder(nn.Module):
             return True
         return bool((torch.sigmoid(gate[rows, steps - 1]) > self.gate_threshold).all())
 
+    def _packed_key(self, params):
+        """cache key of the packed weights: precision, invalidate_packed() epoch, (data_ptr, version) per parameter"""
+        return (self.precision, self._pack_epoch) + tuple((p.data_ptr(), p._version) for p in params)
+
     def _native_state(self, params):
         """(dims, weights struct, packed weights) — repacks when any parameter changed."""
         lib = _native.load()
@@ -176,7 +180,7 @@ class Decoder(nn.Module):
                 raise RuntimeError("genvox_b200: decoder parameters must be contiguous float32 CUDA tensors")
         dims = self._dims()
         weights = self._weights_struct(params)
-        key = (self.precision, self._pack_epoch) + tuple((p.data_ptr(), p._version) for p in params)
+        key = self._packed_key(params)
         if key != self._pack_key:
             nbytes = lib.gvx_dec_packed_bytes(C.byref(dims))
             if nbytes == 0:
@@ -291,6 +295,16 @@ class Decoder(nn.Module):
         if not ignore_gate and tmax >= steps and not self._last_step_gate_fired(gate, n_frames, steps):
             print("Warning! Reached max decoder steps")      # tacotron2.py:408
         return mel[:, :, :tmax], gate[:, :tmax], (align[:, :tmax] if align is not None else None)
+
+    def session(self, N, slots=64, capacity=1024, max_decoder_steps=None, ignore_gate=False, return_alignments=True):
+        """A decoder session (genvox_b200.session.DecoderSession): `slots` decoder rows kept alive between calls, utterances
+        of up to N tokens submitted at any time between calls and decoded through those rows, frames returned per step call.
+        Up to `capacity` utterances may wait in its queue.  Utterance `id` decodes bit-identically to row r of a static
+        `inference` call with the same slots rows, N, seed and precision, id in row r and dropout_row_offset =
+        id + dropout_row_offset - r.  Eval mode only; the parameters must not change while the session runs."""
+        from .session import DecoderSession
+        return DecoderSession(self, N, slots=slots, capacity=capacity, max_decoder_steps=max_decoder_steps,
+                              ignore_gate=ignore_gate, return_alignments=return_alignments)
 
 
 def decoder_kwargs_from(ref_decoder):

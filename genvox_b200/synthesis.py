@@ -16,7 +16,9 @@ the batch is built AROUND it while everything that is not row-independent in the
 decoder (the token split over the two CTAs of a row depends on the padded length).  `sharded_inference` is the
 multi-GPU form: utterances are sharded over ranks, no collective (BASELINE configs[3]).  `continuous_inference` returns
 the same dictionaries from one continuous-batching call (`Decoder.inference_continuous`): a decoder row whose utterance
-stops takes the next utterance of the queue instead of idling until its batch ends.
+stops takes the next utterance of the queue instead of idling until its batch ends.  `SynthesisSession` is the serving
+form (`Decoder.session`): token rows are submitted whenever they arrive, and each `step` returns partial mel chunks and,
+for every utterance that finished, the same dictionary.
 """
 import torch
 
@@ -106,3 +108,64 @@ def continuous_inference(model, token_rows, slots=64, **kw):
             "alignments": align[i:i + 1, :t_i, :n_i].contiguous() if align is not None else None,
         })
     return out
+
+
+class SynthesisSession:
+    """Continuous synthesis for requests that arrive over time, around a decoder session (`Decoder.session`) of
+    `max_tokens` tokens per utterance and `slots` decoder rows; `kw` goes to `Decoder.session` (capacity,
+    max_decoder_steps, ignore_gate, return_alignments).  Utterance `id` draws prenet dropout row id + dropout_row_offset,
+    so with the same N (= max_tokens) and seed its dictionary equals `continuous_inference`'s for the same token rows."""
+
+    def __init__(self, model, max_tokens, slots=64, **kw):
+        self.model = model
+        self.session = model.decoder.session(max_tokens, slots=slots, **kw)
+        self._device = next(model.parameters()).device
+        self._parts = {}        # id -> (n_tokens, [(mel, gate, align)] chunks so far)
+
+    @torch.no_grad()
+    def submit(self, token_rows):
+        """Runs the embedding and `Encoder.inference` per utterance (tacotron2.py:486-487) and queues the outputs.
+        Returns the ids."""
+        rows = _as_rows(token_rows, self._device)
+        if not rows:
+            return []
+        enc = []
+        for r in rows:
+            if r.numel() > self.session.N:
+                raise ValueError(f"genvox_b200.synthesis: {r.numel()} tokens, more than the session's {self.session.N}")
+            emb = self.model.embedding(r.unsqueeze(0)).transpose(1, 2)
+            enc.append(self.model.encoder.inference(emb))
+        lengths = torch.tensor([e.shape[1] for e in enc], dtype=torch.int64, device=self._device)
+        memory = torch.zeros(len(rows), self.session.N, enc[0].shape[2], dtype=torch.float32, device=self._device)
+        for i, e in enumerate(enc):
+            memory[i, :e.shape[1]] = e[0]
+        ids = self.session.submit(memory, lengths)
+        for i, n in zip(ids, lengths.tolist()):
+            self._parts[i] = (n, [])
+        return ids
+
+    @torch.no_grad()
+    def step(self, steps=16):
+        """Runs up to `steps` decoder steps.  Returns (chunks, finished): chunks = {id: mel [1, n_mels, j]} with the new
+        frames of every utterance that advanced; finished = {id: dict with the keys of Tacotron2.inference}, as
+        `continuous_inference` returns it.  The postnet runs once an utterance has finished: its convolutions see the
+        whole utterance."""
+        new, done = self.session.step(steps)
+        chunks = {}
+        for i, part in new.items():
+            self._parts[i][1].append(part)
+            chunks[i] = part[0].unsqueeze(0)
+        finished = {}
+        for i in done:
+            n_tok, parts = self._parts.pop(i)
+            m = torch.cat([p[0] for p in parts], dim=1).unsqueeze(0).contiguous()
+            align = None
+            if self.session.return_alignments:
+                align = torch.cat([p[2] for p in parts], dim=0)[:, :n_tok].unsqueeze(0).contiguous()
+            finished[i] = {
+                "mel_outputs": m,
+                "mel_outputs_postnet": m + self.model.postnet(m),     # tacotron2.py:490-491
+                "gate_outputs": torch.cat([p[1] for p in parts]).unsqueeze(0).contiguous(),
+                "alignments": align,
+            }
+        return chunks, finished

@@ -187,6 +187,55 @@ int gvx_dec_infer_continuous(const gvx_dims *d, const gvx_weights *w, const void
                              float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
                              long long *steps_run, void *workspace, void *stream);
 
+/* Decoder sessions: continuous batching for requests that arrive over time.  A session holds `slots` decoder rows and their
+ * recurrent state in a caller-owned workspace, plus a ring of `capacity` queued utterances (all padded to N tokens).  The
+ * caller submits utterances between calls (ids 0, 1, 2, ... in submission order) and steps the session for up to k decoder
+ * steps at a time: at the head of a step call the idle slots take queued utterances in slot order; during the call a slot
+ * whose utterance stops takes the next queued one on the device, as in gvx_dec_infer_continuous.  Every step call returns
+ * the frames it decoded, tagged per (step, slot).  The session is this struct plus the workspace: the library keeps no
+ * device memory across calls, and both are used on one stream.  Eval mode only.  bf16 mode: slots <= 128.
+ * Output identity: utterance `id` decodes bit-identically to row r of a gvx_dec_infer call with the same slots rows, N,
+ * seed and precision, id in row r and row_offset' = id + row_offset - r, whatever the submission times, the step counts per
+ * call and the other slots were; its frame count is that row's stop step (as gvx_dec_infer_continuous, with frame cap
+ * min(max_steps, frame_caps[id])). */
+typedef struct gvx_session {
+    /* set by the caller before gvx_dec_session_init */
+    int32_t N, slots, capacity, max_steps, ignore_gate, with_alignments, row_offset;
+    float gate_threshold;
+    uint64_t seed;
+    /* maintained by the library */
+    long long steps_run;   /* decoder steps run over the session's life */
+    long long submitted;   /* utterances submitted = the next id */
+    long long admitted;    /* utterances taken into a slot, read back at the end of each step call */
+    long long finished;    /* utterances whose last frame was returned, read back at the end of each step call */
+    int32_t active;        /* slots holding an utterance, read back at the end of each step call */
+    int32_t parity;        /* which half of the workspace's slot-state ping-pong is current */
+    int32_t ready;         /* set by gvx_dec_session_init */
+} gvx_session;
+
+/* Workspace bytes of a session; 0 for bad dims, N, slots or capacity, or bf16 with slots > 128.  It grows by
+ * N * (enc_dim + att_dim) * 4 + 12 bytes per ring entry. */
+size_t gvx_dec_session_workspace_bytes(const gvx_dims *d, int N, int slots, int capacity);
+/* Checks the caller-set fields of *s, zeroes the workspace (every slot idle), stores the seed and resets the counters. */
+int gvx_dec_session_init(const gvx_dims *d, gvx_session *s, void *workspace, void *stream);
+/* Appends k utterances (ids s->submitted .. s->submitted + k - 1) and computes their processed memory.
+ *   memory [k, N, E]; lengths [k] int64 or NULL (all N); frame_caps [k] int32 or NULL (max_steps)
+ * Refused: submitted + k - admitted > capacity, or an id + row_offset past 2^31 - 1.  Asynchronous on `stream`. */
+int gvx_dec_session_submit(const gvx_dims *d, const gvx_weights *w, const void *packed, gvx_session *s,
+                           const float *memory, const int64_t *lengths, const int32_t *frame_caps, int k,
+                           void *workspace, void *stream);
+/* Runs up to max_steps_this_call (>= 1) decoder steps; it ends early once no slot is active (the queue is then empty: it
+ * only grows between calls, and the idle slots take from it at the head of every call).  A session with no active slot
+ * and no queued utterance runs 0 steps and launches nothing.  For step i < *steps_run and slot j (row i * slots + j):
+ *   utt[i][j]    int32: the utterance the slot decoded, -1 = idle (the other outputs of that row are not written)
+ *   frame[i][j]  int32: its local frame index;  last[i][j] int8: 1 on its last frame (its frame count is frame + 1)
+ *   frames[i][j] [n_mels + 1] floats: the [mel | gate] row;  align[i][j] [N] floats (when align is not NULL)
+ * Buffers are [max_steps_this_call][slots][...] device arrays.  Synchronises with the host (the stop poll, every
+ * GVX_STOP_POLL steps and at the end) and updates steps_run, admitted, finished and active. */
+int gvx_dec_session_step(const gvx_dims *d, const gvx_weights *w, const void *packed, gvx_session *s, int max_steps_this_call,
+                         float *frames, float *align, int32_t *utt, int32_t *frame, int8_t *last, int *steps_run,
+                         void *workspace, void *stream);
+
 /* ---- single-phase entry points (used by the parity tests to localise a failure) ---- */
 
 /* The tcgen05 / TMEM / TMA gate-GEMM engine on its own: out[B, Mtot] = X[B, K] . W[Mtot, K]^T with both
