@@ -31,7 +31,8 @@ int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
                    float *gate_out, float *align_out, float *s, cudaStream_t st);
 int infer_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths, int B,
                int N, int max_steps, float gate_threshold, int ignore_gate, uint64_t seed, int training, int row_offset,
-               float *mel_out, float *gate_out, float *align_out, int32_t *n_frames, int *steps_run, float *s, cudaStream_t st);
+               float *mel_out, float *gate_out, float *align_out, int32_t *n_frames, int *steps_run, int win_back, int win_fwd,
+               float *s, cudaStream_t st);
 
 int check_dims(const gvx_dims *d) {
     GVX_CHECK(d != nullptr, "dims is null");
@@ -49,6 +50,13 @@ int check_dims(const gvx_dims *d) {
         GVX_CHECK(d->n_mels % 8 == 0 && d->enc_dim % 8 == 0 && d->att_rnn_dim % 32 == 0 && d->dec_rnn_dim % 32 == 0 &&
                       d->prenet_dim % 8 == 0 && d->att_dim % 8 == 0,
                   "bf16 mode: feature dims must be multiples of 8 and the rnn dims multiples of 32");
+    return 0;
+}
+
+// attention constraint of the inference entry points: att_forward == 0 is off
+int check_window(int att_backward, int att_forward) {
+    GVX_CHECK(att_backward >= 0, "attention window: att_backward must be >= 0");
+    GVX_CHECK(att_forward >= 0, "attention window: att_forward must be >= 0 (0: no constraint)");
     return 0;
 }
 
@@ -171,7 +179,7 @@ int run_query(const Dims &d, const gvx_weights *w, const float *h_att, int B, fl
 int run_attention(const Dims &d, const gvx_weights *w, const float *packed, const float *q, const float *pm,
                   const float *memory, const int64_t *lengths, int B, int N, float *w_prev, float *cum, float *align_out,
                   long long align_bstride, float *cum_stash, float *ctx_out, float *th_stash, float *conv_stash,
-                  cudaStream_t st) {
+                  cudaStream_t st, int win_back = 0, int win_fwd = 0) {
     const PackedL PL(d);
     AttnFwdArgs a;
     memset(&a, 0, sizeof(a));
@@ -183,6 +191,7 @@ int run_attention(const Dims &d, const gvx_weights *w, const float *packed, cons
     a.align_out = align_out; a.align_bstride = align_bstride; a.cum_stash = cum_stash;
     a.ctx_out = ctx_out; a.ctx_ld = d.E;
     a.th_stash = th_stash; a.conv_stash = conv_stash;
+    a.win_back = win_back; a.win_fwd = win_fwd;
     return launch_attention_fwd_best(a, st);
 }
 
@@ -360,11 +369,12 @@ static int train_fwd_body(const gvx_dims *dd, const gvx_weights *w, const void *
 
 // One decoder step of inference (tacotron2.py:398-403): prenet on the previous mel frame `prev` (dropout on, :143), attention
 // LSTM, attention (weights to align_t, row stride align_bstride), decoder LSTM, [mel | gate] projection to out_t.
-// row_frame / row_id: optional per-row prenet dropout frame and row (run_prenet).
+// row_frame / row_id: optional per-row prenet dropout frame and row (run_prenet).  win_back / win_fwd: the attention
+// constraint (AttnFwdArgs; win_fwd == 0: off).
 static int infer_step(const Dims &d, const gvx_weights *w, const float *packed, const InferL &L, float *s, const float *memory,
                       const int64_t *mem_lengths, int B, int N, uint64_t seed, int t, int training, int row_offset,
                       const int *row_frame, const int *row_id, const float *prev, float *align_t, long long align_bstride,
-                      float *out_t, bool fused_prenet, cudaStream_t st) {
+                      float *out_t, bool fused_prenet, int win_back, int win_fwd, cudaStream_t st) {
     const int cur = t & 1, nxt = cur ^ 1;
     const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H;
     int *flags = (int *)(s + L.FLAGS);
@@ -384,7 +394,7 @@ static int infer_step(const Dims &d, const gvx_weights *w, const float *packed, 
     { ProfScope ps(PS_QUERY, st); GVX_TRY(run_query(d, w, s + L.HA + nxt * BA, B, s + L.Q, st)); }
     { ProfScope ps(PS_ATTENTION, st);
       GVX_TRY(run_attention(d, w, packed, s + L.Q, s + L.PM, memory, mem_lengths, B, N, s + L.WPREV, s + L.CUM,
-                            align_t, align_bstride, nullptr, s + L.CTX, nullptr, nullptr, st)); }
+                            align_t, align_bstride, nullptr, s + L.CTX, nullptr, nullptr, st, win_back, win_fwd)); }
     LstmIO c;
     c.x0 = s + L.HA + nxt * BA; c.w0 = d.A; c.ld0 = d.A;
     c.x1 = s + L.CTX; c.w1 = d.E; c.ld1 = d.E;
@@ -398,12 +408,12 @@ static int infer_step(const Dims &d, const gvx_weights *w, const float *packed, 
 static int infer_body(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
                       const int64_t *mem_lengths, int B, int N, int max_steps, float gate_threshold, int ignore_gate,
                       uint64_t seed, int training, int row_offset, float *mel_out, float *gate_out, float *align_out,
-                      int32_t *n_frames, int *steps_run, void *workspace, void *stream) {
+                      int32_t *n_frames, int *steps_run, int win_back, int win_fwd, void *workspace, void *stream) {
     const Dims d(*dd);
     if (dd->precision == GVX_BF16)
         return infer_bf16(d, w, (const float *)packed_, memory, mem_lengths, B, N, max_steps, gate_threshold, ignore_gate, seed,
-                          training, row_offset, mel_out, gate_out, align_out, n_frames, steps_run, (float *)workspace,
-                          (cudaStream_t)stream);
+                          training, row_offset, mel_out, gate_out, align_out, n_frames, steps_run, win_back, win_fwd,
+                          (float *)workspace, (cudaStream_t)stream);
     const InferL L(d, B, N, max_steps);
     const float *packed = (const float *)packed_;
     float *s = (float *)workspace;
@@ -433,7 +443,7 @@ static int infer_body(const gvx_dims *dd, const gvx_weights *w, const void *pack
         const float *prev = t == 0 ? s + L.ZERO : s + L.OUT + (size_t)(t - 1) * B * d.OL;
         float *out_t = s + L.OUT + (size_t)t * B * d.OL;
         GVX_TRY(infer_step(d, w, packed, L, s, memory, mem_lengths, B, N, seed, t, training, row_offset, nullptr, nullptr, prev,
-                           align_out + (size_t)t * N, (long long)max_steps * N, out_t, fused_prenet, st));
+                           align_out + (size_t)t * N, (long long)max_steps * N, out_t, fused_prenet, win_back, win_fwd, st));
         if (!ignore_gate) {
             GVX_CUDA(launch_pdl(k_gate_check, dim3(1), dim3(128), 0, st, (const float *)out_t, B, d.M, d.OL, gate_threshold, t, n_frames, flags));
     GVX_LAUNCHED(1);
@@ -494,14 +504,15 @@ int gvx_dec_train_fwd(const gvx_dims *dd, const gvx_weights *w, const void *pack
     return rc;
 }
 
-int gvx_dec_infer(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
-                  const int64_t *mem_lengths, int B, int N, int max_steps, float gate_threshold, int ignore_gate,
-                  uint64_t seed, int training, int row_offset, float *mel_out, float *gate_out, float *align_out,
-                  int32_t *n_frames, int *steps_run, void *workspace, void *stream) {
+int gvx_dec_infer_windowed(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
+                           const int64_t *mem_lengths, int B, int N, int max_steps, float gate_threshold, int ignore_gate,
+                           uint64_t seed, int training, int row_offset, float *mel_out, float *gate_out, float *align_out,
+                           int32_t *n_frames, int *steps_run, int att_backward, int att_forward, void *workspace, void *stream) {
     GVX_TRY(check_dims(dd));
     GVX_CHECK(w && packed_ && memory && mel_out && gate_out && align_out && n_frames && steps_run && workspace,
               "null argument");
     GVX_CHECK(B > 0 && N > 0 && max_steps > 0, "B, N, max_steps must be positive");
+    GVX_TRY(check_window(att_backward, att_forward));
     GVX_TRY(latch_check());
     cudaStream_t user = (cudaStream_t)stream;
     const Dims d(*dd);
@@ -515,15 +526,17 @@ int gvx_dec_infer(const gvx_dims *dd, const gvx_weights *w, const void *packed_,
     if (ignore_gate) {          // fixed step count: no host polling inside, the whole sequence is one graph
         KeyBuilder kb;
         kb.add((int)3).add(*dd).add(*w).add(packed_).add(memory).add(mem_lengths).add(B).add(N).add(max_steps).add(gate_threshold)
-            .add(training).add(row_offset).add(mel_out).add(gate_out).add(align_out).add(n_frames).add(workspace);
+            .add(training).add(row_offset).add(mel_out).add(gate_out).add(align_out).add(n_frames).add(workspace)
+            .add(att_backward).add(att_forward);       // baked into the captured attention launches
         rc = run_cached(kb.k, user, [&](cudaStream_t st) {
             return infer_body(dd, w, packed_, memory, mem_lengths, B, N, max_steps, gate_threshold, ignore_gate, seed, training,
-                              row_offset, mel_out, gate_out, align_out, n_frames, steps_run, workspace, (void *)st);
+                              row_offset, mel_out, gate_out, align_out, n_frames, steps_run, att_backward, att_forward, workspace,
+                              (void *)st);
         });
         *steps_run = max_steps;
     } else {
         rc = infer_body(dd, w, packed_, memory, mem_lengths, B, N, max_steps, gate_threshold, ignore_gate, seed, training,
-                        row_offset, mel_out, gate_out, align_out, n_frames, steps_run, workspace, stream);
+                        row_offset, mel_out, gate_out, align_out, n_frames, steps_run, att_backward, att_forward, workspace, stream);
     }
     g_seed_ptr = nullptr;
     if (rc == 0 && bf)
@@ -532,6 +545,14 @@ int gvx_dec_infer(const gvx_dims *dd, const gvx_weights *w, const void *packed_,
     if (rc == 0 && !bf)      // error word of the fused inference prenet's grid barrier (gvx_infer_prenet.cuh)
         rc = check_tc_err_public(reinterpret_cast<int *>((float *)workspace + flags_off) + 41, user, "gvx_dec_infer (prenet barrier)");
     return rc;
+}
+
+int gvx_dec_infer(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
+                  const int64_t *mem_lengths, int B, int N, int max_steps, float gate_threshold, int ignore_gate,
+                  uint64_t seed, int training, int row_offset, float *mel_out, float *gate_out, float *align_out,
+                  int32_t *n_frames, int *steps_run, void *workspace, void *stream) {
+    return gvx_dec_infer_windowed(dd, w, packed_, memory, mem_lengths, B, N, max_steps, gate_threshold, ignore_gate, seed, training,
+                                  row_offset, mel_out, gate_out, align_out, n_frames, steps_run, 0, 0, workspace, stream);
 }
 
 int gvx_device_error(int clear) {

@@ -62,7 +62,45 @@ struct AttnFwdArgs {
     float *conv_stash;       // [B, N, F] location-conv output for the backward pass, or null
     int th_bf16;             // k_attention_fwd_c2 only: write th_stash as bf16 rows of 256 B with 16-byte chunks swizzled by (token & 7),
                              // the format the persistent BPTT chain reads (gvx_fused_bwd.cuh)
+    int win_back, win_fwd;   // attention constraint (inference): win_fwd == 0 off, else attend only to
+                             // [last - win_back, last + win_fwd), last = argmax of w_prev's row (attn_window).  The forward
+                             // kernels are instantiated for WIN = (win_fwd != 0), so the unconstrained code is unchanged
 };
+
+// The token window [lo, hi) a constrained step may attend to: last = argmax_n w[n] (lowest index on ties, as torch.argmax),
+// lo = max(0, last - back), hi = min(len, last + fwd).  It is never empty: last lies in the previous step's window.
+// A block reduction of (value, ~index) keys; every thread gets the result.  `scratch`: 64 floats, 8-byte aligned.
+__device__ __forceinline__ int2 attn_window(const float *w, int N, int len, int back, int fwd, float *scratch) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
+    unsigned long long best = 0;
+    for (int n = threadIdx.x; n < N; n += blockDim.x) {
+        const unsigned u = __float_as_uint(w[n]);
+        const unsigned key = (u & 0x80000000u) ? ~u : (u | 0x80000000u);       // order-preserving map of the float
+        const unsigned long long k = ((unsigned long long)key << 32) | (unsigned)(~n);
+        best = k > best ? k : best;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const unsigned long long k = __shfl_xor_sync(0xffffffffu, best, o);
+        best = k > best ? k : best;
+    }
+    unsigned long long *sc = reinterpret_cast<unsigned long long *>(scratch);
+    __syncthreads();
+    if (lane == 0) sc[wid] = best;
+    __syncthreads();
+    if (wid == 0) {
+        unsigned long long x = lane < nw ? sc[lane] : 0ull;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const unsigned long long k = __shfl_xor_sync(0xffffffffu, x, o);
+            x = k > x ? k : x;
+        }
+        if (lane == 0) sc[0] = x;          // lanes 1..31 read only sc[1..31] above
+    }
+    __syncthreads();
+    const int last = (int)~(unsigned)(sc[0] & 0xffffffffull);
+    return make_int2(max(0, last - back), fwd > len - last ? len : last + fwd);
+}
 
 // stage w_{t-1} / cum_{t-1} (zero halo), the small weights and q into shared memory
 __device__ __forceinline__ void attn_stage_inputs(const AttnShape &s, const AttnSmem &L, float *sm, const float *wprev_row,
@@ -97,6 +135,7 @@ __device__ __forceinline__ void attn_conv(const AttnShape &s, const AttnSmem &L,
     }
 }
 
+template <bool WIN>
 __global__ void __launch_bounds__(ATT_THREADS, 1) k_attention_fwd(const AttnFwdArgs a) {
     pdl_trigger();
     pdl_wait();
@@ -109,6 +148,8 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) k_attention_fwd(const AttnFwdA
 
     attn_stage_inputs(s, L, sm, wprev_row, cum_row, a.wlc, a.wldT, a.v, a.q, b);
     __syncthreads();
+    int2 win = make_int2(0, len);
+    if (WIN) win = attn_window(sm + L.wcat + (s.KS - 1) / 2, s.N, len, a.win_back, a.win_fwd, sm + L.scratch);
     attn_conv(s, L, sm);
     __syncthreads();
     if (a.conv_stash) {
@@ -147,7 +188,7 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) k_attention_fwd(const AttnFwdA
             part = fmaf(vv.w, th.w, part);
         }
         part = warp_sum(part);
-        if (lane == 0) sm[L.e + n] = n < len ? part : -INFINITY;
+        if (lane == 0) sm[L.e + n] = (WIN ? n >= win.x && n < win.y : n < len) ? part : -INFINITY;
     }
     __syncthreads();
 
@@ -191,20 +232,25 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) k_attention_fwd(const AttnFwdA
     }
 }
 
+template <bool WIN>
+inline int launch_attention_fwd_k(const AttnFwdArgs &a, size_t bytes, cudaStream_t stream) {
+    static size_t configured = 0;      // per instantiation
+    if (bytes > configured) {
+        GVX_CUDA(cudaFuncSetAttribute(k_attention_fwd<WIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        configured = bytes;
+    }
+    GVX_CUDA(launch_pdl(k_attention_fwd<WIN>, dim3(a.s.B), dim3(ATT_THREADS), bytes, stream, a));
+    GVX_LAUNCHED(1);
+    GVX_CUDA(cudaGetLastError());
+    return 0;
+}
+
 inline int launch_attention_fwd(const AttnFwdArgs &a, cudaStream_t stream) {
     const AttnSmem L(a.s);
     const size_t bytes = (size_t)L.total * sizeof(float);
     GVX_CHECK(bytes <= 200 * 1024, "attention: token count too large for the shared-memory tile");
     GVX_CHECK(a.s.D % 4 == 0, "attention_dim must be a multiple of 4");
-    static size_t configured = 0;
-    if (bytes > configured) {
-        GVX_CUDA(cudaFuncSetAttribute(k_attention_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        configured = bytes;
-    }
-    GVX_CUDA(launch_pdl(k_attention_fwd, dim3(a.s.B), dim3(ATT_THREADS), bytes, stream, a));
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    return 0;
+    return a.win_fwd ? launch_attention_fwd_k<true>(a, bytes, stream) : launch_attention_fwd_k<false>(a, bytes, stream);
 }
 
 // ------------------------------------------------------------------ backward (one step, one CTA per row)

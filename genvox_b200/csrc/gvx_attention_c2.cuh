@@ -53,6 +53,7 @@ struct AttnC2FwdSmem {
     }
 };
 
+template <bool WIN>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AF_THREADS, 1) k_attention_fwd_c2(const AttnFwdArgs a) {
     extern __shared__ __align__(16) float sm[];
     cg::cluster_group cluster = cg::this_cluster();
@@ -86,6 +87,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AF_THREADS, 1) k_att
     }
     if (tid < AF_D) sm[L.q + tid] = src_get(a.q, b, tid);
     __syncthreads();
+    // the constraint needs the argmax of the whole w_{t-1} row: both CTAs reduce it from global memory, before the first
+    // cluster.sync (after it the peer overwrites its half of the row with w_t)
+    int2 win = make_int2(0, len);
+    if (WIN) win = attn_window(wprev_row, N, len, a.win_back, a.win_fwd, sm + L.scratch);
 
     // ---- location conv for the own tokens
     for (int task = tid; task < AF_F * G.nblk; task += AF_THREADS) {
@@ -185,7 +190,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(AF_THREADS, 1) k_att
             if (lane < 4) {
                 const int nl = n0 + lane;
                 const float pv = lane == 0 ? part[0] : (lane == 1 ? part[1] : (lane == 2 ? part[2] : part[3]));
-                if (nl < n_own) sm[L.e + nl] = (n_lo + nl) < len ? pv : -INFINITY;
+                if (nl < n_own) sm[L.e + nl] = (WIN ? n_lo + nl >= win.x && n_lo + nl < win.y : (n_lo + nl) < len) ? pv : -INFINITY;
             }
         }
     }
@@ -650,6 +655,18 @@ inline bool attention_fwd_uses_c2(const AttnShape &s) {
     // the split pays when the rows alone cannot fill the machine
     return attention_c2_enabled() && attention_fast_ok(s) && s.B <= 74 && s.N >= 32 && s.E % 8 == 0 && bytes <= 200 * 1024;
 }
+template <bool WIN>
+inline int launch_attention_fwd_c2_k(const AttnFwdArgs &a, size_t bytes, cudaStream_t stream) {
+    static size_t configured = 0;      // per instantiation
+    if (bytes > configured) {
+        GVX_CUDA(cudaFuncSetAttribute(k_attention_fwd_c2<WIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        configured = bytes;
+    }
+    GVX_CUDA(launch_pdl(k_attention_fwd_c2<WIN>, dim3(2 * a.s.B), dim3(AF_THREADS), bytes, stream, a));
+    GVX_LAUNCHED(1);
+    return 0;
+}
+
 inline int launch_attention_fwd_best(const AttnFwdArgs &a, cudaStream_t stream) {
     const AttnC2FwdSmem L(a.s.N, a.s.E);
     const size_t bytes = (size_t)L.total * sizeof(float);
@@ -657,14 +674,7 @@ inline int launch_attention_fwd_best(const AttnFwdArgs &a, cudaStream_t stream) 
         GVX_CHECK(!a.th_bf16, "the bf16 tanh stash is only written by the cluster attention kernel");
         return launch_attention_fwd_any(a, stream);
     }
-    static size_t configured = 0;
-    if (bytes > configured) {
-        GVX_CUDA(cudaFuncSetAttribute(k_attention_fwd_c2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        configured = bytes;
-    }
-    GVX_CUDA(launch_pdl(k_attention_fwd_c2, dim3(2 * a.s.B), dim3(AF_THREADS), bytes, stream, a));
-    GVX_LAUNCHED(1);
-    return 0;
+    return a.win_fwd ? launch_attention_fwd_c2_k<true>(a, bytes, stream) : launch_attention_fwd_c2_k<false>(a, bytes, stream);
 }
 
 inline bool attention_bwd_uses_c2(const AttnShape &s) {

@@ -49,6 +49,7 @@ struct AttnFastSmem {
     }
 };
 
+template <bool WIN>
 __global__ void __launch_bounds__(AF_THREADS, 1) k_attention_fwd_fast(const AttnFwdArgs a) {
     extern __shared__ __align__(16) float sm[];
     const int N = a.s.N, E = a.s.E;
@@ -73,6 +74,8 @@ __global__ void __launch_bounds__(AF_THREADS, 1) k_attention_fwd_fast(const Attn
     }
     if (tid < AF_D) sm[L.q + tid] = src_get(a.q, b, tid);
     __syncthreads();
+    int2 win = make_int2(0, len);
+    if (WIN) win = attn_window(sm + L.wcat + AF_PAD, N, len, a.win_back, a.win_fwd, sm + L.scratch);
 
     // ---- location conv: task = (filter f, block of 8 tokens); sliding window in registers
     for (int task = tid; task < AF_F * L.nblk; task += AF_THREADS) {
@@ -160,7 +163,7 @@ __global__ void __launch_bounds__(AF_THREADS, 1) k_attention_fwd_fast(const Attn
             if (lane < 4) {
                 const int n = n0 + lane;
                 const float pv = lane == 0 ? part[0] : (lane == 1 ? part[1] : (lane == 2 ? part[2] : part[3]));
-                if (n < N) sm[L.e + n] = n < len ? pv : -INFINITY;
+                if (n < N) sm[L.e + n] = (WIN ? n >= win.x && n < win.y : n < len) ? pv : -INFINITY;
             }
         }
     }
@@ -405,19 +408,24 @@ inline bool attention_fast_ok(const AttnShape &s) {
     return s.F == AF_F && s.KS == AF_KS && s.D == AF_D && s.E % 4 == 0 && s.N >= 1;
 }
 
+template <bool WIN>
+inline int launch_attention_fwd_fast_k(const AttnFwdArgs &a, size_t bytes, cudaStream_t stream) {
+    static size_t configured = 0;      // per instantiation
+    if (bytes > configured) {
+        GVX_CUDA(cudaFuncSetAttribute(k_attention_fwd_fast<WIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        configured = bytes;
+    }
+    GVX_CUDA(launch_pdl(k_attention_fwd_fast<WIN>, dim3(a.s.B), dim3(AF_THREADS), bytes, stream, a));
+    GVX_LAUNCHED(1);
+    GVX_CUDA(cudaGetLastError());
+    return 0;
+}
+
 inline int launch_attention_fwd_any(const AttnFwdArgs &a, cudaStream_t stream) {
     const AttnFastSmem L(a.s.N, a.s.E);
     const size_t bytes = (size_t)L.total * sizeof(float);
     if (!attention_fast_ok(a.s) || bytes > 200 * 1024) return launch_attention_fwd(a, stream);
-    static size_t configured = 0;
-    if (bytes > configured) {
-        GVX_CUDA(cudaFuncSetAttribute(k_attention_fwd_fast, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        configured = bytes;
-    }
-    GVX_CUDA(launch_pdl(k_attention_fwd_fast, dim3(a.s.B), dim3(AF_THREADS), bytes, stream, a));
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    return 0;
+    return a.win_fwd ? launch_attention_fwd_fast_k<true>(a, bytes, stream) : launch_attention_fwd_fast_k<false>(a, bytes, stream);
 }
 
 inline int launch_attention_bwd_any(const AttnBwdArgs &a, cudaStream_t stream) {

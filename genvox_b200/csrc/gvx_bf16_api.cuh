@@ -824,11 +824,12 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
 // ======================================================================================= inference
 // One decoder step (tacotron2.py:398-403): prenet on the previous mel frame `prev` (straight into the attention-LSTM operand
 // image), attention LSTM, query, attention (weights to align_t, row stride align_bstride), decoder LSTM, [mel | gate] projection
-// to out_t.  row_frame / row_id: optional per-row prenet dropout frame and row (run_infer_prenet, run_prenet).
+// to out_t.  row_frame / row_id: optional per-row prenet dropout frame and row (run_infer_prenet, run_prenet).  win_back /
+// win_fwd: the attention constraint (AttnFwdArgs; win_fwd == 0: off).
 static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *packed, const InferBfL &L, float *s, const float *memory,
                            const int64_t *mem_lengths, int B, int N, uint64_t seed, int t, int training, int row_offset,
                            const int *row_frame, const int *row_id, const float *prev, float *align_t, long long align_bstride,
-                           float *out_t, cudaStream_t st) {
+                           float *out_t, int win_back, int win_fwd, cudaStream_t st) {
     const BfGeom g(d);
     const PackedL PL(d);
     const PackedBfL BL(d, PL.total);
@@ -874,6 +875,7 @@ static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *pac
         a.w_prev = s + L.WPREV; a.cum = s + L.CUM;
         a.align_out = align_t; a.align_bstride = align_bstride;
         a.ctx_ld = d.E;
+        a.win_back = win_back; a.win_fwd = win_fwd;
         add_img(a.ctx_bf, xd, d.A, NPAD); add_img(a.ctx_bf, xa_n, d.P, NPAD); add_img(a.ctx_bf, XPI, d.H, NPAD);
         GVX_TRY(launch_attention_fwd_best(a, st));
     }
@@ -898,8 +900,8 @@ static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *pac
 
 int infer_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
                       int B, int N, int max_steps, float gate_threshold, int ignore_gate, uint64_t seed, int training,
-                      int row_offset, float *mel_out, float *gate_out, float *align_out, int32_t *n_frames, int *steps_run, float *s,
-                      cudaStream_t st) {
+                      int row_offset, float *mel_out, float *gate_out, float *align_out, int32_t *n_frames, int *steps_run,
+                      int win_back, int win_fwd, float *s, cudaStream_t st) {
     GVX_TRY(check_bf16_dims(d, B));
     const BfGeom g(d);
     const InferBfL L(d, B, N, max_steps);
@@ -929,7 +931,7 @@ int infer_bf16(const Dims &d, const gvx_weights *w, const float *packed, const f
         const float *prev = t == 0 ? s + L.ZERO : s + L.OUT + (size_t)(t - 1) * B * d.OL;
         float *out_t = s + L.OUT + (size_t)t * B * d.OL;
         GVX_TRY(infer_step_bf16(d, w, packed, L, s, memory, mem_lengths, B, N, seed, t, training, row_offset, nullptr, nullptr, prev,
-                                align_out + (size_t)t * N, (long long)max_steps * N, out_t, st));
+                                align_out + (size_t)t * N, (long long)max_steps * N, out_t, win_back, win_fwd, st));
         if (!ignore_gate) {
             GVX_CUDA(launch_pdl(k_gate_check, dim3(1), dim3(128), 0, st, (const float *)out_t, B, d.M, d.OL, gate_threshold, t, n_frames, flags));
             GVX_LAUNCHED(1);

@@ -7,8 +7,8 @@
 // poll.  Admission is deterministic and uses no atomics: the slots that stop in the same step take queue entries in slot
 // order, and every CTA recomputes all S stop decisions to find its own prefix count.
 //
-// Output identity: utterance u decodes bit-identically to row r of a static call with the same S rows, N, seed and
-// precision, u in row r and dropout_row_offset = u + row_offset - r.  The slot's every piece of recurrent state is zeroed
+// Output identity: utterance u decodes bit-identically to row r of a static call with the same S rows, N, seed, precision
+// and attention window, u in row r and dropout_row_offset = u + row_offset - r.  The slot's every piece of recurrent state is zeroed
 // in the layout it lives in, its memory / processed memory / length are replaced, and the prenet draws its dropout at
 // Philox (row u + row_offset, t = local frame) through the per-row row_frame / row_id arrays.
 #pragma once
@@ -219,7 +219,7 @@ inline void admit_state(AdmitArgs &a, const Dims &d, bool bf, const InferL &Lf, 
 int infer_continuous(const gvx_dims *dd, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
                      int U, int N, int S, int max_steps, const int32_t *frame_caps, float gate_threshold, int ignore_gate,
                      uint64_t seed, int row_offset, float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
-                     long long *steps_run, float *s, cudaStream_t st) {
+                     long long *steps_run, int win_back, int win_fwd, float *s, cudaStream_t st) {
     const Dims d(*dd);
     const bool bf = dd->precision == GVX_BF16;
     if (bf) GVX_TRY(check_bf16_dims(d, S));
@@ -291,9 +291,9 @@ int infer_continuous(const gvx_dims *dd, const gvx_weights *w, const float *pack
         // processed memory before griddepcontrol.wait, and an admission rewrites both
         pdl_barrier_next();
         if (bf) GVX_TRY(infer_step_bf16(d, w, packed, Lb, s, mem_slot, len_slot, S, N, seed, (int)t, 0, row_offset, frame, utt, prev,
-                                        s + C.ALIGN, (long long)N, out_t, st));
+                                        s + C.ALIGN, (long long)N, out_t, win_back, win_fwd, st));
         else GVX_TRY(infer_step(d, w, packed, Lf, s, mem_slot, len_slot, S, N, seed, (int)t, 0, row_offset, frame, utt, prev,
-                                s + C.ALIGN, (long long)N, out_t, fused_prenet, st));
+                                s + C.ALIGN, (long long)N, out_t, fused_prenet, win_back, win_fwd, st));
         a.out_t = out_t;
         a.utt_cur = utt; a.frame_cur = frame; a.next_cur = state + 4 * S + p;
         a.utt_nxt = state + (p ^ 1) * S; a.frame_nxt = state + 2 * S + (p ^ 1) * S; a.next_nxt = state + 4 * S + (p ^ 1);
@@ -324,14 +324,16 @@ size_t gvx_dec_infer_continuous_workspace_bytes(const gvx_dims *d, int U, int N,
     return ContL(dm, continuous_base(dm, bf, slots, N), U, N, slots).total * sizeof(float);
 }
 
-int gvx_dec_infer_continuous(const gvx_dims *dd, const gvx_weights *w, const void *packed, const float *memory,
-                             const int64_t *mem_lengths, int U, int N, int slots, int max_steps, const int32_t *frame_caps,
-                             float gate_threshold, int ignore_gate, uint64_t seed, int row_offset, float *mel_out, float *gate_out,
-                             float *align_out, int32_t *n_frames, long long *steps_run, void *workspace, void *stream) {
+int gvx_dec_infer_continuous_windowed(const gvx_dims *dd, const gvx_weights *w, const void *packed, const float *memory,
+                                      const int64_t *mem_lengths, int U, int N, int slots, int max_steps, const int32_t *frame_caps,
+                                      float gate_threshold, int ignore_gate, uint64_t seed, int row_offset, float *mel_out,
+                                      float *gate_out, float *align_out, int32_t *n_frames, long long *steps_run, int att_backward,
+                                      int att_forward, void *workspace, void *stream) {
     using namespace gvx;
     GVX_TRY(check_dims(dd));
     GVX_CHECK(w && packed && memory && mel_out && gate_out && n_frames && steps_run && workspace, "null argument");
     GVX_CHECK(U > 0 && N > 0 && slots > 0 && max_steps > 0, "U, N, slots, max_steps must be positive");
+    GVX_TRY(check_window(att_backward, att_forward));
     GVX_TRY(latch_check());
     cudaStream_t st = (cudaStream_t)stream;
     const Dims d(*dd);
@@ -342,7 +344,8 @@ int gvx_dec_infer_continuous(const gvx_dims *dd, const gvx_weights *w, const voi
     GVX_TRY(put_seed(slot, seed, st));
     g_seed_ptr = slot;
     int rc = infer_continuous(dd, w, (const float *)packed, memory, mem_lengths, U, N, slots, max_steps, frame_caps, gate_threshold,
-                              ignore_gate, seed, row_offset, mel_out, gate_out, align_out, n_frames, steps_run, (float *)workspace, st);
+                              ignore_gate, seed, row_offset, mel_out, gate_out, align_out, n_frames, steps_run, att_backward, att_forward,
+                              (float *)workspace, st);
     g_seed_ptr = nullptr;
     if (rc == 0 && bf)
         rc = check_tc_err_public(reinterpret_cast<int *>((float *)workspace + InferBfL(d, slots, N, 2).ERR), st,
@@ -351,6 +354,15 @@ int gvx_dec_infer_continuous(const gvx_dims *dd, const gvx_weights *w, const voi
         rc = check_tc_err_public(reinterpret_cast<int *>((float *)workspace + flags_off) + 41, st,
                                  "gvx_dec_infer_continuous (prenet barrier)");
     return rc;
+}
+
+int gvx_dec_infer_continuous(const gvx_dims *dd, const gvx_weights *w, const void *packed, const float *memory,
+                             const int64_t *mem_lengths, int U, int N, int slots, int max_steps, const int32_t *frame_caps,
+                             float gate_threshold, int ignore_gate, uint64_t seed, int row_offset, float *mel_out, float *gate_out,
+                             float *align_out, int32_t *n_frames, long long *steps_run, void *workspace, void *stream) {
+    return gvx_dec_infer_continuous_windowed(dd, w, packed, memory, mem_lengths, U, N, slots, max_steps, frame_caps, gate_threshold,
+                                             ignore_gate, seed, row_offset, mel_out, gate_out, align_out, n_frames, steps_run, 0, 0,
+                                             workspace, stream);
 }
 
 }  // extern "C"

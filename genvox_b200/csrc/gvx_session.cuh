@@ -104,7 +104,8 @@ int session_submit(const Dims &d, bool bf, const gvx_weights *w, const gvx_sessi
 }
 
 int session_step(const Dims &d, bool bf, const gvx_weights *w, const float *packed, gvx_session *ss, int K, float *frames,
-                 float *align, int32_t *utt_out, int32_t *frame_out, int8_t *last_out, int *steps_run, float *s, cudaStream_t st) {
+                 float *align, int32_t *utt_out, int32_t *frame_out, int8_t *last_out, int *steps_run, int win_back, int win_fwd,
+                 float *s, cudaStream_t st) {
     const int S = ss->slots, N = ss->N, cap = ss->capacity;
     const InferL Lf(d, S, N, 2);
     const InferBfL Lb(d, S, N, 2);
@@ -162,9 +163,9 @@ int session_step(const Dims &d, bool bf, const gvx_weights *w, const float *pack
         // processed memory that kernels of the chain read before griddepcontrol.wait)
         pdl_barrier_next();
         if (bf) GVX_TRY(infer_step_bf16(d, w, packed, Lb, s, mem_slot, len_slot, S, N, ss->seed, t, 0, ss->row_offset, a.frame_cur,
-                                        a.utt_cur, prev, s + L.ALIGN, (long long)N, out_t, st));
+                                        a.utt_cur, prev, s + L.ALIGN, (long long)N, out_t, win_back, win_fwd, st));
         else GVX_TRY(infer_step(d, w, packed, Lf, s, mem_slot, len_slot, S, N, ss->seed, t, 0, ss->row_offset, a.frame_cur, a.utt_cur,
-                                prev, s + L.ALIGN, (long long)N, out_t, fused_prenet, st));
+                                prev, s + L.ALIGN, (long long)N, out_t, fused_prenet, win_back, win_fwd, st));
         a.out_t = out_t;
         a.step = i;
         GVX_CUDA(launch_pdl(k_gate_admit, dim3(S), dim3(ADMIT_THREADS), 0, st, a));
@@ -238,11 +239,12 @@ int gvx_dec_session_submit(const gvx_dims *dd, const gvx_weights *w, const void 
     return 0;
 }
 
-int gvx_dec_session_step(const gvx_dims *dd, const gvx_weights *w, const void *packed, gvx_session *ss, int max_steps_this_call,
-                         float *frames, float *align, int32_t *utt, int32_t *frame, int8_t *last, int *steps_run, void *workspace,
-                         void *stream) {
+int gvx_dec_session_step_windowed(const gvx_dims *dd, const gvx_weights *w, const void *packed, gvx_session *ss,
+                                  int max_steps_this_call, float *frames, float *align, int32_t *utt, int32_t *frame, int8_t *last,
+                                  int *steps_run, int att_backward, int att_forward, void *workspace, void *stream) {
     using namespace gvx;
     GVX_TRY(check_session(dd, ss));
+    GVX_TRY(check_window(att_backward, att_forward));
     GVX_CHECK(ss->ready == SESSION_READY, "session: gvx_dec_session_init has not run");
     GVX_CHECK(w && packed && frames && utt && frame && last && steps_run && workspace, "null argument");
     GVX_CHECK(align || !ss->with_alignments, "session: align is null but with_alignments is set");
@@ -255,7 +257,8 @@ int gvx_dec_session_step(const gvx_dims *dd, const gvx_weights *w, const void *p
     cudaStream_t st = (cudaStream_t)stream;
     float *s = (float *)workspace;
     g_seed_ptr = session_seed_slot(d, bf, ss->N, ss->slots, s);
-    int rc = session_step(d, bf, w, (const float *)packed, ss, max_steps_this_call, frames, align, utt, frame, last, steps_run, s, st);
+    int rc = session_step(d, bf, w, (const float *)packed, ss, max_steps_this_call, frames, align, utt, frame, last, steps_run,
+                          att_backward, att_forward, s, st);
     g_seed_ptr = nullptr;
     if (rc == 0 && bf)
         rc = check_tc_err_public(reinterpret_cast<int *>(s + InferBfL(d, ss->slots, ss->N, 2).ERR), st, "gvx_dec_session_step");
@@ -263,6 +266,13 @@ int gvx_dec_session_step(const gvx_dims *dd, const gvx_weights *w, const void *p
         rc = check_tc_err_public(reinterpret_cast<int *>(s + InferL(d, ss->slots, ss->N, 2).FLAGS) + 41, st,
                                  "gvx_dec_session_step (prenet barrier)");
     return rc;
+}
+
+int gvx_dec_session_step(const gvx_dims *dd, const gvx_weights *w, const void *packed, gvx_session *ss, int max_steps_this_call,
+                         float *frames, float *align, int32_t *utt, int32_t *frame, int8_t *last, int *steps_run, void *workspace,
+                         void *stream) {
+    return gvx_dec_session_step_windowed(dd, w, packed, ss, max_steps_this_call, frames, align, utt, frame, last, steps_run, 0, 0,
+                                         workspace, stream);
 }
 
 }  // extern "C"

@@ -7,6 +7,7 @@ device memory, streams and autograd plumbing only.  There is no CPU path: non-CU
 """
 import ctypes as C
 
+import numpy as np
 import torch
 from torch import nn
 
@@ -32,6 +33,29 @@ def _f32c(t, name):
 
 def _buffer(nbytes, device):
     return torch.empty((nbytes + 3) // 4, dtype=torch.float32, device=device)
+
+
+class _FromAttribute:
+    def __repr__(self):
+        return "<Decoder.attention_window>"
+
+
+FROM_ATTRIBUTE = _FromAttribute()      # default of every `attention_window=` argument: use the decoder's attribute
+
+
+def attention_window_args(window):
+    """(att_backward, att_forward) for the C ABI: a (backward >= 0, forward >= 1) pair of ints turns the attention constraint
+    on, None turns it off (0, 0).  Anything else raises ValueError."""
+    if window is None:
+        return 0, 0
+    try:
+        back, fwd = window
+    except (TypeError, ValueError):
+        raise ValueError(f"genvox_b200: attention_window must be None or a (backward, forward) pair, got {window!r}") from None
+    for name, v, lo in (("backward", back, 0), ("forward", fwd, 1)):
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not lo <= int(v) <= 2 ** 31 - 1:
+            raise ValueError(f"genvox_b200: attention_window {name} must be an int in {lo} .. 2^31 - 1, got {v!r}")
+    return int(back), int(fwd)
 
 
 class _TeacherForced(torch.autograd.Function):
@@ -122,6 +146,10 @@ class Decoder(nn.Module):
         self.last_dropout_seed = None
         self.last_n_frames = None
         self.last_steps_run = None      # decoder steps of the last inference_continuous call
+        # attention constraint of inference (include/genvox_b200.h, gvx_dec_infer_windowed): None, or (backward, forward)
+        # to attend only to tokens [last - backward, last + forward) around the previous step's argmax.  Not a parameter
+        # or buffer, so not in the state_dict.
+        self.attention_window = None
         self._pack_key = None
         self._packed = None
         self._pack_epoch = 0          # bumped by invalidate_packed()
@@ -159,6 +187,9 @@ class Decoder(nn.Module):
         version counter (`p.data.copy_(...)`, an EMA swap through `.data`, manual re-initialisation): the cache key is
         (data_ptr, version) per parameter and `.data` writes do not bump the version."""
         self._pack_epoch += 1
+
+    def _window(self, attention_window):
+        return attention_window_args(self.attention_window if attention_window is FROM_ATTRIBUTE else attention_window)
 
     def _last_step_gate_fired(self, gate, n_frames, steps):
         """True when every row that reached the last allowed step did so because its gate fired there (then the reference's
@@ -206,10 +237,12 @@ class Decoder(nn.Module):
         return _TeacherForced.apply(self, memory, mel_in, lengths, self._next_seed(), *params)
 
     @torch.no_grad()
-    def inference(self, memory, memory_lengths=None, ignore_gate=False, max_decoder_steps=None):
+    def inference(self, memory, memory_lengths=None, ignore_gate=False, max_decoder_steps=None, attention_window=FROM_ATTRIBUTE):
         """Autoregressive decoding, tacotron2.py:390-414, for B >= 1 rows.  Returns the reference's triple
         (mel [B,n_mels,Tmax], gate [B,Tmax], alignments [B,Tmax,N]) with Tmax = max over rows of the per-row
-        frame count; the per-row counts are left in `self.last_n_frames` (int32 [B], device)."""
+        frame count; the per-row counts are left in `self.last_n_frames` (int32 [B], device).
+        attention_window: None or (backward, forward), the attention constraint; left out, `self.attention_window`."""
+        win = self._window(attention_window)
         lib = _native.load()
         memory = _f32c(memory, "memory")
         B, N, _ = memory.shape
@@ -226,11 +259,11 @@ class Decoder(nn.Module):
         n_frames = torch.empty(B, device=dev, dtype=torch.int32)
         work = _buffer(lib.gvx_dec_infer_workspace_bytes(C.byref(dims), B, N, steps), dev)
         ran = C.c_int(0)
-        _native.check(lib.gvx_dec_infer(C.byref(dims), C.byref(weights), _ptr(packed), _ptr(memory), _ptr(lengths), B, N,
-                                        steps, float(self.gate_threshold), int(bool(ignore_gate)), self._next_seed(),
-                                        int(self.training), self.dropout_row_offset, _ptr(mel), _ptr(gate), _ptr(align),
-                                        _ptr(n_frames), C.byref(ran), _ptr(work), _stream()),
-                      "gvx_dec_infer")
+        _native.check(lib.gvx_dec_infer_windowed(C.byref(dims), C.byref(weights), _ptr(packed), _ptr(memory), _ptr(lengths), B, N,
+                                                 steps, float(self.gate_threshold), int(bool(ignore_gate)), self._next_seed(),
+                                                 int(self.training), self.dropout_row_offset, _ptr(mel), _ptr(gate), _ptr(align),
+                                                 _ptr(n_frames), C.byref(ran), *win, _ptr(work), _stream()),
+                      "gvx_dec_infer_windowed")
         self.last_n_frames = n_frames
         tmax = steps if ignore_gate else int(n_frames.max().item())
         # tacotron2.py:405-409 breaks on the gate BEFORE it tests the step count: a row whose gate fires on the last allowed
@@ -241,13 +274,15 @@ class Decoder(nn.Module):
 
     @torch.no_grad()
     def inference_continuous(self, memory, memory_lengths, slots=64, max_decoder_steps=None, frame_caps=None, ignore_gate=False,
-                             return_alignments=True):
+                             return_alignments=True, attention_window=FROM_ATTRIBUTE):
         """Continuous batching: decode the U utterances of `memory` [U,N,E] through `slots` decoder rows; a row whose utterance
         stops takes the next one of the queue on the device (include/genvox_b200.h, gvx_dec_infer_continuous).  Utterance u
         stops at its first gate over the threshold or after min(max_decoder_steps, frame_caps[u]) frames, and draws the prenet
         dropout of row u + dropout_row_offset.  Returns (mel [U,n_mels,Tmax], gate [U,Tmax], alignments [U,Tmax,N] or None)
         with Tmax = max over utterances of the frame count; frames past an utterance's count are zero.  The counts are left
-        in `self.last_n_frames` (int32 [U], device).  Eval mode only."""
+        in `self.last_n_frames` (int32 [U], device).  Eval mode only.  attention_window: as in `inference`; utterance u
+        then decodes as a static `inference` row with the same window."""
+        win = self._window(attention_window)
         lib = _native.load()
         steps = int(max_decoder_steps if max_decoder_steps is not None else self.max_decoder_steps)
         if self.training:
@@ -283,11 +318,12 @@ class Decoder(nn.Module):
             _native.check(1, "gvx_dec_infer_continuous_workspace_bytes")
         work = _buffer(nbytes, dev)
         ran = C.c_longlong(0)
-        _native.check(lib.gvx_dec_infer_continuous(C.byref(dims), C.byref(weights), _ptr(packed), _ptr(memory), _ptr(lengths), U, N,
-                                                   int(slots), steps, _ptr(caps), float(self.gate_threshold), int(bool(ignore_gate)),
-                                                   self._next_seed(), self.dropout_row_offset, _ptr(mel), _ptr(gate), _ptr(align),
-                                                   _ptr(n_frames), C.byref(ran), _ptr(work), _stream()),
-                      "gvx_dec_infer_continuous")
+        _native.check(lib.gvx_dec_infer_continuous_windowed(C.byref(dims), C.byref(weights), _ptr(packed), _ptr(memory),
+                                                            _ptr(lengths), U, N, int(slots), steps, _ptr(caps),
+                                                            float(self.gate_threshold), int(bool(ignore_gate)), self._next_seed(),
+                                                            self.dropout_row_offset, _ptr(mel), _ptr(gate), _ptr(align),
+                                                            _ptr(n_frames), C.byref(ran), *win, _ptr(work), _stream()),
+                      "gvx_dec_infer_continuous_windowed")
         self.last_n_frames = n_frames
         self.last_steps_run = int(ran.value)
         tmax = int(n_frames.max().item())
@@ -296,15 +332,19 @@ class Decoder(nn.Module):
             print("Warning! Reached max decoder steps")      # tacotron2.py:408
         return mel[:, :, :tmax], gate[:, :tmax], (align[:, :tmax] if align is not None else None)
 
-    def session(self, N, slots=64, capacity=1024, max_decoder_steps=None, ignore_gate=False, return_alignments=True):
+    def session(self, N, slots=64, capacity=1024, max_decoder_steps=None, ignore_gate=False, return_alignments=True,
+                attention_window=FROM_ATTRIBUTE):
         """A decoder session (genvox_b200.session.DecoderSession): `slots` decoder rows kept alive between calls, utterances
         of up to N tokens submitted at any time between calls and decoded through those rows, frames returned per step call.
         Up to `capacity` utterances may wait in its queue.  Utterance `id` decodes bit-identically to row r of a static
         `inference` call with the same slots rows, N, seed and precision, id in row r and dropout_row_offset =
-        id + dropout_row_offset - r.  Eval mode only; the parameters must not change while the session runs."""
+        id + dropout_row_offset - r.  Eval mode only; the parameters must not change while the session runs.
+        attention_window: as in `inference`, fixed for the session's life; the identity then holds against a static call
+        with the same window."""
         from .session import DecoderSession
         return DecoderSession(self, N, slots=slots, capacity=capacity, max_decoder_steps=max_decoder_steps,
-                              ignore_gate=ignore_gate, return_alignments=return_alignments)
+                              ignore_gate=ignore_gate, return_alignments=return_alignments,
+                              attention_window=self.attention_window if attention_window is FROM_ATTRIBUTE else attention_window)
 
 
 def decoder_kwargs_from(ref_decoder):

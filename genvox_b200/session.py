@@ -6,8 +6,9 @@ calls, and `step(k)` runs up to k decoder steps and returns the frames decoded i
 a long decode joins at the next call and its first frames leave after the call it was admitted in.
 
 Contract (as `inference_continuous`): utterance `id` decodes bit-identically to row r of a static `Decoder.inference` call
-with the same `slots` rows, the session's N, the same seed and precision, id in row r and dropout_row_offset =
-id + row_offset - r, whatever the submission times, step counts and other slots were.
+with the same `slots` rows, the session's N, the same seed, precision and attention window (fixed when the session is
+made), id in row r and dropout_row_offset = id + row_offset - r, whatever the submission times, step counts and other
+slots were.
 """
 import ctypes as C
 
@@ -15,13 +16,15 @@ import numpy as np
 import torch
 
 from . import _native
-from .decoder import _buffer, _f32c, _ptr, _stream
+from .decoder import _buffer, _f32c, _ptr, _stream, attention_window_args
 
 
 class DecoderSession:
     """Made by `Decoder.session(...)`.  Eval mode only; the decoder's parameters must not change while it runs."""
 
-    def __init__(self, dec, N, slots=64, capacity=1024, max_decoder_steps=None, ignore_gate=False, return_alignments=True):
+    def __init__(self, dec, N, slots=64, capacity=1024, max_decoder_steps=None, ignore_gate=False, return_alignments=True,
+                 attention_window=None):
+        self._win = attention_window_args(attention_window)       # fixed here: every step call passes the same window
         if dec.training:
             raise RuntimeError("genvox_b200: decoder sessions run in eval mode only (call .eval())")
         steps = int(max_decoder_steps if max_decoder_steps is not None else dec.max_decoder_steps)
@@ -138,10 +141,11 @@ class DecoderSession:
         utt, frame = tags[:4 * K * S].view(torch.int32), tags[4 * K * S:8 * K * S].view(torch.int32)
         last = tags[8 * K * S:].view(torch.int8)
         ran = C.c_int(0)
-        _native.check(self._lib.gvx_dec_session_step(C.byref(self._dims), C.byref(self._weights), _ptr(self._packed),
-                                                     C.byref(self._s), steps, _ptr(frames), _ptr(align), _ptr(utt),
-                                                     _ptr(frame), _ptr(last), C.byref(ran), _ptr(self._work), _stream()),
-                      "gvx_dec_session_step")
+        _native.check(self._lib.gvx_dec_session_step_windowed(C.byref(self._dims), C.byref(self._weights), _ptr(self._packed),
+                                                              C.byref(self._s), steps, _ptr(frames), _ptr(align), _ptr(utt),
+                                                              _ptr(frame), _ptr(last), C.byref(ran), *self._win, _ptr(self._work),
+                                                              _stream()),
+                      "gvx_dec_session_step_windowed")
         n = int(ran.value) * S          # rows [step][slot] written by this call
         if n == 0:
             return {}, {}

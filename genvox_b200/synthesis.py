@@ -22,6 +22,7 @@ for every utterance that finished, the same dictionary.
 """
 import torch
 
+from .decoder import FROM_ATTRIBUTE
 from .training import shard_rows
 
 
@@ -36,16 +37,18 @@ def _as_rows(token_rows, device):
 
 
 @torch.no_grad()
-def batched_inference(model, token_rows, max_batch=64, ignore_gate=False, max_decoder_steps=None):
+def batched_inference(model, token_rows, max_batch=64, ignore_gate=False, max_decoder_steps=None, attention_window=FROM_ATTRIBUTE):
     """`model`: a reference Tacotron2 whose decoder was swapped by `genvox_b200.install` (needs `.embedding`,
     `.encoder.inference`, `.decoder.inference`, `.postnet`).  `token_rows`: sequence of 1-D integer token-id sequences.
     Returns a list (input order) of dicts with the reference's keys (tacotron2.py:492-498):
-    mel_outputs [1,n_mels,T_i], mel_outputs_postnet [1,n_mels,T_i], gate_outputs [1,T_i], alignments [1,T_i,n_tok_i]."""
+    mel_outputs [1,n_mels,T_i], mel_outputs_postnet [1,n_mels,T_i], gate_outputs [1,T_i], alignments [1,T_i,n_tok_i].
+    attention_window goes to `Decoder.inference` (left out: the decoder's `attention_window` attribute)."""
     dev = next(model.parameters()).device
     rows = _as_rows(token_rows, dev)
     # longest first inside every decoder batch (the decoder's mask only needs lengths; sorting keeps batches dense)
     order = sorted(range(len(rows)), key=lambda i: -rows[i].numel())
     out = [None] * len(rows)
+    win = {} if attention_window is FROM_ATTRIBUTE else {"attention_window": attention_window}   # decoders without the option work
     for lo in range(0, len(order), max_batch):
         idx = order[lo:lo + max_batch]
         enc = []
@@ -58,7 +61,7 @@ def batched_inference(model, token_rows, max_batch=64, ignore_gate=False, max_de
         for r, e in enumerate(enc):
             memory[r, :e.shape[1]] = e[0]
         mel, gate, align = model.decoder.inference(memory, memory_lengths=lengths, ignore_gate=ignore_gate,
-                                                   max_decoder_steps=max_decoder_steps)
+                                                   max_decoder_steps=max_decoder_steps, **win)
         n_frames = model.decoder.last_n_frames.tolist()          # one device->host read per batch (reference: one per step)
         for r, i in enumerate(idx):
             t_i, n_i = int(n_frames[r]), int(lengths[r])
@@ -83,8 +86,8 @@ def sharded_inference(model, token_rows, rank, world, **kwargs):
 def continuous_inference(model, token_rows, slots=64, **kw):
     """Like `batched_inference`, but the decoder runs every utterance in one `Decoder.inference_continuous` call through
     `slots` rows, in the order given (utterance i draws prenet dropout row i + dropout_row_offset).  `kw` goes to
-    `inference_continuous` (max_decoder_steps, frame_caps, ignore_gate, return_alignments); "alignments" is None when
-    alignments are not returned."""
+    `inference_continuous` (max_decoder_steps, frame_caps, ignore_gate, return_alignments, attention_window); "alignments"
+    is None when alignments are not returned."""
     dev = next(model.parameters()).device
     rows = _as_rows(token_rows, dev)
     enc = []
@@ -113,7 +116,7 @@ def continuous_inference(model, token_rows, slots=64, **kw):
 class SynthesisSession:
     """Continuous synthesis for requests that arrive over time, around a decoder session (`Decoder.session`) of
     `max_tokens` tokens per utterance and `slots` decoder rows; `kw` goes to `Decoder.session` (capacity,
-    max_decoder_steps, ignore_gate, return_alignments).  Utterance `id` draws prenet dropout row id + dropout_row_offset,
+    max_decoder_steps, ignore_gate, return_alignments, attention_window).  Utterance `id` draws prenet dropout row id + dropout_row_offset,
     so with the same N (= max_tokens) and seed its dictionary equals `continuous_inference`'s for the same token rows."""
 
     def __init__(self, model, max_tokens, slots=64, **kw):

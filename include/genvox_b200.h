@@ -167,6 +167,22 @@ int gvx_dec_infer(const gvx_dims *d, const gvx_weights *w, const void *packed,
                   float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
                   int *steps_run, void *workspace, void *stream);
 
+/* Attention constraint (inference only; ESPnet's use_att_constraint, for any batch).  A window is (att_backward >= 0,
+ * att_forward >= 1); att_forward == 0 means unconstrained, and negative values are refused.  At decoder step t, per row b:
+ *   last = argmax_n w_{t-1}[b, n] over all N tokens, lowest index on ties (as torch.argmax); w_{t-1} is the previous
+ *          step's attention weights, all zero at t = 0 and after a slot admits an utterance, so last = 0 there;
+ *   tokens n < last - att_backward or n >= last + att_forward get energy -inf, in addition to the memory-length mask.
+ * The attended window [max(0, last - att_backward), min(length, last + att_forward)) is never empty.  Softmax, context and
+ * the cumulative weights are unchanged; masked tokens get weight exactly 0.  Teacher-forced forward and BPTT never apply it.
+ * The *_windowed entry points take the arguments of the function they extend plus the window; the plain ones are the
+ * windowed ones with (0, 0), so an unconstrained call is bit-identical and launches the same kernels either way. */
+int gvx_dec_infer_windowed(const gvx_dims *d, const gvx_weights *w, const void *packed,
+                           const float *memory, const int64_t *mem_lengths,
+                           int B, int N, int max_steps, float gate_threshold, int ignore_gate,
+                           uint64_t seed, int training, int row_offset,
+                           float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
+                           int *steps_run, int att_backward, int att_forward, void *workspace, void *stream);
+
 /* Continuous batching: decode a queue of U utterances (all padded to N tokens) through `slots` decoder rows.  Slots start
  * with utterances 0 .. slots-1; when a slot's utterance stops, the slot takes the next utterance of the queue on the device
  * before the next decoder step (slots stopping in the same step take them in slot order), with its recurrent state zeroed.
@@ -175,6 +191,8 @@ int gvx_dec_infer(const gvx_dims *d, const gvx_weights *w, const void *packed,
  * u + row_offset, t = f.  Eval mode only (no LSTM-state dropout).  bf16 mode: slots <= 128.
  * Output identity: utterance u's frames 0 .. n_frames[u]-1 are bit-identical to row r of a gvx_dec_infer call with the same
  * slots rows, N, seed and precision, u in row r and row_offset' = u + row_offset - r; n_frames[u] is that row's stop step.
+ * With an attention window (gvx_dec_infer_continuous_windowed), the identity holds against gvx_dec_infer_windowed with
+ * the same window.
  *   memory [U, N, E]; mem_lengths [U] int64 or NULL; frame_caps [U] int32 or NULL
  *   mel_out [U, n_mels, max_steps], gate_out [U, max_steps], align_out [U, max_steps, N] or NULL, n_frames [U] int32
  *   *steps_run (host) = decoder steps executed (at most ceil(U / slots) * max_steps)
@@ -186,6 +204,12 @@ int gvx_dec_infer_continuous(const gvx_dims *d, const gvx_weights *w, const void
                              uint64_t seed, int row_offset,
                              float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
                              long long *steps_run, void *workspace, void *stream);
+int gvx_dec_infer_continuous_windowed(const gvx_dims *d, const gvx_weights *w, const void *packed,
+                                      const float *memory, const int64_t *mem_lengths, int U, int N, int slots,
+                                      int max_steps, const int32_t *frame_caps, float gate_threshold, int ignore_gate,
+                                      uint64_t seed, int row_offset,
+                                      float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
+                                      long long *steps_run, int att_backward, int att_forward, void *workspace, void *stream);
 
 /* Decoder sessions: continuous batching for requests that arrive over time.  A session holds `slots` decoder rows and their
  * recurrent state in a caller-owned workspace, plus a ring of `capacity` queued utterances (all padded to N tokens).  The
@@ -197,7 +221,8 @@ int gvx_dec_infer_continuous(const gvx_dims *d, const gvx_weights *w, const void
  * Output identity: utterance `id` decodes bit-identically to row r of a gvx_dec_infer call with the same slots rows, N,
  * seed and precision, id in row r and row_offset' = id + row_offset - r, whatever the submission times, the step counts per
  * call and the other slots were; its frame count is that row's stop step (as gvx_dec_infer_continuous, with frame cap
- * min(max_steps, frame_caps[id])). */
+ * min(max_steps, frame_caps[id])).  With an attention window (gvx_dec_session_step_windowed), the identity holds against
+ * gvx_dec_infer_windowed with the same window when every step call of the session passes that window. */
 typedef struct gvx_session {
     /* set by the caller before gvx_dec_session_init */
     int32_t N, slots, capacity, max_steps, ignore_gate, with_alignments, row_offset;
@@ -235,6 +260,10 @@ int gvx_dec_session_submit(const gvx_dims *d, const gvx_weights *w, const void *
 int gvx_dec_session_step(const gvx_dims *d, const gvx_weights *w, const void *packed, gvx_session *s, int max_steps_this_call,
                          float *frames, float *align, int32_t *utt, int32_t *frame, int8_t *last, int *steps_run,
                          void *workspace, void *stream);
+int gvx_dec_session_step_windowed(const gvx_dims *d, const gvx_weights *w, const void *packed, gvx_session *s,
+                                  int max_steps_this_call, float *frames, float *align, int32_t *utt, int32_t *frame,
+                                  int8_t *last, int *steps_run, int att_backward, int att_forward,
+                                  void *workspace, void *stream);
 
 /* ---- single-phase entry points (used by the parity tests to localise a failure) ---- */
 
