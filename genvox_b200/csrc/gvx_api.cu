@@ -1,6 +1,6 @@
-// genvox_b200 — C-ABI entry points: weight repack, teacher-forced forward, batched inference,
-// and the single-phase hooks used by the parity tests.  See include/genvox_b200.h for the
-// contract and the reference file:line each entry point replaces.
+// genvox_b200 — C-ABI entry points: weight repack, teacher-forced forward, and the single-phase
+// hooks used by the parity tests (inference: gvx_infer.cuh and the files after it, same translation
+// unit).  See include/genvox_b200.h for the contract and the reference file:line each entry point replaces.
 #include "../../include/genvox_b200.h"
 #include "gvx_infer_prenet.cuh"
 #include "gvx_attention_c2.cuh"
@@ -20,19 +20,11 @@ thread_local char g_err[512] = {0};
 size_t packed_total_bf16(const Dims &d);
 size_t stash_total_bf16(const Dims &d, int B, int N, int T);
 size_t bwd_total_bf16(const Dims &d, int B, int N, int T);
-size_t infer_total_bf16(const Dims &d, int B, int N, int steps);
 size_t stash_seed_off_bf16(const Dims &d, int B, int N, int T);
-size_t infer_flags_off_bf16(const Dims &d, int B, int N, int steps);
-size_t infer_err_off_bf16(const Dims &d, int B, int N, int steps);
-int check_tc_err_public(int *err_dev, cudaStream_t st, const char *what);
 int pack_weights_bf16(const Dims &d, const gvx_weights *w, float *packed, cudaStream_t st);
 int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const float *mel_in,
                    const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training, int row_offset, float *mel_out,
                    float *gate_out, float *align_out, float *s, cudaStream_t st);
-int infer_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths, int B,
-               int N, int max_steps, float gate_threshold, int ignore_gate, uint64_t seed, int training, int row_offset,
-               float *mel_out, float *gate_out, float *align_out, int32_t *n_frames, int *steps_run, int win_back, int win_fwd,
-               float *s, cudaStream_t st);
 
 int check_dims(const gvx_dims *d) {
     GVX_CHECK(d != nullptr, "dims is null");
@@ -296,11 +288,6 @@ size_t gvx_dec_bwd_workspace_bytes(const gvx_dims *d, int B, int N, int T) {
     if (d->precision == GVX_BF16) return bwd_total_bf16(Dims(*d), B, N, T) * sizeof(float);
     return BwdL(Dims(*d), B, N, T).total * sizeof(float);
 }
-size_t gvx_dec_infer_workspace_bytes(const gvx_dims *d, int B, int N, int max_steps) {
-    if (check_dims(d) || B <= 0 || N <= 0 || max_steps <= 0) return 0;
-    if (d->precision == GVX_BF16) return infer_total_bf16(Dims(*d), B, N, max_steps) * sizeof(float);
-    return InferL(Dims(*d), B, N, max_steps).total * sizeof(float);
-}
 
 static int train_fwd_body(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
                           const float *mel_in, const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training,
@@ -367,108 +354,6 @@ static int train_fwd_body(const gvx_dims *dd, const gvx_weights *w, const void *
     return 0;
 }
 
-// One decoder step of inference (tacotron2.py:398-403): prenet on the previous mel frame `prev` (dropout on, :143), attention
-// LSTM, attention (weights to align_t, row stride align_bstride), decoder LSTM, [mel | gate] projection to out_t.
-// row_frame / row_id: optional per-row prenet dropout frame and row (run_prenet).  win_back / win_fwd: the attention
-// constraint (AttnFwdArgs; win_fwd == 0: off).
-static int infer_step(const Dims &d, const gvx_weights *w, const float *packed, const InferL &L, float *s, const float *memory,
-                      const int64_t *mem_lengths, int B, int N, uint64_t seed, int t, int training, int row_offset,
-                      const int *row_frame, const int *row_id, const float *prev, float *align_t, long long align_bstride,
-                      float *out_t, bool fused_prenet, int win_back, int win_fwd, cudaStream_t st) {
-    const int cur = t & 1, nxt = cur ^ 1;
-    const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H;
-    int *flags = (int *)(s + L.FLAGS);
-    { ProfScope ps(PS_PRENET, st);
-      if (fused_prenet) {
-          GVX_TRY(run_infer_prenet(d, w, prev, d.OL, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, nullptr, (unsigned *)(flags + 40), flags + 41, st,
-                                   row_frame, row_id));
-      } else {
-          GVX_TRY(run_prenet(d, w, prev, d.OL, B, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, st, nullptr, row_frame, row_id));
-      } }
-    LstmIO a;
-    a.x0 = s + L.PRE2; a.w0 = d.P; a.ld0 = d.P;
-    a.x1 = s + L.CTX; a.w1 = d.E; a.ld1 = d.E;
-    a.x2 = s + L.HA + cur * BA; a.w2 = d.A; a.ld2 = d.A;
-    a.c_prev = s + L.CA; a.c_out = s + L.CA; a.h_out = s + L.HA + nxt * BA; a.gates_out = nullptr;
-    { ProfScope ps(PS_ATT_LSTM, st); GVX_TRY(run_lstm(d, packed, 0, a, B, seed, t, training, row_offset, st)); }
-    { ProfScope ps(PS_QUERY, st); GVX_TRY(run_query(d, w, s + L.HA + nxt * BA, B, s + L.Q, st)); }
-    { ProfScope ps(PS_ATTENTION, st);
-      GVX_TRY(run_attention(d, w, packed, s + L.Q, s + L.PM, memory, mem_lengths, B, N, s + L.WPREV, s + L.CUM,
-                            align_t, align_bstride, nullptr, s + L.CTX, nullptr, nullptr, st, win_back, win_fwd)); }
-    LstmIO c;
-    c.x0 = s + L.HA + nxt * BA; c.w0 = d.A; c.ld0 = d.A;
-    c.x1 = s + L.CTX; c.w1 = d.E; c.ld1 = d.E;
-    c.x2 = s + L.HD + cur * BH; c.w2 = d.H; c.ld2 = d.H;
-    c.c_prev = s + L.CD; c.c_out = s + L.CD; c.h_out = s + L.HD + nxt * BH; c.gates_out = nullptr;
-    { ProfScope ps(PS_DEC_LSTM, st); GVX_TRY(run_lstm(d, packed, 1, c, B, seed, t, training, row_offset, st)); }
-    { ProfScope ps(PS_PROJ, st); GVX_TRY(run_projection(d, packed, s + L.HD + nxt * BH, d.H, s + L.CTX, d.E, B, out_t, st, true)); }
-    return 0;
-}
-
-static int infer_body(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
-                      const int64_t *mem_lengths, int B, int N, int max_steps, float gate_threshold, int ignore_gate,
-                      uint64_t seed, int training, int row_offset, float *mel_out, float *gate_out, float *align_out,
-                      int32_t *n_frames, int *steps_run, int win_back, int win_fwd, void *workspace, void *stream) {
-    const Dims d(*dd);
-    if (dd->precision == GVX_BF16)
-        return infer_bf16(d, w, (const float *)packed_, memory, mem_lengths, B, N, max_steps, gate_threshold, ignore_gate, seed,
-                          training, row_offset, mel_out, gate_out, align_out, n_frames, steps_run, win_back, win_fwd,
-                          (float *)workspace, (cudaStream_t)stream);
-    const InferL L(d, B, N, max_steps);
-    const float *packed = (const float *)packed_;
-    float *s = (float *)workspace;
-    cudaStream_t st = (cudaStream_t)stream;
-    const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H;
-    int *flags = (int *)(s + L.FLAGS);
-
-    GVX_TRY(run_processed_memory(d, w, memory, B, N, s + L.PM, st));
-    GVX_CUDA(cudaMemsetAsync(s + L.HA, 0, 2 * BA * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.CA, 0, BA * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.HD, 0, 2 * BH * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.CD, 0, BH * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.CTX, 0, (size_t)B * d.E * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.WPREV, 0, (size_t)B * N * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.CUM, 0, (size_t)B * N * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.ZERO, 0, (size_t)B * d.OL * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(flags, 0, 32 * sizeof(int), st));       // [0] rows still running; [32..33] hold the dropout seed (gvx_dec_infer)
-    GVX_CUDA(cudaMemsetAsync(flags + 40, 0, 2 * sizeof(int), st));   // [40] prenet grid barrier, [41] its error word
-    k_fill_i32<<<grid_for(B), 256, 0, st>>>(n_frames, B, ignore_gate ? max_steps : -1, 0);
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    const bool fused_prenet = infer_prenet_fused_ok(d, B);
-
-    int t = 0, host_running = B;
-    pdl_barrier_next();
-    for (; t < max_steps; ++t) {
-        const float *prev = t == 0 ? s + L.ZERO : s + L.OUT + (size_t)(t - 1) * B * d.OL;
-        float *out_t = s + L.OUT + (size_t)t * B * d.OL;
-        GVX_TRY(infer_step(d, w, packed, L, s, memory, mem_lengths, B, N, seed, t, training, row_offset, nullptr, nullptr, prev,
-                           align_out + (size_t)t * N, (long long)max_steps * N, out_t, fused_prenet, win_back, win_fwd, st));
-        if (!ignore_gate) {
-            GVX_CUDA(launch_pdl(k_gate_check, dim3(1), dim3(128), 0, st, (const float *)out_t, B, d.M, d.OL, gate_threshold, t, n_frames, flags));
-    GVX_LAUNCHED(1);
-            GVX_CUDA(cudaGetLastError());
-            if ((t + 1) % GVX_STOP_POLL == 0 || t + 1 == max_steps) {
-                GVX_CUDA(cudaMemcpyAsync(&host_running, flags, sizeof(int), cudaMemcpyDeviceToHost, st));
-                GVX_CUDA(cudaStreamSynchronize(st));
-                if (host_running == 0) { ++t; break; }
-            }
-        }
-    }
-    const int steps = t < max_steps ? t : max_steps;
-    if (!ignore_gate) {   // rows that never fired stop at max_decoder_steps (tacotron2.py:407)
-        k_fill_i32<<<grid_for(B), 256, 0, st>>>(n_frames, B, steps, 1);
-    GVX_LAUNCHED(1);
-        GVX_CUDA(cudaGetLastError());
-    }
-    k_unpack_out<<<grid_for((size_t)B * (d.M + 1) * steps), 256, 0, st>>>(s + L.OUT, B, d.M, d.OL, steps, max_steps, mel_out,
-                                                                         gate_out);
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    *steps_run = steps;
-    return 0;
-}
-
 // ---------------------------------------------------------------- graph-cached entry points
 static uint32_t *seed_slot_train(const gvx_dims *dd, void *stash, int B, int N, int T) {
     const Dims d(*dd);
@@ -502,57 +387,6 @@ int gvx_dec_train_fwd(const gvx_dims *dd, const gvx_weights *w, const void *pack
     });
     g_seed_ptr = nullptr;
     return rc;
-}
-
-int gvx_dec_infer_windowed(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
-                           const int64_t *mem_lengths, int B, int N, int max_steps, float gate_threshold, int ignore_gate,
-                           uint64_t seed, int training, int row_offset, float *mel_out, float *gate_out, float *align_out,
-                           int32_t *n_frames, int *steps_run, int att_backward, int att_forward, void *workspace, void *stream) {
-    GVX_TRY(check_dims(dd));
-    GVX_CHECK(w && packed_ && memory && mel_out && gate_out && align_out && n_frames && steps_run && workspace,
-              "null argument");
-    GVX_CHECK(B > 0 && N > 0 && max_steps > 0, "B, N, max_steps must be positive");
-    GVX_TRY(check_window(att_backward, att_forward));
-    GVX_TRY(latch_check());
-    cudaStream_t user = (cudaStream_t)stream;
-    const Dims d(*dd);
-    const bool bf = dd->precision == GVX_BF16;
-    const size_t flags_off = bf ? infer_flags_off_bf16(d, B, N, max_steps) : InferL(d, B, N, max_steps).FLAGS;
-    // the seed slot sits behind the stop flags; the drivers only clear the first 32 ints of that block
-    uint32_t *slot = reinterpret_cast<uint32_t *>((float *)workspace + flags_off) + 32;
-    GVX_TRY(put_seed(slot, seed, user));
-    g_seed_ptr = slot;
-    int rc;
-    if (ignore_gate) {          // fixed step count: no host polling inside, the whole sequence is one graph
-        KeyBuilder kb;
-        kb.add((int)3).add(*dd).add(*w).add(packed_).add(memory).add(mem_lengths).add(B).add(N).add(max_steps).add(gate_threshold)
-            .add(training).add(row_offset).add(mel_out).add(gate_out).add(align_out).add(n_frames).add(workspace)
-            .add(att_backward).add(att_forward);       // baked into the captured attention launches
-        rc = run_cached(kb.k, user, [&](cudaStream_t st) {
-            return infer_body(dd, w, packed_, memory, mem_lengths, B, N, max_steps, gate_threshold, ignore_gate, seed, training,
-                              row_offset, mel_out, gate_out, align_out, n_frames, steps_run, att_backward, att_forward, workspace,
-                              (void *)st);
-        });
-        *steps_run = max_steps;
-    } else {
-        rc = infer_body(dd, w, packed_, memory, mem_lengths, B, N, max_steps, gate_threshold, ignore_gate, seed, training,
-                        row_offset, mel_out, gate_out, align_out, n_frames, steps_run, att_backward, att_forward, workspace, stream);
-    }
-    g_seed_ptr = nullptr;
-    if (rc == 0 && bf)
-        rc = check_tc_err_public(reinterpret_cast<int *>((float *)workspace + infer_err_off_bf16(d, B, N, max_steps)), user,
-                                 "gvx_dec_infer");
-    if (rc == 0 && !bf)      // error word of the fused inference prenet's grid barrier (gvx_infer_prenet.cuh)
-        rc = check_tc_err_public(reinterpret_cast<int *>((float *)workspace + flags_off) + 41, user, "gvx_dec_infer (prenet barrier)");
-    return rc;
-}
-
-int gvx_dec_infer(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
-                  const int64_t *mem_lengths, int B, int N, int max_steps, float gate_threshold, int ignore_gate,
-                  uint64_t seed, int training, int row_offset, float *mel_out, float *gate_out, float *align_out,
-                  int32_t *n_frames, int *steps_run, void *workspace, void *stream) {
-    return gvx_dec_infer_windowed(dd, w, packed_, memory, mem_lengths, B, N, max_steps, gate_threshold, ignore_gate, seed, training,
-                                  row_offset, mel_out, gate_out, align_out, n_frames, steps_run, 0, 0, workspace, stream);
 }
 
 int gvx_device_error(int clear) {
@@ -647,5 +481,6 @@ int gvx_attention_step(const gvx_dims *dd, const gvx_weights *w, const void *pac
 // backward through time (gvx_dec_train_bwd) lives in its own file, same translation unit
 #include "gvx_bwd.cuh"
 #include "gvx_bf16_api.cuh"
+#include "gvx_infer.cuh"
 #include "gvx_continuous.cuh"
 #include "gvx_session.cuh"

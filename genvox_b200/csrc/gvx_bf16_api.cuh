@@ -822,18 +822,14 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
 }
 
 // ======================================================================================= inference
-// One decoder step (tacotron2.py:398-403): prenet on the previous mel frame `prev` (straight into the attention-LSTM operand
-// image), attention LSTM, query, attention (weights to align_t, row stride align_bstride), decoder LSTM, [mel | gate] projection
-// to out_t.  row_frame / row_id: optional per-row prenet dropout frame and row (run_infer_prenet, run_prenet).  win_back /
-// win_fwd: the attention constraint (AttnFwdArgs; win_fwd == 0: off).
-static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *packed, const InferBfL &L, float *s, const float *memory,
-                           const int64_t *mem_lengths, int B, int N, uint64_t seed, int t, int training, int row_offset,
-                           const int *row_frame, const int *row_id, const float *prev, float *align_t, long long align_bstride,
-                           float *out_t, int win_back, int win_fwd, cudaStream_t st) {
+// One decoder step (tacotron2.py:398-403): prenet on the previous mel frame io.prev (straight into the attention-LSTM operand
+// image), attention LSTM, query, attention, decoder LSTM, [mel | gate] projection to io.out_t.
+static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *packed, const InferBfL &L, float *s, int B, int N,
+                           bool fused_prenet, const InferStepArgs &io, cudaStream_t st) {
     const BfGeom g(d);
     const PackedL PL(d);
     const PackedBfL BL(d, PL.total);
-    const int NPAD = L.NPAD;
+    const int NPAD = L.NPAD, t = io.t;
     bf16 *XAI = (bf16 *)(s + L.XAI), *XDI = (bf16 *)(s + L.XDI), *XPI = (bf16 *)(s + L.XPI);
     int *err = (int *)(s + L.ERR), *flags = (int *)(s + L.FLAGS);
     const bf16 *WaI = (const bf16 *)(packed + BL.WaI), *WdI = (const bf16 *)(packed + BL.WdI), *WqI = (const bf16 *)(packed + BL.WqI),
@@ -845,11 +841,12 @@ static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *pac
         BfDsts bf;
         memset(&bf, 0, sizeof(bf));
         add_img(bf, xa, 0, NPAD);
-        if (infer_prenet_fused_ok(d, B)) {
-            GVX_TRY(run_infer_prenet(d, w, prev, d.OL, B, seed, t, row_offset, s + L.PRE1, nullptr, &bf, (unsigned *)(flags + 40), err, st,
-                                     row_frame, row_id));
+        if (fused_prenet) {
+            GVX_TRY(run_infer_prenet(d, w, io.prev, d.OL, B, io.seed, t, io.row_offset, s + L.PRE1, nullptr, &bf, (unsigned *)(flags + 40),
+                                     err, st, io.row_frame, io.row_id));
         } else {
-            GVX_TRY(run_prenet(d, w, prev, d.OL, B, B, seed, t, row_offset, s + L.PRE1, s + L.PRE2, st, &bf, row_frame, row_id));
+            GVX_TRY(run_prenet(d, w, io.prev, d.OL, B, B, io.seed, t, io.row_offset, s + L.PRE1, s + L.PRE2, st, &bf, io.row_frame,
+                               io.row_id));
         }
     }
     {
@@ -857,8 +854,8 @@ static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *pac
         BfDsts h;
         memset(&h, 0, sizeof(h));
         add_img(h, xd, 0, NPAD); add_img(h, xa_n, d.P + d.E, NPAD);
-        GVX_TRY(run_lstm_bf16(d, packed, 0, WaI, xa, s + L.PA, L.KSa, g.Ta, g.Kpa, s + L.CA, s + L.CA, nullptr, h, B, seed, t,
-                              training, row_offset, err, st));
+        GVX_TRY(run_lstm_bf16(d, packed, 0, WaI, xa, s + L.PA, L.KSa, g.Ta, g.Kpa, s + L.CA, s + L.CA, nullptr, h, B, io.seed, t,
+                              io.training, io.row_offset, err, st));
     }
     {
         ProfScope ps(PS_QUERY, st);
@@ -870,12 +867,12 @@ static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *pac
         memset(&a, 0, sizeof(a));
         a.s = AttnShape{B, N, d.D, d.E, d.F, d.KS};
         a.q = src_split(s + L.PQ, g.Tq * TC_M, L.KSq, (long long)B * g.Tq * TC_M);
-        a.pm = s + L.PM; a.memory = memory;
-        a.wlc = w->loc_conv_w; a.wldT = packed + PL.wldT; a.v = w->v_w; a.lengths = mem_lengths;
+        a.pm = s + L.PM; a.memory = io.memory;
+        a.wlc = w->loc_conv_w; a.wldT = packed + PL.wldT; a.v = w->v_w; a.lengths = io.lengths;
         a.w_prev = s + L.WPREV; a.cum = s + L.CUM;
-        a.align_out = align_t; a.align_bstride = align_bstride;
+        a.align_out = io.align_t; a.align_bstride = io.align_bstride;
         a.ctx_ld = d.E;
-        a.win_back = win_back; a.win_fwd = win_fwd;
+        a.win_back = io.win_back; a.win_fwd = io.win_fwd;
         add_img(a.ctx_bf, xd, d.A, NPAD); add_img(a.ctx_bf, xa_n, d.P, NPAD); add_img(a.ctx_bf, XPI, d.H, NPAD);
         GVX_TRY(launch_attention_fwd_best(a, st));
     }
@@ -884,85 +881,24 @@ static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *pac
         BfDsts h;
         memset(&h, 0, sizeof(h));
         add_img(h, XPI, 0, NPAD); add_img(h, xd_n, d.A + d.E, NPAD);
-        GVX_TRY(run_lstm_bf16(d, packed, 1, WdI, xd, s + L.PD, L.KSd, g.Td, g.Kpd, s + L.CD, s + L.CD, nullptr, h, B, seed, t,
-                              training, row_offset, err, st));
+        GVX_TRY(run_lstm_bf16(d, packed, 1, WdI, xd, s + L.PD, L.KSd, g.Td, g.Kpd, s + L.CD, s + L.CD, nullptr, h, B, io.seed, t,
+                              io.training, io.row_offset, err, st));
     }
     {
         ProfScope ps(PS_PROJ, st);
         GVX_TRY(run_tc(WpgI, XPI, s + L.PP, g.Tp, g.Kpp, L.KSp, B, err, st));
         GVX_CUDA(launch_pdl(k_bf_finalize, dim3(grid_for((size_t)B * (d.M + 1))), dim3(256), 0, st, (const float *)(s + L.PP), L.KSp,
-                            B, g.Tp * TC_M, d.M + 1, (const float *)(packed + PL.bpg), out_t, d.OL));
+                            B, g.Tp * TC_M, d.M + 1, (const float *)(packed + PL.bpg), io.out_t, d.OL));
         GVX_LAUNCHED(1);
         GVX_CUDA(cudaGetLastError());
     }
     return 0;
 }
 
-int infer_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
-                      int B, int N, int max_steps, float gate_threshold, int ignore_gate, uint64_t seed, int training,
-                      int row_offset, float *mel_out, float *gate_out, float *align_out, int32_t *n_frames, int *steps_run,
-                      int win_back, int win_fwd, float *s, cudaStream_t st) {
-    GVX_TRY(check_bf16_dims(d, B));
-    const BfGeom g(d);
-    const InferBfL L(d, B, N, max_steps);
-    const int NPAD = L.NPAD;
-    bf16 *XAI = (bf16 *)(s + L.XAI), *XDI = (bf16 *)(s + L.XDI), *XPI = (bf16 *)(s + L.XPI);
-    int *err = (int *)(s + L.ERR), *flags = (int *)(s + L.FLAGS);
-
-    GVX_TRY(run_processed_memory(d, w, memory, B, N, s + L.PM, st));
-    GVX_CUDA(cudaMemsetAsync(err, 0, 64 * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(flags, 0, 32 * sizeof(int), st));       // [0] rows still running; [32..33] hold the dropout seed (gvx_dec_infer)
-    GVX_CUDA(cudaMemsetAsync(flags + 40, 0, 2 * sizeof(int), st));   // [40] prenet grid barrier
-    GVX_CUDA(cudaMemsetAsync(XAI, 0, 2 * L.xai_stride * sizeof(bf16), st));
-    GVX_CUDA(cudaMemsetAsync(XDI, 0, 2 * L.xdi_stride * sizeof(bf16), st));
-    GVX_CUDA(cudaMemsetAsync(XPI, 0, (size_t)g.Kpp * NPAD * sizeof(bf16), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.CA, 0, (size_t)B * d.A * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.CD, 0, (size_t)B * d.H * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.WPREV, 0, (size_t)B * N * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.CUM, 0, (size_t)B * N * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + L.ZERO, 0, (size_t)B * d.OL * sizeof(float), st));
-    k_fill_i32<<<grid_for(B), 256, 0, st>>>(n_frames, B, ignore_gate ? max_steps : -1, 0);
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-
-    int t = 0, host_running = B;
-    pdl_barrier_next();
-    for (; t < max_steps; ++t) {
-        const float *prev = t == 0 ? s + L.ZERO : s + L.OUT + (size_t)(t - 1) * B * d.OL;
-        float *out_t = s + L.OUT + (size_t)t * B * d.OL;
-        GVX_TRY(infer_step_bf16(d, w, packed, L, s, memory, mem_lengths, B, N, seed, t, training, row_offset, nullptr, nullptr, prev,
-                                align_out + (size_t)t * N, (long long)max_steps * N, out_t, win_back, win_fwd, st));
-        if (!ignore_gate) {
-            GVX_CUDA(launch_pdl(k_gate_check, dim3(1), dim3(128), 0, st, (const float *)out_t, B, d.M, d.OL, gate_threshold, t, n_frames, flags));
-            GVX_LAUNCHED(1);
-            GVX_CUDA(cudaGetLastError());
-            if ((t + 1) % GVX_STOP_POLL == 0 || t + 1 == max_steps) {
-                GVX_CUDA(cudaMemcpyAsync(&host_running, flags, sizeof(int), cudaMemcpyDeviceToHost, st));
-                GVX_CUDA(cudaStreamSynchronize(st));
-                if (host_running == 0) { ++t; break; }
-            }
-        }
-    }
-    const int steps = t < max_steps ? t : max_steps;
-    if (!ignore_gate) {
-        k_fill_i32<<<grid_for(B), 256, 0, st>>>(n_frames, B, steps, 1);
-        GVX_LAUNCHED(1);
-    }
-    k_unpack_out<<<grid_for((size_t)B * (d.M + 1) * steps), 256, 0, st>>>(s + L.OUT, B, d.M, d.OL, steps, max_steps, mel_out, gate_out);
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    *steps_run = steps;
-    return 0;
-}
-
 size_t packed_total_bf16(const Dims &d) { return PackedBfL(d, PackedL(d).total).total; }
 size_t stash_total_bf16(const Dims &d, int B, int N, int T) { return StashBfL(d, B, N, T).total; }
 size_t bwd_total_bf16(const Dims &d, int B, int N, int T) { return BwdBfL(d, B, N, T).total; }
-size_t infer_total_bf16(const Dims &d, int B, int N, int steps) { return InferBfL(d, B, N, steps).total; }
 size_t stash_seed_off_bf16(const Dims &d, int B, int N, int T) { return StashBfL(d, B, N, T).SEED; }
-size_t infer_flags_off_bf16(const Dims &d, int B, int N, int steps) { return InferBfL(d, B, N, steps).FLAGS; }
-size_t infer_err_off_bf16(const Dims &d, int B, int N, int steps) { return InferBfL(d, B, N, steps).ERR; }
-int check_tc_err_public(int *err_dev, cudaStream_t st, const char *what) { return check_tc_err(err_dev, st, what); }
 
 }  // namespace gvx
 

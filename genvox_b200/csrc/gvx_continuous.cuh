@@ -12,11 +12,11 @@
 // in the layout it lives in, its memory / processed memory / length are replaced, and the prenet draws its dropout at
 // Philox (row u + row_offset, t = local frame) through the per-row row_frame / row_id arrays.
 #pragma once
-#include "gvx_bf16_api.cuh"
+#include "gvx_infer.cuh"
 
 namespace gvx {
 
-// ---- workspace: the static inference layout for S rows and a two-frame output ring (steps = 2), then this block
+// ---- workspace: the inference plan's layout for S rows and a two-frame output ring (steps = 2), then this block
 struct ContL {
     size_t MEM, PMQ, ALIGN, LEN, ST, total;
     ContL(const Dims &d, size_t base, int U, int N, int S) {
@@ -192,42 +192,20 @@ __global__ void k_slot_start(int S, int U, int N, const int64_t *__restrict__ le
     }
 }
 
-inline size_t continuous_base(const Dims &d, bool bf, int S, int N) {
-    return bf ? InferBfL(d, S, N, 2).total : InferL(d, S, N, 2).total;
+// admission resets a slot's rows of the plan's recurrent state (InferPlan::state)
+inline void admit_state(AdmitArgs &a, const InferPlan &P, float *s) {
+    P.state(s, [&](float *p, int width) { a.zero[a.nzero] = p; a.zero_w[a.nzero] = width; ++a.nzero; },
+            [&](bf16 *p, int kpad) { a.img[a.nimg] = p; a.img_k[a.nimg] = kpad; ++a.nimg; a.npad = P.Lb.NPAD; });
 }
 
-// the per-row recurrent state an admission zeroes, in the layout it lives in: fp32 h/c of both LSTMs, ctx, attention weights
-// and cumulative weights; in bf16 mode the cell states, attention weights and the slot's rows of the tcgen05 operand images
-inline void admit_state(AdmitArgs &a, const Dims &d, bool bf, const InferL &Lf, const InferBfL &Lb, float *s, int S, int N) {
-    auto zrow = [&](float *p, int width) { a.zero[a.nzero] = p; a.zero_w[a.nzero] = width; ++a.nzero; };
-    if (bf) {
-        const BfGeom g(d);
-        zrow(s + Lb.CA, d.A); zrow(s + Lb.CD, d.H); zrow(s + Lb.WPREV, N); zrow(s + Lb.CUM, N);
-        bf16 *XAI = (bf16 *)(s + Lb.XAI), *XDI = (bf16 *)(s + Lb.XDI);
-        a.img[0] = XAI; a.img[1] = XAI + Lb.xai_stride; a.img_k[0] = a.img_k[1] = g.Kpa;
-        a.img[2] = XDI; a.img[3] = XDI + Lb.xdi_stride; a.img_k[2] = a.img_k[3] = g.Kpd;
-        a.img[4] = (bf16 *)(s + Lb.XPI); a.img_k[4] = g.Kpp;
-        a.nimg = 5;
-        a.npad = Lb.NPAD;
-    } else {
-        zrow(s + Lf.HA, d.A); zrow(s + Lf.HA + (size_t)S * d.A, d.A); zrow(s + Lf.CA, d.A);
-        zrow(s + Lf.HD, d.H); zrow(s + Lf.HD + (size_t)S * d.H, d.H); zrow(s + Lf.CD, d.H);
-        zrow(s + Lf.CTX, d.E); zrow(s + Lf.WPREV, N); zrow(s + Lf.CUM, N);
-    }
-}
-
-int infer_continuous(const gvx_dims *dd, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
-                     int U, int N, int S, int max_steps, const int32_t *frame_caps, float gate_threshold, int ignore_gate,
-                     uint64_t seed, int row_offset, float *mel_out, float *gate_out, float *align_out, int32_t *n_frames,
-                     long long *steps_run, int win_back, int win_fwd, float *s, cudaStream_t st) {
-    const Dims d(*dd);
-    const bool bf = dd->precision == GVX_BF16;
-    if (bf) GVX_TRY(check_bf16_dims(d, S));
-    const InferL Lf(d, S, N, 2);
-    const InferBfL Lb(d, S, N, 2);
-    const ContL C(d, continuous_base(d, bf, S, N), U, N, S);
-    const size_t PM = bf ? Lb.PM : Lf.PM, OUT = bf ? Lb.OUT : Lf.OUT, FLAGS = bf ? Lb.FLAGS : Lf.FLAGS;
-    int *flags = (int *)(s + FLAGS), *state = (int *)(s + C.ST);
+int infer_continuous(const InferPlan &P, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
+                     int U, int max_steps, const int32_t *frame_caps, float gate_threshold, int ignore_gate, uint64_t seed,
+                     int row_offset, float *mel_out, float *gate_out, float *align_out, int32_t *n_frames, long long *steps_run,
+                     int win_back, int win_fwd, float *s, cudaStream_t st) {
+    const Dims &d = P.d;
+    const int S = P.B, N = P.N;
+    const ContL C(d, P.total, U, N, S);
+    int *flags = P.flags(s), *state = (int *)(s + C.ST);
     int64_t *len_slot = (int64_t *)(s + C.LEN);
     float *mem_slot = s + C.MEM;
     const size_t SNE = (size_t)S * N * d.E;
@@ -247,7 +225,7 @@ int infer_continuous(const gvx_dims *dd, const gvx_weights *w, const float *pack
     const int first = U < S ? U : S;
     GVX_CUDA(cudaMemsetAsync(mem_slot, 0, SNE * sizeof(float), st));
     GVX_CUDA(cudaMemcpyAsync(mem_slot, memory, (size_t)first * N * d.E * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    GVX_CUDA(cudaMemcpyAsync(s + PM, s + C.PMQ, (size_t)S * N * d.D * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    GVX_CUDA(cudaMemcpyAsync(s + P.PM, s + C.PMQ, (size_t)S * N * d.D * sizeof(float), cudaMemcpyDeviceToDevice, st));
     k_slot_start<<<grid_for(S), 256, 0, st>>>(S, U, N, mem_lengths, len_slot, state);
     GVX_LAUNCHED(1);
     k_fill_i32<<<grid_for(U), 256, 0, st>>>(n_frames, U, 0, 0);
@@ -255,28 +233,23 @@ int infer_continuous(const gvx_dims *dd, const gvx_weights *w, const float *pack
     GVX_CUDA(cudaGetLastError());
 
     // recurrent state: zero at the start, and per row at every admission (k_gate_admit)
+    GVX_TRY(P.reset(s, st));
+    GVX_CUDA(cudaMemsetAsync(s + P.OUT, 0, (size_t)2 * S * d.OL * sizeof(float), st));     // the previous-frame ring: go frames
     AdmitArgs a;
     memset(&a, 0, sizeof(a));
-    admit_state(a, d, bf, Lf, Lb, s, S, N);
-    if (bf) {
-        const BfGeom g(d);
-        GVX_CUDA(cudaMemsetAsync(s + Lb.ERR, 0, 64 * sizeof(float), st));
-        GVX_CUDA(cudaMemsetAsync(a.img[0], 0, 2 * Lb.xai_stride * sizeof(bf16), st));
-        GVX_CUDA(cudaMemsetAsync(a.img[2], 0, 2 * Lb.xdi_stride * sizeof(bf16), st));
-        GVX_CUDA(cudaMemsetAsync(a.img[4], 0, (size_t)g.Kpp * Lb.NPAD * sizeof(bf16), st));
-    }
-    for (int z = 0; z < a.nzero; ++z) GVX_CUDA(cudaMemsetAsync(a.zero[z], 0, (size_t)S * a.zero_w[z] * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + OUT, 0, (size_t)2 * S * d.OL * sizeof(float), st));     // the previous-frame ring: go frames
-    GVX_CUDA(cudaMemsetAsync(flags, 0, 32 * sizeof(int), st));       // [0] active slots; [32..33] hold the dropout seed
-    GVX_CUDA(cudaMemsetAsync(flags + 40, 0, 2 * sizeof(int), st));   // [40] prenet grid barrier, [41] its error word
-
+    admit_state(a, P, s);
     a.align_t = s + C.ALIGN;
     a.memory = memory; a.pmq = s + C.PMQ; a.lengths = mem_lengths; a.caps = frame_caps;
-    a.mem_slot = mem_slot; a.pm_slot = s + PM; a.len_slot = len_slot;
+    a.mem_slot = mem_slot; a.pm_slot = s + P.PM; a.len_slot = len_slot;
     a.mel_out = mel_out; a.gate_out = gate_out; a.align_out = align_out; a.n_frames = n_frames; a.flags = flags;
     a.thr = gate_threshold;
     a.ignore_gate = ignore_gate; a.S = S; a.U = U; a.N = N; a.E = d.E; a.D = d.D; a.M = d.M; a.OL = d.OL; a.max_steps = max_steps;
-    const bool fused_prenet = infer_prenet_fused_ok(d, S);
+    InferStepArgs io;
+    memset(&io, 0, sizeof(io));
+    io.memory = mem_slot; io.lengths = len_slot;
+    io.align_t = s + C.ALIGN; io.align_bstride = N;
+    io.seed = seed; io.row_offset = row_offset;
+    io.win_back = win_back; io.win_fwd = win_fwd;
 
     // every slot runs at most ceil(U/S) utterances' worth of max_steps before the queue is empty and its last one stops
     const long long bound = (long long)((U + S - 1) / S) * max_steps;
@@ -284,17 +257,16 @@ int infer_continuous(const gvx_dims *dd, const gvx_weights *w, const float *pack
     int host_running = first;
     for (; t < bound; ++t) {
         const int p = (int)(t & 1);
-        const float *prev = s + OUT + (size_t)(p ^ 1) * S * d.OL;
-        float *out_t = s + OUT + (size_t)p * S * d.OL;
         int *utt = state + p * S, *frame = state + 2 * S + p * S;
+        io.t = (int)t;
+        io.row_frame = frame; io.row_id = utt;
+        io.prev = s + P.OUT + (size_t)(p ^ 1) * S * d.OL;
+        io.out_t = s + P.OUT + (size_t)p * S * d.OL;
         // full dependency on the previous step's k_gate_admit: kernels of the chain read the lengths and prefetch the
         // processed memory before griddepcontrol.wait, and an admission rewrites both
         pdl_barrier_next();
-        if (bf) GVX_TRY(infer_step_bf16(d, w, packed, Lb, s, mem_slot, len_slot, S, N, seed, (int)t, 0, row_offset, frame, utt, prev,
-                                        s + C.ALIGN, (long long)N, out_t, win_back, win_fwd, st));
-        else GVX_TRY(infer_step(d, w, packed, Lf, s, mem_slot, len_slot, S, N, seed, (int)t, 0, row_offset, frame, utt, prev,
-                                s + C.ALIGN, (long long)N, out_t, fused_prenet, win_back, win_fwd, st));
-        a.out_t = out_t;
+        GVX_TRY(P.step(w, packed, s, io, st));
+        a.out_t = io.out_t;
         a.utt_cur = utt; a.frame_cur = frame; a.next_cur = state + 4 * S + p;
         a.utt_nxt = state + (p ^ 1) * S; a.frame_nxt = state + 2 * S + (p ^ 1) * S; a.next_nxt = state + 4 * S + (p ^ 1);
         GVX_CUDA(launch_pdl(k_gate_admit, dim3(S), dim3(ADMIT_THREADS), 0, st, a));
@@ -318,10 +290,9 @@ extern "C" {
 size_t gvx_dec_infer_continuous_workspace_bytes(const gvx_dims *d, int U, int N, int slots) {
     using namespace gvx;
     if (check_dims(d) || U <= 0 || N <= 0 || slots <= 0) return 0;
-    const Dims dm(*d);
-    const bool bf = d->precision == GVX_BF16;
-    if (bf && check_bf16_dims(dm, slots)) return 0;
-    return ContL(dm, continuous_base(dm, bf, slots, N), U, N, slots).total * sizeof(float);
+    const InferPlan P(*d, slots, N, 2);
+    if (P.bf && check_bf16_dims(P.d, slots)) return 0;
+    return ContL(P.d, P.total, U, N, slots).total * sizeof(float);
 }
 
 int gvx_dec_infer_continuous_windowed(const gvx_dims *dd, const gvx_weights *w, const void *packed, const float *memory,
@@ -335,25 +306,14 @@ int gvx_dec_infer_continuous_windowed(const gvx_dims *dd, const gvx_weights *w, 
     GVX_CHECK(U > 0 && N > 0 && slots > 0 && max_steps > 0, "U, N, slots, max_steps must be positive");
     GVX_TRY(check_window(att_backward, att_forward));
     GVX_TRY(latch_check());
+    const InferPlan P(*dd, slots, N, 2);
+    if (P.bf) GVX_TRY(check_bf16_dims(P.d, slots));
     cudaStream_t st = (cudaStream_t)stream;
-    const Dims d(*dd);
-    const bool bf = dd->precision == GVX_BF16;
-    if (bf) GVX_TRY(check_bf16_dims(d, slots));
-    const size_t flags_off = bf ? InferBfL(d, slots, N, 2).FLAGS : InferL(d, slots, N, 2).FLAGS;
-    uint32_t *slot = reinterpret_cast<uint32_t *>((float *)workspace + flags_off) + 32;
-    GVX_TRY(put_seed(slot, seed, st));
-    g_seed_ptr = slot;
-    int rc = infer_continuous(dd, w, (const float *)packed, memory, mem_lengths, U, N, slots, max_steps, frame_caps, gate_threshold,
-                              ignore_gate, seed, row_offset, mel_out, gate_out, align_out, n_frames, steps_run, att_backward, att_forward,
-                              (float *)workspace, st);
-    g_seed_ptr = nullptr;
-    if (rc == 0 && bf)
-        rc = check_tc_err_public(reinterpret_cast<int *>((float *)workspace + InferBfL(d, slots, N, 2).ERR), st,
-                                 "gvx_dec_infer_continuous");
-    if (rc == 0 && !bf)
-        rc = check_tc_err_public(reinterpret_cast<int *>((float *)workspace + flags_off) + 41, st,
-                                 "gvx_dec_infer_continuous (prenet barrier)");
-    return rc;
+    float *s = (float *)workspace;
+    return infer_call(P, s, true, seed, st, "gvx_dec_infer_continuous", [&] {
+        return infer_continuous(P, w, (const float *)packed, memory, mem_lengths, U, max_steps, frame_caps, gate_threshold, ignore_gate,
+                                seed, row_offset, mel_out, gate_out, align_out, n_frames, steps_run, att_backward, att_forward, s, st);
+    });
 }
 
 int gvx_dec_infer_continuous(const gvx_dims *dd, const gvx_weights *w, const void *packed, const float *memory,

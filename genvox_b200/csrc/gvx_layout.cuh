@@ -119,4 +119,19 @@ struct InferL {
     }
 };
 
+// per-step arguments of the inference step functions (infer_step, infer_step_bf16)
+struct InferStepArgs {
+    const float *memory;
+    const int64_t *lengths;
+    const int *row_frame, *row_id;     // optional per-row prenet dropout frame and row (run_prenet), or null
+    const float *prev;                 // the previous [mel | gate] rows (the go frame at the first step)
+    float *align_t;                    // this step's attention weights, row stride align_bstride
+    long long align_bstride;
+    float *out_t;                      // this step's [mel | gate] rows
+    int t;
+    uint64_t seed;
+    int training, row_offset;
+    int win_back, win_fwd;             // the attention constraint (AttnFwdArgs; win_fwd == 0: off)
+};
+
 }  // namespace gvx

@@ -21,7 +21,7 @@ namespace gvx {
 
 constexpr int32_t SESSION_READY = 0x53455353;
 
-// workspace: the static inference layout for S rows and a two-frame output ring, then this block
+// workspace: the inference plan's layout for S rows and a two-frame output ring (steps = 2), then this block
 struct SessL {
     size_t MEM, STG, STGP, RMEM, RPM, RLEN, RCAP, ALIGN, LEN, ST, CTL, total;
     SessL(const Dims &d, size_t base, int N, int S, int cap) {
@@ -42,9 +42,7 @@ struct SessL {
     }
 };
 
-inline SessL session_layout(const Dims &d, bool bf, int N, int S, int cap) {
-    return SessL(d, continuous_base(d, bf, S, N), N, S, cap);
-}
+inline SessL session_layout(const InferPlan &P, int cap) { return SessL(P.d, P.total, P.N, P.B, cap); }
 
 // length and frame cap of ids first .. first + k - 1 into the ring
 __global__ void k_session_put(int64_t *__restrict__ rlen, int32_t *__restrict__ rcap, const int64_t *__restrict__ lengths,
@@ -65,15 +63,11 @@ inline int check_session(const gvx_dims *dd, const gvx_session *s) {
     return 0;
 }
 
-inline uint32_t *session_seed_slot(const Dims &d, bool bf, int N, int S, float *s) {
-    const size_t flags_off = bf ? InferBfL(d, S, N, 2).FLAGS : InferL(d, S, N, 2).FLAGS;
-    return reinterpret_cast<uint32_t *>(s + flags_off) + 32;
-}
-
-int session_submit(const Dims &d, bool bf, const gvx_weights *w, const gvx_session *ss, const float *memory,
-                   const int64_t *lengths, const int32_t *caps, int k, float *s, cudaStream_t st) {
+int session_submit(const InferPlan &P, const gvx_weights *w, const gvx_session *ss, const float *memory, const int64_t *lengths,
+                   const int32_t *caps, int k, float *s, cudaStream_t st) {
+    const Dims &d = P.d;
     const int S = ss->slots, N = ss->N, cap = ss->capacity;
-    const SessL L = session_layout(d, bf, N, S, cap);
+    const SessL L = session_layout(P, cap);
     const size_t NE = (size_t)N * d.E, ND = (size_t)N * d.D;
     // processed memory in launches of exactly S x N rows (the static call's row count, so every row gets the bits the
     // static call computes), through staging buffers: the slot-memory buffer holds live state
@@ -103,31 +97,34 @@ int session_submit(const Dims &d, bool bf, const gvx_weights *w, const gvx_sessi
     return 0;
 }
 
-int session_step(const Dims &d, bool bf, const gvx_weights *w, const float *packed, gvx_session *ss, int K, float *frames,
-                 float *align, int32_t *utt_out, int32_t *frame_out, int8_t *last_out, int *steps_run, int win_back, int win_fwd,
-                 float *s, cudaStream_t st) {
+int session_step(const InferPlan &P, const gvx_weights *w, const float *packed, gvx_session *ss, int K, float *frames, float *align,
+                 int32_t *utt_out, int32_t *frame_out, int8_t *last_out, int *steps_run, int win_back, int win_fwd, float *s,
+                 cudaStream_t st) {
+    const Dims &d = P.d;
     const int S = ss->slots, N = ss->N, cap = ss->capacity;
-    const InferL Lf(d, S, N, 2);
-    const InferBfL Lb(d, S, N, 2);
-    const SessL L = session_layout(d, bf, N, S, cap);
-    const size_t PM = bf ? Lb.PM : Lf.PM, OUT = bf ? Lb.OUT : Lf.OUT, FLAGS = bf ? Lb.FLAGS : Lf.FLAGS;
+    const SessL L = session_layout(P, cap);
     int *state = (int *)(s + L.ST), *ctl = (int *)(s + L.CTL);
     int64_t *len_slot = (int64_t *)(s + L.LEN);
     float *mem_slot = s + L.MEM;
-    const bool fused_prenet = infer_prenet_fused_ok(d, S);
 
     AdmitArgs a;
     memset(&a, 0, sizeof(a));
-    admit_state(a, d, bf, Lf, Lb, s, S, N);
+    admit_state(a, P, s);
     a.align_t = s + L.ALIGN;
     a.memory = s + L.RMEM; a.pmq = s + L.RPM; a.lengths = (const int64_t *)(s + L.RLEN); a.caps = (const int32_t *)(s + L.RCAP);
-    a.mem_slot = mem_slot; a.pm_slot = s + PM; a.len_slot = len_slot;
+    a.mem_slot = mem_slot; a.pm_slot = s + P.PM; a.len_slot = len_slot;
     a.ch_frames = frames; a.ch_align = ss->with_alignments ? align : nullptr;
     a.ch_utt = utt_out; a.ch_frame = frame_out; a.ch_last = last_out;
     a.flags = ctl;
     a.thr = ss->gate_threshold;
     a.ignore_gate = ss->ignore_gate; a.S = S; a.N = N; a.E = d.E; a.D = d.D; a.M = d.M; a.OL = d.OL; a.max_steps = ss->max_steps;
     a.U = (int)ss->submitted; a.cap = cap;
+    InferStepArgs io;
+    memset(&io, 0, sizeof(io));
+    io.memory = mem_slot; io.lengths = len_slot;
+    io.align_t = s + L.ALIGN; io.align_bstride = N;
+    io.seed = ss->seed; io.row_offset = ss->row_offset;
+    io.win_back = win_back; io.win_fwd = win_fwd;
 
     const int hp = (int)(ss->steps_run & 1);       // parity of the h / c ping-pong and of the output ring
     int up = ss->parity;                           // current half of the utt / frame / next / cap ping-pong
@@ -140,8 +137,8 @@ int session_step(const Dims &d, bool bf, const gvx_weights *w, const float *pack
     // the first step reads.  The queue only grows between calls, so once this admission has run, a slot that goes idle
     // during the call does so because the queue is empty: idle slots and queued utterances never coexist inside a call.
     a.head = 1;
-    a.out_t = s + OUT + (size_t)(hp ^ 1) * S * d.OL;
-    a.bar = fused_prenet ? (unsigned *)(s + FLAGS) + 40 : nullptr;
+    a.out_t = s + P.OUT + (size_t)(hp ^ 1) * S * d.OL;
+    a.bar = P.fused_prenet ? (unsigned *)P.flags(s) + 40 : nullptr;
     a.bar_value = (unsigned)(d.P / IPN_COLS) * (unsigned)hp;
     slots_at(up);
     pdl_barrier_next();
@@ -156,17 +153,16 @@ int session_step(const Dims &d, bool bf, const gvx_weights *w, const float *pack
     int i = 0;
     for (; i < K; ++i) {
         const int t = hp + i, p = t & 1;
-        const float *prev = s + OUT + (size_t)(p ^ 1) * S * d.OL;
-        float *out_t = s + OUT + (size_t)p * S * d.OL;
         slots_at(up);
+        io.t = t;
+        io.row_frame = a.frame_cur; io.row_id = a.utt_cur;
+        io.prev = s + P.OUT + (size_t)(p ^ 1) * S * d.OL;
+        io.out_t = s + P.OUT + (size_t)p * S * d.OL;
         // full dependency on the previous k_gate_admit, as in the continuous loop (an admission rewrites lengths and
         // processed memory that kernels of the chain read before griddepcontrol.wait)
         pdl_barrier_next();
-        if (bf) GVX_TRY(infer_step_bf16(d, w, packed, Lb, s, mem_slot, len_slot, S, N, ss->seed, t, 0, ss->row_offset, a.frame_cur,
-                                        a.utt_cur, prev, s + L.ALIGN, (long long)N, out_t, win_back, win_fwd, st));
-        else GVX_TRY(infer_step(d, w, packed, Lf, s, mem_slot, len_slot, S, N, ss->seed, t, 0, ss->row_offset, a.frame_cur, a.utt_cur,
-                                prev, s + L.ALIGN, (long long)N, out_t, fused_prenet, win_back, win_fwd, st));
-        a.out_t = out_t;
+        GVX_TRY(P.step(w, packed, s, io, st));
+        a.out_t = io.out_t;
         a.step = i;
         GVX_CUDA(launch_pdl(k_gate_admit, dim3(S), dim3(ADMIT_THREADS), 0, st, a));
         GVX_LAUNCHED(1);
@@ -194,10 +190,9 @@ extern "C" {
 size_t gvx_dec_session_workspace_bytes(const gvx_dims *d, int N, int slots, int capacity) {
     using namespace gvx;
     if (check_dims(d) || N <= 0 || slots <= 0 || capacity <= 0) return 0;
-    const Dims dm(*d);
-    const bool bf = d->precision == GVX_BF16;
-    if (bf && check_bf16_dims(dm, slots)) return 0;
-    return session_layout(dm, bf, N, slots, capacity).total * sizeof(float);
+    const InferPlan P(*d, slots, N, 2);
+    if (P.bf && check_bf16_dims(P.d, slots)) return 0;
+    return session_layout(P, capacity).total * sizeof(float);
 }
 
 int gvx_dec_session_init(const gvx_dims *dd, gvx_session *ss, void *workspace, void *stream) {
@@ -205,17 +200,16 @@ int gvx_dec_session_init(const gvx_dims *dd, gvx_session *ss, void *workspace, v
     GVX_TRY(check_session(dd, ss));
     GVX_CHECK(workspace != nullptr, "null argument");
     GVX_TRY(latch_check());
-    const Dims d(*dd);
-    const bool bf = dd->precision == GVX_BF16;
-    const int S = ss->slots, N = ss->N;
-    const SessL L = session_layout(d, bf, N, S, ss->capacity);
+    const InferPlan P(*dd, ss->slots, ss->N, 2);
+    const SessL L = session_layout(P, ss->capacity);
     float *s = (float *)workspace;
     cudaStream_t st = (cudaStream_t)stream;
-    GVX_CUDA(cudaMemsetAsync(s, 0, L.total * sizeof(float), st));      // every slot's state, the output ring, the error words
-    k_slot_start<<<grid_for(S), 256, 0, st>>>(S, 0, N, nullptr, (int64_t *)(s + L.LEN), (int *)(s + L.ST));   // all idle
+    // the whole workspace, a superset of the plan's reset: every slot's state, the output ring, the flags and error words
+    GVX_CUDA(cudaMemsetAsync(s, 0, L.total * sizeof(float), st));
+    k_slot_start<<<grid_for(P.B), 256, 0, st>>>(P.B, 0, P.N, nullptr, (int64_t *)(s + L.LEN), (int *)(s + L.ST));   // all idle
     GVX_LAUNCHED(1);
     GVX_CUDA(cudaGetLastError());
-    GVX_TRY(put_seed(session_seed_slot(d, bf, N, S, s), ss->seed, st));
+    GVX_TRY(put_seed(P.seed_slot(s), ss->seed, st));
     ss->steps_run = ss->submitted = ss->admitted = ss->finished = 0;
     ss->active = 0;
     ss->parity = 0;
@@ -233,7 +227,7 @@ int gvx_dec_session_submit(const gvx_dims *dd, const gvx_weights *w, const void 
     GVX_CHECK(ss->submitted + k - ss->admitted <= ss->capacity, "session: the queue ring is full (submitted + k - admitted > capacity)");
     GVX_CHECK(ss->submitted + k - 1 + ss->row_offset <= 2147483647LL, "session: utterance id + row_offset would pass 2^31 - 1");
     GVX_TRY(latch_check());
-    GVX_TRY(session_submit(Dims(*dd), dd->precision == GVX_BF16, w, ss, memory, lengths, frame_caps, k, (float *)workspace,
+    GVX_TRY(session_submit(InferPlan(*dd, ss->slots, ss->N, 2), w, ss, memory, lengths, frame_caps, k, (float *)workspace,
                            (cudaStream_t)stream));
     ss->submitted += k;
     return 0;
@@ -252,20 +246,13 @@ int gvx_dec_session_step_windowed(const gvx_dims *dd, const gvx_weights *w, cons
     *steps_run = 0;
     if (ss->active == 0 && ss->submitted == ss->admitted) return 0;      // nothing queued, nothing running
     GVX_TRY(latch_check());
-    const Dims d(*dd);
-    const bool bf = dd->precision == GVX_BF16;
+    const InferPlan P(*dd, ss->slots, ss->N, 2);
     cudaStream_t st = (cudaStream_t)stream;
     float *s = (float *)workspace;
-    g_seed_ptr = session_seed_slot(d, bf, ss->N, ss->slots, s);
-    int rc = session_step(d, bf, w, (const float *)packed, ss, max_steps_this_call, frames, align, utt, frame, last, steps_run,
-                          att_backward, att_forward, s, st);
-    g_seed_ptr = nullptr;
-    if (rc == 0 && bf)
-        rc = check_tc_err_public(reinterpret_cast<int *>(s + InferBfL(d, ss->slots, ss->N, 2).ERR), st, "gvx_dec_session_step");
-    if (rc == 0 && !bf)
-        rc = check_tc_err_public(reinterpret_cast<int *>(s + InferL(d, ss->slots, ss->N, 2).FLAGS) + 41, st,
-                                 "gvx_dec_session_step (prenet barrier)");
-    return rc;
+    return infer_call(P, s, false, ss->seed, st, "gvx_dec_session_step", [&] {      // the seed words were written at init
+        return session_step(P, w, (const float *)packed, ss, max_steps_this_call, frames, align, utt, frame, last, steps_run,
+                            att_backward, att_forward, s, st);
+    });
 }
 
 int gvx_dec_session_step(const gvx_dims *dd, const gvx_weights *w, const void *packed, gvx_session *ss, int max_steps_this_call,
