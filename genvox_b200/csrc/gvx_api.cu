@@ -1,6 +1,7 @@
-// genvox_b200 — C-ABI entry points: weight repack, teacher-forced forward, and the single-phase
-// hooks used by the parity tests (inference: gvx_infer.cuh and the files after it, same translation
-// unit).  See include/genvox_b200.h for the contract and the reference file:line each entry point replaces.
+// genvox_b200 — C-ABI entry points: weight repack, the fp32 teacher-forced forward, and the single-phase
+// hooks used by the parity tests (training entry points: gvx_train.cuh; inference: gvx_infer.cuh and the
+// files after it; same translation unit).  See include/genvox_b200.h for the contract and the reference
+// file:line each entry point replaces.
 #include "../../include/genvox_b200.h"
 #include "gvx_infer_prenet.cuh"
 #include "gvx_attention_c2.cuh"
@@ -18,13 +19,7 @@ thread_local char g_err[512] = {0};
 
 // bf16 mode drivers (gvx_bf16_api.cuh, same translation unit)
 size_t packed_total_bf16(const Dims &d);
-size_t stash_total_bf16(const Dims &d, int B, int N, int T);
-size_t bwd_total_bf16(const Dims &d, int B, int N, int T);
-size_t stash_seed_off_bf16(const Dims &d, int B, int N, int T);
 int pack_weights_bf16(const Dims &d, const gvx_weights *w, float *packed, cudaStream_t st);
-int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const float *mel_in,
-                   const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training, int row_offset, float *mel_out,
-                   float *gate_out, float *align_out, float *s, cudaStream_t st);
 
 int check_dims(const gvx_dims *d) {
     GVX_CHECK(d != nullptr, "dims is null");
@@ -202,6 +197,64 @@ int run_projection(const Dims &d, const float *packed, const float *hd, int hd_l
     return small ? launch_gemm<8, EpiStore>(g, e, st) : launch_gemm<32, EpiStore>(g, e, st);
 }
 
+// Decoder.forward (tacotron2.py:365-388) in fp32 mode: the stash S is read by train_bwd_fp32 (gvx_bwd.cuh)
+int train_fwd_fp32(const Dims &d, const StashL &S, const gvx_weights *w, const float *packed, const float *memory,
+                   const float *mel_in, const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training, int row_offset,
+                   float *mel_out, float *gate_out, float *align_out, float *s, cudaStream_t st) {
+    const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H, BE = (size_t)B * d.E;
+
+    // go frame + parse_decoder_inputs, prenet over all frames (tacotron2.py:370-373)
+    ProfScope *ps_setup = new ProfScope(PS_SETUP, st);
+    k_pack_frames<<<grid_for((size_t)T * B * d.M), 256, 0, st>>>(mel_in, B, d.M, T, s + S.FR);
+    GVX_LAUNCHED(1);
+    GVX_CUDA(cudaGetLastError());
+    GVX_TRY(run_prenet(d, w, s + S.FR, d.M, T * B, B, seed, 0, row_offset, s + S.PRE1, s + S.PRE2, st));
+    // initialize_decoder_states (tacotron2.py:303-315)
+    GVX_TRY(run_processed_memory(d, w, memory, B, N, s + S.PM, st));
+    GVX_CUDA(cudaMemsetAsync(s + S.HA, 0, BA * sizeof(float), st));
+    GVX_CUDA(cudaMemsetAsync(s + S.CA, 0, BA * sizeof(float), st));
+    GVX_CUDA(cudaMemsetAsync(s + S.HD, 0, BH * sizeof(float), st));
+    GVX_CUDA(cudaMemsetAsync(s + S.CD, 0, BH * sizeof(float), st));
+    GVX_CUDA(cudaMemsetAsync(s + S.CTX, 0, BE * sizeof(float), st));
+    GVX_CUDA(cudaMemsetAsync(s + S.WPREV, 0, (size_t)B * N * sizeof(float), st));
+    GVX_CUDA(cudaMemsetAsync(s + S.CUM, 0, (size_t)B * N * sizeof(float), st));
+    delete ps_setup;
+
+    pdl_barrier_next();
+    for (int t = 0; t < T; ++t) {   // Decoder.decode, tacotron2.py:333-363
+        LstmIO a;
+        a.x0 = s + S.PRE2 + (size_t)t * B * d.P; a.w0 = d.P; a.ld0 = d.P;
+        a.x1 = s + S.CTX + t * BE; a.w1 = d.E; a.ld1 = d.E;
+        a.x2 = s + S.HA + t * BA; a.w2 = d.A; a.ld2 = d.A;
+        a.c_prev = s + S.CA + t * BA; a.c_out = s + S.CA + (t + 1) * BA; a.h_out = s + S.HA + (t + 1) * BA;
+        a.gates_out = s + S.GA + (size_t)t * 4 * BA;
+        { ProfScope ps(PS_ATT_LSTM, st); GVX_TRY(run_lstm(d, packed, 0, a, B, seed, t, training, row_offset, st)); }
+        float *q = s + S.Q + (size_t)t * B * d.D;
+        { ProfScope ps(PS_QUERY, st); GVX_TRY(run_query(d, w, s + S.HA + (t + 1) * BA, B, q, st)); }
+        ProfScope *pa = new ProfScope(PS_ATTENTION, st);
+        GVX_TRY(run_attention(d, w, packed, q, s + S.PM, memory, mem_lengths, B, N, s + S.WPREV, s + S.CUM,
+                              s + S.ALIGN + (size_t)t * N, (long long)T * N, s + S.CUMS + (size_t)t * N,
+                              s + S.CTX + (t + 1) * BE, s + S.TH + (size_t)t * B * N * d.D,
+                              s + S.CONVS + (size_t)t * B * N * d.F, st));
+        delete pa;
+        LstmIO c;
+        c.x0 = s + S.HA + (t + 1) * BA; c.w0 = d.A; c.ld0 = d.A;
+        c.x1 = s + S.CTX + (t + 1) * BE; c.w1 = d.E; c.ld1 = d.E;
+        c.x2 = s + S.HD + t * BH; c.w2 = d.H; c.ld2 = d.H;
+        c.c_prev = s + S.CD + t * BH; c.c_out = s + S.CD + (t + 1) * BH; c.h_out = s + S.HD + (t + 1) * BH;
+        c.gates_out = s + S.GD + (size_t)t * 4 * BH;
+        { ProfScope ps(PS_DEC_LSTM, st); GVX_TRY(run_lstm(d, packed, 1, c, B, seed, t, training, row_offset, st)); }
+    }
+    ProfScope ps_out(PS_OUTPUT, st);
+    // projections for all frames at once, then parse_decoder_outputs (tacotron2.py:360-362,:322-331)
+    GVX_TRY(run_projection(d, packed, s + S.HD + BH, d.H, s + S.CTX + BE, d.E, T * B, s + S.OUT, st, false));
+    k_unpack_out<<<grid_for((size_t)B * (d.M + 1) * T), 256, 0, st>>>(s + S.OUT, B, d.M, d.OL, T, T, mel_out, gate_out);
+    GVX_LAUNCHED(1);
+    GVX_CUDA(cudaGetLastError());
+    GVX_CUDA(cudaMemcpyAsync(align_out, s + S.ALIGN, (size_t)B * T * N * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
 }  // namespace gvx
 
 using namespace gvx;
@@ -278,115 +331,12 @@ int gvx_dec_pack_weights(const gvx_dims *dd, const gvx_weights *w, void *packed_
     return 0;
 }
 
-size_t gvx_dec_stash_bytes(const gvx_dims *d, int B, int N, int T) {
-    if (check_dims(d) || B <= 0 || N <= 0 || T <= 0) return 0;
-    if (d->precision == GVX_BF16) return stash_total_bf16(Dims(*d), B, N, T) * sizeof(float);
-    return StashL(Dims(*d), B, N, T).total * sizeof(float);
-}
-size_t gvx_dec_bwd_workspace_bytes(const gvx_dims *d, int B, int N, int T) {
-    if (check_dims(d) || B <= 0 || N <= 0 || T <= 0) return 0;
-    if (d->precision == GVX_BF16) return bwd_total_bf16(Dims(*d), B, N, T) * sizeof(float);
-    return BwdL(Dims(*d), B, N, T).total * sizeof(float);
-}
-
-static int train_fwd_body(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
-                          const float *mel_in, const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training,
-                          int row_offset, float *mel_out, float *gate_out, float *align_out, void *stash_, void *stream) {
-    const Dims d(*dd);
-    if (dd->precision == GVX_BF16)
-        return train_fwd_bf16(d, w, (const float *)packed_, memory, mel_in, mem_lengths, B, N, T, seed, training, row_offset, mel_out,
-                              gate_out, align_out, (float *)stash_, (cudaStream_t)stream);
-    const StashL S(d, B, N, T);
-    const float *packed = (const float *)packed_;
-    float *s = (float *)stash_;
-    cudaStream_t st = (cudaStream_t)stream;
-    const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H, BE = (size_t)B * d.E;
-
-    // go frame + parse_decoder_inputs, prenet over all frames (tacotron2.py:370-373)
-    ProfScope *ps_setup = new ProfScope(PS_SETUP, st);
-    k_pack_frames<<<grid_for((size_t)T * B * d.M), 256, 0, st>>>(mel_in, B, d.M, T, s + S.FR);
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    GVX_TRY(run_prenet(d, w, s + S.FR, d.M, T * B, B, seed, 0, row_offset, s + S.PRE1, s + S.PRE2, st));
-    // initialize_decoder_states (tacotron2.py:303-315)
-    GVX_TRY(run_processed_memory(d, w, memory, B, N, s + S.PM, st));
-    GVX_CUDA(cudaMemsetAsync(s + S.HA, 0, BA * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + S.CA, 0, BA * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + S.HD, 0, BH * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + S.CD, 0, BH * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + S.CTX, 0, BE * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + S.WPREV, 0, (size_t)B * N * sizeof(float), st));
-    GVX_CUDA(cudaMemsetAsync(s + S.CUM, 0, (size_t)B * N * sizeof(float), st));
-    delete ps_setup;
-
-    pdl_barrier_next();
-    for (int t = 0; t < T; ++t) {   // Decoder.decode, tacotron2.py:333-363
-        LstmIO a;
-        a.x0 = s + S.PRE2 + (size_t)t * B * d.P; a.w0 = d.P; a.ld0 = d.P;
-        a.x1 = s + S.CTX + t * BE; a.w1 = d.E; a.ld1 = d.E;
-        a.x2 = s + S.HA + t * BA; a.w2 = d.A; a.ld2 = d.A;
-        a.c_prev = s + S.CA + t * BA; a.c_out = s + S.CA + (t + 1) * BA; a.h_out = s + S.HA + (t + 1) * BA;
-        a.gates_out = s + S.GA + (size_t)t * 4 * BA;
-        { ProfScope ps(PS_ATT_LSTM, st); GVX_TRY(run_lstm(d, packed, 0, a, B, seed, t, training, row_offset, st)); }
-        float *q = s + S.Q + (size_t)t * B * d.D;
-        { ProfScope ps(PS_QUERY, st); GVX_TRY(run_query(d, w, s + S.HA + (t + 1) * BA, B, q, st)); }
-        ProfScope *pa = new ProfScope(PS_ATTENTION, st);
-        GVX_TRY(run_attention(d, w, packed, q, s + S.PM, memory, mem_lengths, B, N, s + S.WPREV, s + S.CUM,
-                              s + S.ALIGN + (size_t)t * N, (long long)T * N, s + S.CUMS + (size_t)t * N,
-                              s + S.CTX + (t + 1) * BE, s + S.TH + (size_t)t * B * N * d.D,
-                              s + S.CONVS + (size_t)t * B * N * d.F, st));
-        delete pa;
-        LstmIO c;
-        c.x0 = s + S.HA + (t + 1) * BA; c.w0 = d.A; c.ld0 = d.A;
-        c.x1 = s + S.CTX + (t + 1) * BE; c.w1 = d.E; c.ld1 = d.E;
-        c.x2 = s + S.HD + t * BH; c.w2 = d.H; c.ld2 = d.H;
-        c.c_prev = s + S.CD + t * BH; c.c_out = s + S.CD + (t + 1) * BH; c.h_out = s + S.HD + (t + 1) * BH;
-        c.gates_out = s + S.GD + (size_t)t * 4 * BH;
-        { ProfScope ps(PS_DEC_LSTM, st); GVX_TRY(run_lstm(d, packed, 1, c, B, seed, t, training, row_offset, st)); }
-    }
-    ProfScope ps_out(PS_OUTPUT, st);
-    // projections for all frames at once, then parse_decoder_outputs (tacotron2.py:360-362,:322-331)
-    GVX_TRY(run_projection(d, packed, s + S.HD + BH, d.H, s + S.CTX + BE, d.E, T * B, s + S.OUT, st, false));
-    k_unpack_out<<<grid_for((size_t)B * (d.M + 1) * T), 256, 0, st>>>(s + S.OUT, B, d.M, d.OL, T, T, mel_out, gate_out);
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    GVX_CUDA(cudaMemcpyAsync(align_out, s + S.ALIGN, (size_t)B * T * N * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    return 0;
-}
-
-// ---------------------------------------------------------------- graph-cached entry points
-static uint32_t *seed_slot_train(const gvx_dims *dd, void *stash, int B, int N, int T) {
-    const Dims d(*dd);
-    const size_t off = dd->precision == GVX_BF16 ? stash_seed_off_bf16(d, B, N, T) : StashL(d, B, N, T).SEED;
-    return reinterpret_cast<uint32_t *>((float *)stash + off);
-}
+// the dropout seed of a call into its workspace slot (the kernels read it there: a captured graph outlives the call)
 static int put_seed(uint32_t *slot, uint64_t seed, cudaStream_t st) {
     k_set_seed<<<1, 1, 0, st>>>(slot, (uint32_t)(seed & 0xffffffffull), (uint32_t)(seed >> 32));
     GVX_LAUNCHED(1);
     GVX_CUDA(cudaGetLastError());
     return 0;
-}
-
-int gvx_dec_train_fwd(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
-                      const float *mel_in, const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training,
-                      int row_offset, float *mel_out, float *gate_out, float *align_out, void *stash_, void *stream) {
-    GVX_TRY(check_dims(dd));
-    GVX_CHECK(w && packed_ && memory && mel_in && mel_out && gate_out && align_out && stash_, "null argument");
-    GVX_CHECK(B > 0 && N > 0 && T > 0, "B, N, T must be positive");
-    GVX_TRY(latch_check());
-    cudaStream_t user = (cudaStream_t)stream;
-    uint32_t *slot = seed_slot_train(dd, stash_, B, N, T);
-    GVX_TRY(put_seed(slot, seed, user));
-    KeyBuilder kb;
-    kb.add((int)1).add(*dd).add(*w).add(packed_).add(memory).add(mel_in).add(mem_lengths).add(B).add(N).add(T).add(training)
-        .add(row_offset).add(mel_out).add(gate_out).add(align_out).add(stash_);
-    g_seed_ptr = slot;
-    const int rc = run_cached(kb.k, user, [&](cudaStream_t st) {
-        return train_fwd_body(dd, w, packed_, memory, mel_in, mem_lengths, B, N, T, seed, training, row_offset, mel_out, gate_out,
-                              align_out, stash_, (void *)st);
-    });
-    g_seed_ptr = nullptr;
-    return rc;
 }
 
 int gvx_device_error(int clear) {
@@ -478,9 +428,10 @@ int gvx_attention_step(const gvx_dims *dd, const gvx_weights *w, const void *pac
 
 }  // extern "C"
 
-// backward through time (gvx_dec_train_bwd) lives in its own file, same translation unit
+// the backward (gvx_bwd.cuh), the bf16 drivers, the training and inference entry points: same translation unit
 #include "gvx_bwd.cuh"
 #include "gvx_bf16_api.cuh"
+#include "gvx_train.cuh"
 #include "gvx_infer.cuh"
 #include "gvx_continuous.cuh"
 #include "gvx_session.cuh"

@@ -115,91 +115,6 @@ __global__ void __launch_bounds__(256) k_bf_lstm_bwd(const BfLstmBwd a) {
     }
 }
 
-
-// ------------------------------------------------------------------ attention-LSTM cell backward with d q . W_query folded in
-// Step S4 of BPTT used to be two launches: a tcgen05 GEMM  d h_q = d q . W_query  (K = att_dim = 128: far too small for the
-// engine - two k-blocks on 8 CTAs) and the pointwise kernel above.  Here a block owns 8 hidden units x all rows:
-// it stages its [16 x D] slice of W_query^T and the d q rows (both rounded to bf16 like the engine's operands, fp32
-// accumulate) in shared memory, contracts them with FFMA, and goes straight on with the cell backward.
-// Thread = (unit u = tid & 7, row pair tid >> 3): 8 consecutive lanes cover 8 consecutive units, so the gate / state
-// loads and the bf16 d-gate stores stay contiguous runs.
-constexpr int LBQ_UB = 8;               // hidden units per block
-constexpr int LBQ_THREADS = 256;
-struct BfLstmBwdQ {
-    BfLstmBwd p;                        // s0 unused
-    const __nv_bfloat16 *dq_rm;         // [B][D] row-major d q of this step
-    const float *WqT;                   // [HID][D]  W_query^T (fp32, rounded to bf16 on the fly)
-    int D;
-};
-__global__ void __launch_bounds__(LBQ_THREADS) k_bf_lstm_bwd_q(const BfLstmBwdQ q) {
-    extern __shared__ __align__(16) float lbq_sm[];
-    const BfLstmBwd &a = q.p;
-    pdl_trigger();
-    const int D = q.D;
-    if ((int)blockIdx.x >= a.main_blocks) {
-        pdl_wait();
-        const int total = a.B * a.P;
-        for (int idx = (blockIdx.x - a.main_blocks) * blockDim.x + threadIdx.x; idx < total;
-             idx += (gridDim.x - a.main_blocks) * blockDim.x) {
-            const int b = idx / a.P, pp = idx - b * a.P;
-            a.dz2[idx] = a.pre2[idx] > 0.f ? 2.f * src_get(a.dpre_src, b, pp) : 0.f;
-        }
-        return;
-    }
-    // thread = (unit ul = tid & 7, row pair tid >> 3): 32 row pairs per pass
-    const int RS = ((a.B + 1) & ~1) + 2;                 // row stride of sQ: even (float2 reads), +2 spreads the banks of the staging stores
-    float *sW = lbq_sm;                                  // [8][D + 1]
-    float *sQ = lbq_sm + ((LBQ_UB * (D + 1) + 3) & ~3);  // [D][RS]
-    const int u0 = blockIdx.x * LBQ_UB, tid = threadIdx.x;
-    // weights do not depend on the previous kernel of the chain: staged before griddepcontrol.wait
-    for (int i = tid; i < LBQ_UB * D; i += LBQ_THREADS) {
-        const int u = i / D, dd = i - u * D;
-        sW[u * (D + 1) + dd] = u0 + u < a.HID ? __bfloat162float(__float2bfloat16(q.WqT[(size_t)(u0 + u) * D + dd])) : 0.f;
-    }
-    const int ul = tid & 7, u = u0 + ul;
-    // everything of the cell backward that does not depend on the previous kernel either (forward stashes)
-    pdl_wait();
-    {   // d q rows: coalesced bf16x2 reads along d, transposed stores (bank = (RS * d + b) mod 32: RS = 2 mod 4 -> 2-way at worst)
-        const int half = D / 2;
-        for (int i = tid; i < a.B * half; i += LBQ_THREADS) {
-            const int b = i / half, d2 = i - b * half;
-            const __nv_bfloat162 v2 = *reinterpret_cast<const __nv_bfloat162 *>(q.dq_rm + (size_t)b * D + 2 * d2);
-            sQ[(2 * d2) * RS + b] = __bfloat162float(v2.x);
-            sQ[(2 * d2 + 1) * RS + b] = __bfloat162float(v2.y);
-        }
-        if (a.B & 1)
-            for (int dd = tid; dd < D; dd += LBQ_THREADS) sQ[dd * RS + a.B] = 0.f;
-    }
-    __syncthreads();
-    for (int bp = tid >> 3; 2 * bp < a.B; bp += LBQ_THREADS / 8) {
-        float acc0 = 0.f, acc1 = 0.f;
-        const float *wr = sW + ul * (D + 1);
-#pragma unroll 16
-        for (int dd = 0; dd < D; ++dd) {
-            const float wv = wr[dd];
-            const float2 qv = *reinterpret_cast<const float2 *>(sQ + dd * RS + 2 * bp);
-            acc0 = fmaf(qv.x, wv, acc0);
-            acc1 = fmaf(qv.y, wv, acc1);
-        }
-        if (u >= a.HID) continue;
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-            const int b = 2 * bp + j;
-            if (b >= a.B) break;
-            const size_t idx = (size_t)b * a.HID + u;
-            float dh = j == 0 ? acc0 : acc1;
-            if (a.s1.nsplit) dh += src_get(a.s1, b, u);
-            if (a.s2.nsplit) dh += src_get(a.s2, b, u);
-            const float mult = drop_mult(a.drop, a.site, a.t, (uint32_t)(b + a.row_offset), (uint32_t)u);
-            const float4 ga = *reinterpret_cast<const float4 *>(a.gates + (size_t)b * 4 * a.HID + 4 * u);
-            float dcp;
-            const float4 dp = lstm_bwd_point(dh, mult, ga, a.c_prev[idx], a.c_new[idx], a.dc[idx], dcp);
-            a.dc[idx] = dcp;
-            bf_store4(a.dg_dst, b, 4 * u, make_uint2(pack_bf2(dp.x, dp.y), pack_bf2(dp.z, dp.w)));
-        }
-    }
-}
-
 // out[b, m] = sum_s P[s][b][m] + bias[m]   (inference projection epilogue)
 __global__ void k_bf_finalize(const float *__restrict__ P, int KS, int B, int ldp, int M, const float *__restrict__ bias,
                               float *__restrict__ out, int ldo) {

@@ -1,10 +1,8 @@
 // genvox_b200 — bf16 mode drivers: packed operand images, teacher-forced forward, BPTT, inference.
-// Same entry points as fp32 mode (gvx_api.cu dispatches on gvx_dims.precision); see gvx_bf16.cuh /
-// gvx_tc.cuh for the kernels.  Reference lines: Decoder.forward tacotron2.py:365-388, decode :333-363,
+// Same entry points as fp32 mode (TrainPlan, gvx_train.cuh, and InferPlan, gvx_infer.cuh, dispatch on gvx_dims.precision);
+// see gvx_bf16.cuh / gvx_tc.cuh for the kernels.  Reference lines: Decoder.forward tacotron2.py:365-388, decode :333-363,
 // inference :390-414, BPTT = loss.backward() :520.
 #pragma once
-#include <cublas_v2.h>
-
 #include "gvx_attention_c2.cuh"
 #include "gvx_bf16.cuh"
 #include "gvx_blas.cuh"
@@ -295,54 +293,6 @@ inline int check_tc_err(int *err_dev, cudaStream_t st, const char *what) {
     return 0;
 }
 
-// bf16 x bf16 -> fp32 time-batched GEMMs (plain library GEMMs): row-major C[M,N] = op(A) . op(B)
-inline int gemm_tn_bf16(cudaStream_t st, int M, int N, int K, const bf16 *A, int lda, const bf16 *Bm, int ldb, float *Cm, int ldc) {
-    cublasHandle_t h;
-    GVX_TRY(blas(&h, st));
-    const float alpha = 1.f, beta = 0.f;
-    cublasStatus_t s = cublasGemmEx(h, CUBLAS_OP_N, CUBLAS_OP_T, N, M, K, &alpha, Bm, CUDA_R_16BF, ldb, A, CUDA_R_16BF, lda, &beta, Cm,
-                                    CUDA_R_32F, ldc, CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
-    if (s != CUBLAS_STATUS_SUCCESS) { snprintf(g_err, sizeof(g_err), "cublasGemmEx(TN bf16) failed: %d", (int)s); return 1; }
-    return 0;
-}
-// C[M,N] = A[M,K] . W[N,K]^T
-inline int gemm_nt_bf16(cudaStream_t st, int M, int N, int K, const bf16 *A, int lda, const bf16 *Wm, int ldw, float *Cm, int ldc) {
-    cublasHandle_t h;
-    GVX_TRY(blas(&h, st));
-    const float alpha = 1.f, beta = 0.f;
-    cublasStatus_t s = cublasGemmEx(h, CUBLAS_OP_T, CUBLAS_OP_N, N, M, K, &alpha, Wm, CUDA_R_16BF, ldw, A, CUDA_R_16BF, lda, &beta, Cm,
-                                    CUDA_R_32F, ldc, CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
-    if (s != CUBLAS_STATUS_SUCCESS) { snprintf(g_err, sizeof(g_err), "cublasGemmEx(NT bf16) failed: %d", (int)s); return 1; }
-    return 0;
-}
-
-// C[M,N] = A[M,K] . Wm[K,N]   (all row-major)
-inline int gemm_nn_bf16(cudaStream_t st, int M, int N, int K, const bf16 *A, int lda, const bf16 *Wm, int ldw, float *Cm, int ldc) {
-    cublasHandle_t h;
-    GVX_TRY(blas(&h, st));
-    const float alpha = 1.f, beta = 0.f;
-    cublasStatus_t s = cublasGemmEx(h, CUBLAS_OP_N, CUBLAS_OP_N, N, M, K, &alpha, Wm, CUDA_R_16BF, ldw, A, CUDA_R_16BF, lda, &beta, Cm,
-                                    CUDA_R_32F, ldc, CUBLAS_COMPUTE_32F, CUBLAS_GEMM_DEFAULT);
-    if (s != CUBLAS_STATUS_SUCCESS) { snprintf(g_err, sizeof(g_err), "cublasGemmEx(NN bf16) failed: %d", (int)s); return 1; }
-    return 0;
-}
-
-// The all-frames contractions run on the own tcgen05 GEMM (gvx_nt_gemm.cuh).  GVX_OWN_GEMM=0 sends them to cuBLAS instead
-// (comparison runs only).
-inline bool own_gemm() {
-    static int on = -1;
-    if (on < 0) {
-        const char *e = getenv("GVX_OWN_GEMM");
-        on = (e && e[0] == '0') ? 0 : 1;
-    }
-    return on == 1;
-}
-// C[M,N] = A[M,K] . W[N,K]^T
-inline int gemm_nt(cudaStream_t st, int M, int N, int K, const bf16 *A, int lda, const bf16 *Wm, int ldw, float *Cm, int ldc, int *err) {
-    if (own_gemm() && K % 8 == 0 && lda % 8 == 0 && ldw % 8 == 0) return nt_gemm_bf16(st, M, N, K, A, lda, Wm, ldw, Cm, ldc, err);
-    return gemm_nt_bf16(st, M, N, K, A, lda, Wm, ldw, Cm, ldc);
-}
-
 __global__ void k_add_bias_rows(float *x, size_t rows, int cols, int ld, const float *__restrict__ bias) {
     const size_t total = rows * cols;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
@@ -352,39 +302,51 @@ __global__ void k_add_bias_rows(float *x, size_t rows, int cols, int ld, const f
     }
 }
 
-// the fused persistent attention chains (forward + BPTT) go together: they share the bf16 / swizzled tanh stash
-inline bool fused_chains_ok(const Dims &d, int B, int N) {
-    return pc_enabled() && pc_supported(d.H, B) && fa_enabled() && fa_supported(d, B, N) && fb_supported(d, B, N);
-}
-// the persistent BPTT attention chain behind a PER-STEP forward chain (shapes the persistent forward does not cover, e.g.
-// configs[4]: B = 32, N = 300): the per-step attention kernel then writes the stashes in the formats the BPTT chain reads
-// (bf16 / swizzled tanh rows, fp32 context per frame) and the bf16 copy of the encoder memory is made up front
-inline bool fused_bwd_only_ok(const Dims &d, int B, int N) {
-    return pc_enabled() && pc_supported(d.H, B) && fa_enabled() && !fa_supported(d, B, N) && fb_supported(d, B, N) &&
-           attention_fwd_uses_c2(AttnShape{B, N, d.D, d.E, d.F, d.KS});
+// The chains a bf16 train step runs.  The forward writes the stash in the formats the backward of the same path reads, so
+// both take this one decision (TrainPlan, gvx_train.cuh) and decide nothing themselves.
+struct BfTrainPath {
+    // persistent decoder-LSTM chains (gvx_persist.cuh): under teacher forcing the decoder LSTM's input does not depend on
+    // it, so the attention chain runs first for all frames and the decoder-LSTM recurrence follows in ONE launch (its BPTT
+    // likewise)
+    bool persistent;
+    // persistent attention forward chain (gvx_fused_fwd.cuh): attention LSTM + query + attention of all frames in ONE launch
+    bool fused_fwd;
+    // persistent attention BPTT chain (gvx_fused_bwd.cuh).  The stash then holds the formats it reads: bf16 / chunk-swizzled
+    // tanh rows, the bf16 copy of the encoder memory (MEMB) and the fp32 context per frame (CTX32).  Behind the persistent
+    // forward chain, or behind a PER-STEP forward where the persistent one does not fit (e.g. configs[4]: B = 32, N = 300)
+    // but the per-step attention runs on the cluster kernel, which writes those formats
+    bool fused_bwd;
+    // d q . W_query folded into the 2-CTA cluster attention-backward kernel of the per-step BPTT (its conv-transpose phase
+    // leaves 320 threads idle): one launch less per step
+    bool dhq_folded;
+};
+
+inline BfTrainPath bf_train_path(const Dims &d, int B, int N) {
+    const AttnShape as{B, N, d.D, d.E, d.F, d.KS};
+    BfTrainPath p;
+    p.persistent = pc_enabled() && pc_supported(d.H, B);
+    const bool chains = p.persistent && fa_enabled() && fb_supported(d, B, N);
+    p.fused_fwd = chains && fa_supported(d, B, N);
+    p.fused_bwd = p.fused_fwd || (chains && attention_fwd_uses_c2(as));
+    p.dhq_folded = d.A % 16 == 0 && d.A <= 1024 && attention_bwd_uses_c2(as);
+    return p;
 }
 
 // ======================================================================================= forward (training)
-int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const float *mel_in,
-                          const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training, int row_offset,
-                          float *mel_out, float *gate_out, float *align_out, float *s, cudaStream_t st) {
+int train_fwd_bf16(const Dims &d, const BfTrainPath &path, const StashBfL &S, const gvx_weights *w, const float *packed,
+                   const float *memory, const float *mel_in, const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training,
+                   int row_offset, float *mel_out, float *gate_out, float *align_out, float *s, cudaStream_t st) {
     GVX_TRY(check_bf16_dims(d, B));
     const BfGeom g(d);
     const PackedL PL(d);
     const PackedBfL BL(d, PL.total);
-    const StashBfL S(d, B, N, T);
     const int NPAD = S.NPAD;
     const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H;
     bf16 *XAI = (bf16 *)(s + S.XAI), *XDI = (bf16 *)(s + S.XDI), *XARM = (bf16 *)(s + S.XARM), *XDRM = (bf16 *)(s + S.XDRM),
          *HCRM = (bf16 *)(s + S.HCRM);
     int *err = (int *)(s + S.ERR);
     const bf16 *WaI = (const bf16 *)(packed + BL.WaI), *WdI = (const bf16 *)(packed + BL.WdI), *WqI = (const bf16 *)(packed + BL.WqI);
-    // persistent decoder-LSTM chain: its input part does not depend on the decoder LSTM under teacher forcing, so the
-    // attention chain runs first for all frames and the decoder-LSTM recurrence follows in ONE launch (gvx_persist.cuh)
-    const bool pc = pc_enabled() && pc_supported(d.H, B);
-    // fused attention chain: attention LSTM + query + attention of all frames in ONE persistent launch (gvx_fused_fwd.cuh)
-    const bool fa = fused_chains_ok(d, B, N);
-    const bool fbo = !fa && fused_bwd_only_ok(d, B, N);      // per-step forward, persistent BPTT attention chain
+    const bool pc = path.persistent, fa = path.fused_fwd, fb = path.fused_bwd;
 
     ProfScope *ps_setup = new ProfScope(PS_SETUP, st);
     GVX_CUDA(cudaMemsetAsync(err, 0, 64 * sizeof(float), st));
@@ -395,7 +357,7 @@ int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
     } else {
         GVX_CUDA(cudaMemsetAsync(s + S.XIMG, 0, fa_ximg_bytes(), st));
     }
-    if (fa || fbo) {
+    if (fb) {
         k_to_bf16<<<grid_for((size_t)B * N * d.E), 256, 0, st>>>(memory, d.E, (size_t)B * N, d.E, (bf16 *)(s + S.MEMB), d.E);
         GVX_LAUNCHED(1);
     }
@@ -421,7 +383,7 @@ int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
     if (fa) {
         {   // prenet part of the attention-LSTM gate pre-activations for all frames (tacotron2.py:338-340)
             ProfScope ps(PS_ATT_LSTM, st);
-            GVX_TRY(gemm_nt(st, T * B, 4 * d.A, d.P, XARM, d.Ka, (const bf16 *)(packed + BL.WaPRM), d.P, s + S.GA, 4 * d.A, err));
+            GVX_TRY(nt_gemm_bf16(st, T * B, 4 * d.A, d.P, XARM, d.Ka, (const bf16 *)(packed + BL.WaPRM), d.P, s + S.GA, 4 * d.A, err));
         }
         ProfScope ps(PS_ATTENTION, st);
         FaArgs f;
@@ -478,7 +440,7 @@ int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
             add_img(a.ctx_bf, xa_n, d.P, NPAD); add_rm(a.ctx_bf, xarm_n, d.P, d.Ka);
             add_rm(a.ctx_bf, hcrm, d.H, d.Kp);
             a.th_stash = s + S.TH + (size_t)t * B * N * d.D;
-            if (fbo) {
+            if (fb) {       // the formats the persistent BPTT chain reads
                 a.th_bf16 = 1;
                 a.th_stash = reinterpret_cast<float *>(reinterpret_cast<bf16 *>(s + S.TH) + (size_t)t * B * N * d.D);
                 a.ctx_out = s + S.CTX32 + (size_t)t * B * d.E;
@@ -499,7 +461,7 @@ int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
     if (pc) {   // decoder LSTM (:355-358) for all frames: time-batched input part, then the persistent recurrence
         {
             ProfScope ps(PS_DEC_IN_GEMM, st);
-            GVX_TRY(gemm_nt(st, T * B, 4 * d.H, d.A + d.E, XDRM, d.Kd, (const bf16 *)(packed + BL.WdRM), d.Kd, s + S.GD, 4 * d.H, err));
+            GVX_TRY(nt_gemm_bf16(st, T * B, 4 * d.H, d.A + d.E, XDRM, d.Kd, (const bf16 *)(packed + BL.WdRM), d.Kd, s + S.GD, 4 * d.H, err));
         }
         ProfScope ps(PS_DEC_LSTM, st);
         GVX_CUDA(cudaMemsetAsync(s + S.HIMG, 0, pc_himg_elems(d.H) * sizeof(bf16), st));
@@ -518,7 +480,7 @@ int train_fwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
     }
     ProfScope ps_out(PS_OUTPUT, st);
     // mel / gate projections for all frames (:360-362): [T*B, H+E] bf16 . Wpg^T
-    GVX_TRY(gemm_nt(st, T * B, d.M + 1, d.Kp, HCRM, d.Kp, (const bf16 *)(packed + BL.WpgRM), d.Kp, s + S.OUT, d.OL, err));
+    GVX_TRY(nt_gemm_bf16(st, T * B, d.M + 1, d.Kp, HCRM, d.Kp, (const bf16 *)(packed + BL.WpgRM), d.Kp, s + S.OUT, d.OL, err));
     k_add_bias_rows<<<grid_for((size_t)T * B * (d.M + 1)), 256, 0, st>>>(s + S.OUT, (size_t)T * B, d.M + 1, d.OL, packed + PL.bpg);
     GVX_LAUNCHED(1);
     k_unpack_out<<<grid_for((size_t)B * (d.M + 1) * T), 256, 0, st>>>(s + S.OUT, B, d.M, d.OL, T, T, mel_out, gate_out);
@@ -552,48 +514,15 @@ inline int run_bf_lstm_bwd(const Dims &d, int which, const SrcSum &s0, const Src
     return 0;
 }
 
-// attention-LSTM cell backward of one step with d q . W_query computed inside (k_bf_lstm_bwd_q)
-inline int run_bf_lstm_bwd_q(const Dims &d, const bf16 *dq_rm, const float *WqT, const SrcSum &s1, const SrcSum &s2, const float *gates,
-                             const float *c_prev, const float *c_new, float *dc, const BfDsts &dg, int B, uint64_t seed, int t,
-                             int training, int row_offset, const SrcSum *dpre_src, const float *pre2, float *dz2, cudaStream_t st) {
-    BfLstmBwdQ q;
-    memset(&q, 0, sizeof(q));
-    BfLstmBwd &a = q.p;
-    a.s1 = s1; a.s2 = s2;
-    a.drop = make_drop(seed, d.p_att, training);
-    a.site = SITE_ATT;
-    a.t = (uint32_t)t; a.row_offset = row_offset; a.B = B; a.HID = d.A;
-    a.gates = gates; a.c_prev = c_prev; a.c_new = c_new; a.dc = dc; a.dg_dst = dg;
-    a.main_blocks = (d.A + LBQ_UB - 1) / LBQ_UB;
-    int extra = 0;
-    if (dpre_src) {
-        a.dpre_src = *dpre_src; a.pre2 = pre2; a.dz2 = dz2; a.P = d.P;
-        extra = grid_for((size_t)B * d.P);
-        if (extra > 64) extra = 64;
-    }
-    q.dq_rm = dq_rm; q.WqT = WqT; q.D = d.D;
-    const size_t smem = ((size_t)((LBQ_UB * (d.D + 1) + 3) & ~3) + (size_t)d.D * (((B + 1) & ~1) + 2)) * sizeof(float);
-    static size_t configured = 0;
-    if (smem > configured) {
-        GVX_CUDA(cudaFuncSetAttribute(k_bf_lstm_bwd_q, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = smem;
-    }
-    GVX_CUDA(launch_pdl(k_bf_lstm_bwd_q, dim3(a.main_blocks + extra), dim3(LBQ_THREADS), smem, st, q));
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    return 0;
-}
-
 // ======================================================================================= backward (BPTT)
-int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
-                   int B, int N, int T, uint64_t seed, int training, int row_offset, const float *d_mel, const float *d_gate,
-                   const float *d_align, const float *s, float *x, const gvx_grads *g, float *d_memory, cudaStream_t st) {
+int train_bwd_bf16(const Dims &d, const BfTrainPath &path, const StashBfL &S, const BwdBfL &W, const gvx_weights *w,
+                   const float *packed, const float *memory, const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training,
+                   int row_offset, const float *d_mel, const float *d_gate, const float *d_align, const float *s, float *x,
+                   const gvx_grads *g, float *d_memory, cudaStream_t st) {
     GVX_TRY(check_bf16_dims(d, B));
     const BfGeom gm(d);
     const PackedL PL(d);
     const PackedBfL BL(d, PL.total);
-    const StashBfL S(d, B, N, T);
-    const BwdBfL W(d, B, N, T);
     const int NPAD = W.NPAD, TB = T * B;
     const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H, BE = (size_t)B * d.E;
     const bf16 *WaTI = (const bf16 *)(packed + BL.WaTI), *WdTI = (const bf16 *)(packed + BL.WdTI), *WqTI = (const bf16 *)(packed + BL.WqTI);
@@ -621,7 +550,7 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
     GVX_CUDA(cudaGetLastError());
     GVX_TRY(gemm_nn(st, TB, d.Kp, d.M + 1, x + W.DOUT, d.OL, packed + PL.Wpg, d.Kp, x + W.DHC, d.Kp, 0.f));
 
-    const bool pc = pc_enabled() && pc_supported(d.H, B);
+    const bool pc = path.persistent, fb = path.fused_bwd, dhq_folded = path.dhq_folded;
     const int AE = d.A + d.E;
     if (pc) {
         {   // BPTT of the decoder-LSTM recurrence for all frames in one persistent launch (gvx_persist.cuh)
@@ -640,22 +569,10 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
         }
         {   // d [h_att_t | ctx_t] from the decoder-LSTM input, all frames: d gates_dec . W_ih
             ProfScope ps(PS_BWD_DEC_GEMM, st);
-            if (own_gemm()) GVX_TRY(nt_gemm_bf16(st, TB, AE, 4 * d.H, DGDRM, 4 * d.H, (const bf16 *)(packed + BL.WdTRM), 4 * d.H, x + W.DXDALL, AE, err));
-            else GVX_TRY(gemm_nn_bf16(st, TB, AE, 4 * d.H, DGDRM, 4 * d.H, (const bf16 *)(packed + BL.WdRM), d.Kd, x + W.DXDALL, AE));
+            GVX_TRY(nt_gemm_bf16(st, TB, AE, 4 * d.H, DGDRM, 4 * d.H, (const bf16 *)(packed + BL.WdTRM), 4 * d.H, x + W.DXDALL, AE, err));
         }
     }
 
-    // OPT-IN (GVX_S4_FUSED=1): measured on B200 at configs[2] the folded kernel is SLOWER than GEMM + pointwise (phase 13.3 ms
-    // vs 10.6 ms per train step, whole step 73.1 vs 65.8 ms): its 128 blocks serialise staging, contraction and the
-    // latency-bound cell backward, while the two-launch version overlaps them through programmatic dependent launch
-    static const bool s4_fused = getenv("GVX_S4_FUSED") && getenv("GVX_S4_FUSED")[0] == '1';
-    // d q . W_query folded into the 2-CTA cluster attention-backward kernel (its conv-transpose phase leaves 320 threads idle):
-    // one launch less per step.  GVX_DHQ_FOLDED=0 restores the separate engine GEMM.
-    static const bool dhq_env = !(getenv("GVX_DHQ_FOLDED") && getenv("GVX_DHQ_FOLDED")[0] == '0');
-    const bool dhq_folded = dhq_env && !s4_fused && d.A % 16 == 0 && d.A <= 1024 && attention_bwd_uses_c2(AttnShape{B, N, d.D, d.E, d.F, d.KS});
-    // the fused forward chain left a bf16 copy of the encoder memory in the stash: operand of d w in the attention backward
-    const bool fb = fused_chains_ok(d, B, N) || fused_bwd_only_ok(d, B, N);
-    const bool have_memb = fb;
     if (fb) {   // BPTT of the attention chain for all frames in one persistent launch (gvx_fused_bwd.cuh)
         ProfScope ps(PS_BWD_ATTENTION, st);
         FbArgs f;
@@ -717,7 +634,6 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
             a.dconv_out = x + W.DCONV + (size_t)t * B * N * d.F;
             a.dbg = pc_dbg_buffer() ? pc_dbg_buffer() + 32 * 1024 : nullptr;     // plane 1, row = frame (the decoder-LSTM BPTT chain
             a.dbg_t = t;                                                         // of the same call wrote its stamps there before)
-            if (have_memb) a.memb = (const bf16 *)(s + S.MEMB);
             a.dctx12_static = pc ? 1 : 0;      // DHC and DXDALL are complete before the per-step chain starts
             if (dhq_folded) { a.WqB = (const bf16 *)(packed + BL.WqB); a.dhq_out = x + W.PS4; a.A = d.A; }
             GVX_TRY(launch_attention_bwd_best(a, st));
@@ -730,19 +646,11 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
             SrcSum dpre = last ? src_none() : src_split(pdxa_n, lda, W.KSaT, sa);
             const SrcSum s1 = pc ? src_plain(dxd_t, AE) : src_split(pdxd, ldd, W.KSdT, sd);
             const SrcSum s2 = last ? src_none() : src_split(pdxa_n + d.P + d.E, lda, W.KSaT, sa);
-            if (s4_fused) {
-                // d q . W_query inside the pointwise kernel: one launch instead of a K = 128 engine GEMM + pointwise
-                GVX_TRY(run_bf_lstm_bwd_q(d, DQRM + (size_t)t * B * d.D, packed + PL.WqT, s1, s2, s + S.GA + (size_t)t * 4 * BA,
-                                          s + S.CA + t * BA, s + S.CA + (t + 1) * BA, x + W.DCA, dg, B, seed, t, training, row_offset,
-                                          last ? nullptr : &dpre, last ? nullptr : s + S.PRE2 + (size_t)(t + 1) * B * d.P,
-                                          last ? nullptr : x + W.DZ2 + (size_t)(t + 1) * B * d.P, st));
-            } else {
-                if (!dhq_folded) GVX_TRY(run_tc(WqTI, DQI, x + W.PS4, gm.TqT, gm.Dp, W.KSs4, B, err, st));
-                GVX_TRY(run_bf_lstm_bwd(d, 0, dhq_folded ? src_plain(x + W.PS4, d.A) : src_split(x + W.PS4, lds4, W.KSs4, (long long)B * lds4), s1, s2,
-                                        s + S.GA + (size_t)t * 4 * BA, s + S.CA + t * BA, s + S.CA + (t + 1) * BA, x + W.DCA, dg, B, seed,
-                                        t, training, row_offset, last ? nullptr : &dpre, last ? nullptr : s + S.PRE2 + (size_t)(t + 1) * B * d.P,
-                                        last ? nullptr : x + W.DZ2 + (size_t)(t + 1) * B * d.P, st));
-            }
+            if (!dhq_folded) GVX_TRY(run_tc(WqTI, DQI, x + W.PS4, gm.TqT, gm.Dp, W.KSs4, B, err, st));
+            GVX_TRY(run_bf_lstm_bwd(d, 0, dhq_folded ? src_plain(x + W.PS4, d.A) : src_split(x + W.PS4, lds4, W.KSs4, (long long)B * lds4), s1, s2,
+                                    s + S.GA + (size_t)t * 4 * BA, s + S.CA + t * BA, s + S.CA + (t + 1) * BA, x + W.DCA, dg, B, seed,
+                                    t, training, row_offset, last ? nullptr : &dpre, last ? nullptr : s + S.PRE2 + (size_t)(t + 1) * B * d.P,
+                                    last ? nullptr : x + W.DZ2 + (size_t)(t + 1) * B * d.P, st));
         }
         {   // S5: d x_att = d gates_att . W_att
             ProfScope ps(PS_BWD_ATT_GEMM, st);
@@ -751,8 +659,7 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
     }
     ProfScope ps_batched(PS_BWD_BATCHED, st);
     if (fb) {   // prenet columns of d x_att for all frames: d gates_att . W_ih[:, prenet], then the relu / dropout mask (:143)
-        if (own_gemm()) GVX_TRY(nt_gemm_bf16(st, TB, d.P, 4 * d.A, DGARM, 4 * d.A, (const bf16 *)(packed + BL.WaTRM), 4 * d.A, x + W.DZ1, d.P, err));
-        else GVX_TRY(gemm_nn_bf16(st, TB, d.P, 4 * d.A, DGARM, 4 * d.A, (const bf16 *)(packed + BL.WaPRM), d.P, x + W.DZ1, d.P));
+        GVX_TRY(nt_gemm_bf16(st, TB, d.P, 4 * d.A, DGARM, 4 * d.A, (const bf16 *)(packed + BL.WaTRM), 4 * d.A, x + W.DZ1, d.P, err));
         k_prenet_bwd_mask<<<grid_for((size_t)TB * d.P), 256, 0, st>>>(x + W.DZ1, d.P, s + S.PRE2, TB, d.P, x + W.DZ2);
         GVX_LAUNCHED(1);
         GVX_CUDA(cudaGetLastError());
@@ -769,11 +676,9 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
     }
     // projections: d Wpg = DOUT^T . [h_dec | ctx];  biases = column sums
     float *tmp = x + W.TMP;
-    // weight gradients: d W = G^T . X over all frames.  Own GEMM: the frame-major operands are consumed as they lie in HBM (MN-major
+    // weight gradients: d W = G^T . X over all frames.  The frame-major operands are consumed as they lie in HBM (MN-major
     // tcgen05 operands, gvx_nt_gemm.cuh: no transpose pass), small outputs split over K (deterministic reduction)
-    const bool og = own_gemm();
-    if (og) GVX_TRY(tn_gemm_bf16(st, d.M + 1, d.Kp, TB, DOUTB, OLB, HCRM, d.Kp, tmp, d.Kp, err, x + W.GWS, W.gws_floats));
-    else GVX_TRY(gemm_tn_bf16(st, d.M + 1, d.Kp, TB, DOUTB, OLB, HCRM, d.Kp, tmp, d.Kp));
+    GVX_TRY(tn_gemm_bf16(st, d.M + 1, d.Kp, TB, DOUTB, OLB, HCRM, d.Kp, tmp, d.Kp, err, x + W.GWS, W.gws_floats));
     GVX_CUDA(cudaMemcpyAsync(g->proj_w, tmp, (size_t)d.M * d.Kp * sizeof(float), cudaMemcpyDeviceToDevice, st));
     GVX_CUDA(cudaMemcpyAsync(g->gate_w, tmp + (size_t)d.M * d.Kp, (size_t)d.Kp * sizeof(float), cudaMemcpyDeviceToDevice, st));
     GVX_TRY(colsum(st, x + W.DOUT, TB, d.M + 1, d.OL, x + W.ONES, x + W.DBIAS));
@@ -789,15 +694,13 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
         GVX_CUDA(cudaGetLastError());
         return 0;
     };
-    if (og) GVX_TRY(tn_gemm_bf16(st, 4 * d.H, d.Kd, TB, DGDRM, 4 * d.H, XDRM, d.Kd, x + W.DWD, d.Kd, err, x + W.GWS, W.gws_floats));
-    else GVX_TRY(gemm_tn_bf16(st, 4 * d.H, d.Kd, TB, DGDRM, 4 * d.H, XDRM, d.Kd, x + W.DWD, d.Kd));
+    GVX_TRY(tn_gemm_bf16(st, 4 * d.H, d.Kd, TB, DGDRM, 4 * d.H, XDRM, d.Kd, x + W.DWD, d.Kd, err, x + W.GWS, W.gws_floats));
     k_unpack_lstm_grad<<<grid_for((size_t)4 * d.H * d.Kd), 256, 0, st>>>(x + W.DWD, d.H, d.A + d.E, g->dec_w_ih, g->dec_w_hh);
     GVX_LAUNCHED(1);
     GVX_TRY(colsum_bf(DGDRM, 4 * d.H, x + W.DBIAS));
     k_unpack_bias_grad<<<grid_for((size_t)4 * d.H), 256, 0, st>>>(x + W.DBIAS, d.H, g->dec_b_ih, g->dec_b_hh);
     GVX_LAUNCHED(1);
-    if (og) GVX_TRY(tn_gemm_bf16(st, 4 * d.A, d.Ka, TB, DGARM, 4 * d.A, XARM, d.Ka, x + W.DWA, d.Ka, err, x + W.GWS, W.gws_floats));
-    else GVX_TRY(gemm_tn_bf16(st, 4 * d.A, d.Ka, TB, DGARM, 4 * d.A, XARM, d.Ka, x + W.DWA, d.Ka));
+    GVX_TRY(tn_gemm_bf16(st, 4 * d.A, d.Ka, TB, DGARM, 4 * d.A, XARM, d.Ka, x + W.DWA, d.Ka, err, x + W.GWS, W.gws_floats));
     k_unpack_lstm_grad<<<grid_for((size_t)4 * d.A * d.Ka), 256, 0, st>>>(x + W.DWA, d.A, d.P + d.E, g->att_w_ih, g->att_w_hh);
     GVX_LAUNCHED(1);
     GVX_TRY(colsum_bf(DGARM, 4 * d.A, x + W.DBIAS));
@@ -805,8 +708,7 @@ int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, con
     GVX_LAUNCHED(1);
     GVX_CUDA(cudaGetLastError());
     // query layer: d Wq [D, A] = DQ^T . h_att   (h_att_t = first A columns of the decoder-LSTM input rows)
-    if (og) GVX_TRY(tn_gemm_bf16(st, d.D, d.A, TB, DQRM, d.D, XDRM, d.Kd, g->query_w, d.A, err, x + W.GWS, W.gws_floats));
-    else GVX_TRY(gemm_tn_bf16(st, d.D, d.A, TB, DQRM, d.D, XDRM, d.Kd, g->query_w, d.A));
+    GVX_TRY(tn_gemm_bf16(st, d.D, d.A, TB, DQRM, d.D, XDRM, d.Kd, g->query_w, d.A, err, x + W.GWS, W.gws_floats));
 
     BwdPostArgs pa;
     pa.TH = s + S.TH; pa.DE = x + W.DE; pa.CONVS = s + S.CONVS; pa.DCONV = x + W.DCONV; pa.ALIGN = s + S.ALIGN;
@@ -896,9 +798,6 @@ static int infer_step_bf16(const Dims &d, const gvx_weights *w, const float *pac
 }
 
 size_t packed_total_bf16(const Dims &d) { return PackedBfL(d, PackedL(d).total).total; }
-size_t stash_total_bf16(const Dims &d, int B, int N, int T) { return StashBfL(d, B, N, T).total; }
-size_t bwd_total_bf16(const Dims &d, int B, int N, int T) { return BwdBfL(d, B, N, T).total; }
-size_t stash_seed_off_bf16(const Dims &d, int B, int N, int T) { return StashBfL(d, B, N, T).SEED; }
 
 }  // namespace gvx
 

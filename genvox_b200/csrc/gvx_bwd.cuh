@@ -19,7 +19,6 @@
 #include "../../include/genvox_b200.h"
 #include "gvx_attention_c2.cuh"
 #include "gvx_blas.cuh"
-#include "gvx_graph.cuh"
 #include "gvx_common.cuh"
 #include "gvx_gemm.cuh"
 #include "gvx_layout.cuh"
@@ -27,7 +26,6 @@
 #include "gvx_post_tc.cuh"
 
 namespace gvx {
-int check_dims(const gvx_dims *d);
 
 // S1: decoder-LSTM pointwise backward.  d h_dropped = dh1 (+ dh2)
 __global__ void k_lstm_bwd_pointwise(const float *__restrict__ dh1, int ld1, const float *__restrict__ dh2, int ld2,
@@ -422,31 +420,13 @@ inline int bwd_post_common(const Dims &d, const gvx_weights *w, const float *mem
     return 0;
 }
 
-int train_bwd_bf16(const Dims &d, const gvx_weights *w, const float *packed, const float *memory, const int64_t *mem_lengths,
-                   int B, int N, int T, uint64_t seed, int training, int row_offset, const float *d_mel, const float *d_gate,
-                   const float *d_align, const float *s, float *x, const gvx_grads *g, float *d_memory, cudaStream_t st);
-
-}  // namespace gvx
-
-using namespace gvx;
-
-static int train_bwd_body(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
-                          const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training, int row_offset,
-                          const float *d_mel, const float *d_gate, const float *d_align, const void *stash_, void *workspace,
-                          const gvx_grads *g, float *d_memory, void *stream) {
-    const Dims d(*dd);
-    GVX_CHECK(d.F <= 64 && d.D <= 512, "backward supports loc_filters <= 64 and att_dim <= 512");
-    if (dd->precision == GVX_BF16)
-        return train_bwd_bf16(d, w, (const float *)packed_, memory, mem_lengths, B, N, T, seed, training, row_offset, d_mel, d_gate,
-                              d_align, (const float *)stash_, (float *)workspace, g, d_memory, (cudaStream_t)stream);
+// BPTT in fp32 mode: reads the stash S of train_fwd_fp32, works in W
+int train_bwd_fp32(const Dims &d, const StashL &S, const BwdL &W, const gvx_weights *w, const float *packed, const float *memory,
+                   const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training, int row_offset, const float *d_mel,
+                   const float *d_gate, const float *d_align, const float *s, float *x, const gvx_grads *g, float *d_memory,
+                   cudaStream_t st) {
     GVX_CHECK(d.F * 2 * d.KS <= 8 * 512, "location conv too large for the backward reduction kernel");
-    const StashL S(d, B, N, T);
-    const BwdL W(d, B, N, T);
     const PackedL PL(d);
-    const float *packed = (const float *)packed_;
-    const float *s = (const float *)stash_;
-    float *x = (float *)workspace;
-    cudaStream_t st = (cudaStream_t)stream;
     const int TB = T * B;
     const size_t BA = (size_t)B * d.A, BH = (size_t)B * d.H, BE = (size_t)B * d.E;
 
@@ -586,34 +566,4 @@ static int train_bwd_body(const gvx_dims *dd, const gvx_weights *w, const void *
     return bwd_post_common(d, w, memory, B, N, T, pa, g, d_memory, st);
 }
 
-
-namespace gvx {
-size_t stash_seed_off_bf16(const Dims &d, int B, int N, int T);
-}
-
-extern "C" int gvx_dec_train_bwd(const gvx_dims *dd, const gvx_weights *w, const void *packed_, const float *memory,
-                                 const int64_t *mem_lengths, int B, int N, int T, uint64_t seed, int training,
-                                 int row_offset, const float *d_mel, const float *d_gate, const float *d_align,
-                                 const void *stash_, void *workspace, const gvx_grads *g, float *d_memory, void *stream) {
-    GVX_TRY(check_dims(dd));
-    GVX_CHECK(w && packed_ && memory && d_mel && d_gate && stash_ && workspace && g && d_memory, "null argument");
-    GVX_CHECK(B > 0 && N > 0 && T > 0, "B, N, T must be positive");
-    GVX_TRY(latch_check());
-    cudaStream_t user = (cudaStream_t)stream;
-    const Dims d(*dd);
-    const size_t off = dd->precision == GVX_BF16 ? stash_seed_off_bf16(d, B, N, T) : StashL(d, B, N, T).SEED;
-    uint32_t *slot = reinterpret_cast<uint32_t *>((float *)const_cast<void *>(stash_) + off);
-    k_set_seed<<<1, 1, 0, user>>>(slot, (uint32_t)(seed & 0xffffffffull), (uint32_t)(seed >> 32));   // same value the forward stored
-    GVX_LAUNCHED(1);
-    GVX_CUDA(cudaGetLastError());
-    KeyBuilder kb;
-    kb.add((int)2).add(*dd).add(*w).add(packed_).add(memory).add(mem_lengths).add(B).add(N).add(T).add(training).add(row_offset)
-        .add(d_mel).add(d_gate).add(d_align).add(stash_).add(workspace).add(*g).add(d_memory);
-    g_seed_ptr = slot;
-    const int rc = run_cached(kb.k, user, [&](cudaStream_t st) {
-        return train_bwd_body(dd, w, packed_, memory, mem_lengths, B, N, T, seed, training, row_offset, d_mel, d_gate, d_align,
-                              stash_, workspace, g, d_memory, (void *)st);
-    });
-    g_seed_ptr = nullptr;
-    return rc;
-}
+}  // namespace gvx
